@@ -29,6 +29,25 @@ W_MILLER4_M = 65 * (36 + 20 + 4 * 43) + 21 * (37 + 4 * 43) + 2 * (37 + 4 * 43)
 W_FINALEXP_M = 8410
 W_RISC0_M = W_MILLER3_M + W_FINALEXP_M + 1800 + 40 + 1000
 W_SP1_M = W_MILLER3_M + W_FINALEXP_M + 1800 + 40 + 1700
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs: at most this much in all, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array (all of one length n) as out_dir/<name>.npy in float32, so that two builds can be compared output for
+    output.  Past DUMP_BYTES in all, every array keeps the same fixed, seeded sample of indices, written as sample_index.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    per = 4 * len(arrays)
+    index_path = os.path.join(out_dir, "sample_index.npy")
+    if n * per + 4096 > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(n, (DUMP_BYTES - 4096) // (per + 8), replace=False))
+        np.save(index_path, idx.astype(np.float64))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+    elif os.path.exists(index_path):
+        os.remove(index_path)          # left by an earlier, sampled dump into the same directory
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def ncu_summary(kernel):
@@ -53,9 +72,23 @@ def ncu_summary(kernel):
 
 def workload_config(shape, n):
     """`config` of the JSON line: the workload only, shared verbatim by this repo's arm and the --impl reference arm"""
-    return {"workload": "%s: 2^%d synthetic %s-shape Groth16 proofs per GPU per step (%d public inputs, fixed random vk, trapdoor-simulated, all valid)" %
-            ("configs[1]" if shape == "risc0" else "configs[2] shape", n.bit_length() - 1, "RISC Zero" if shape == "risc0" else "SP1 v5", 5 if shape == "risc0" else 2),
+    return {"workload": "%s: 2^%d synthetic %s-shape Groth16 proofs per GPU per step (%d public inputs, fixed random vk, trapdoor-simulated; a seeded half "
+                        "carries one flipped bit of its %s and is rejected after the full verification path)" %
+            ("configs[1]" if shape == "risc0" else "configs[2] shape", n.bit_length() - 1, "RISC Zero" if shape == "risc0" else "SP1 v5", 5 if shape == "risc0" else 2,
+             "journal digest" if shape == "risc0" else "public values"),
             "proofs_per_gpu": n, "sharding": "contiguous proof ranges, no collective"}
+
+
+def tamper_half(S, batch, shape, seed):
+    """Flips one bit of the journal digest (RISC Zero) or of the public values (SP1) of a fixed, seeded half of the proofs, in place, and
+    sets their expected status to VerificationFailed.  Such a proof changes only a hashed public input: it runs the whole verification
+    path at the cost of a valid one (decode, hashing, vk_x, G2 check, Miller loop, final exponentiation) and is rejected by the final
+    comparison, so the per-proof statuses depend on every stage of the computation."""
+    import numpy as np
+    field = batch.journals if shape == "risc0" else batch.public_values
+    for i in np.flatnonzero(np.random.default_rng(seed).random(len(field)) < 0.5):
+        b = bytearray(field[i]); b[-1] ^= 1; field[i] = bytes(b)
+        batch.expect[i] = S.ST_VERIFICATION_FAILED
 
 
 def dist_env():
@@ -109,11 +142,12 @@ def make_workload(Z, S, consts, device, n, shape, seed):
         v = Z.RiscZeroVerifier(kv, devices=[device])
         v.initialize(h(r["control_root"]), h(r["bn254_control_id"]))
         b = S.make_risc0_batch(gpu, vk, v.get_selector(), h(r["control_root"]), h(r["bn254_control_id"]), h(consts["risc0_system_state_zero_digest"]), n, seed, pool=4096)
-        return v, kv, vk, b
-    vk = S.make_vk(gpu, 1, 3, 0xB2000003)
-    kv = Z.VerificationKey(1, vk.alpha, vk.beta, vk.gamma, vk.delta, vk.ic, devices=[device])
-    v = Z.Sp1Verifier(kv, devices=[device])
-    b = S.make_sp1_batch(gpu, vk, n, seed, pool=4096)
+    else:
+        vk = S.make_vk(gpu, 1, 3, 0xB2000003)
+        kv = Z.VerificationKey(1, vk.alpha, vk.beta, vk.gamma, vk.delta, vk.ic, devices=[device])
+        v = Z.Sp1Verifier(kv, devices=[device])
+        b = S.make_sp1_batch(gpu, vk, n, seed, pool=4096)
+    tamper_half(S, b, shape, seed)
     return v, kv, vk, b
 
 
@@ -133,7 +167,7 @@ def cpu_baseline(O, shape, vk, batch, consts, target_s=12.0):
     rate0 = m0 / (t1 - t0)
     m = int(min(len(batch.expect), max(m0, rate0 * target_s)))
     t0 = time.perf_counter(); st = run(m); t1 = time.perf_counter()
-    assert int((np.asarray(st) == 0).sum()) == m, "oracle rejected a synthetic valid proof"
+    assert np.asarray(st).tolist() == batch.expect[:m], "oracle status differs from the synthetic batch's expectation"
     return {"value": m / (t1 - t0), "unit": "verifies/s", "cores": cores, "kind": "port",
             "sample": "first %d proofs of the same batch, oracle/zkv_oracle.c under OpenMP schedule(dynamic), %.1f s" % (m, t1 - t0)}, st
 
@@ -162,13 +196,16 @@ def run_reference(args, rank, world):
     ro.initialize(h(r["control_root"]), h(r["bn254_control_id"]))
     m = 4096                            # bounded sample per step: the first 4096 proofs of the same seeded workload (about 1 s on 16 threads)
     b = S.make_risc0_batch(OB(), vk, ro.selector(), h(r["control_root"]), h(r["bn254_control_id"]), h(consts["risc0_system_state_zero_digest"]), m, 0xB2000001, pool=256)
+    tamper_half(S, b, "risc0", 0xB2000001)
     for _ in range(args.warmup):
         ro.verify_batch(b.seals, b.image_ids, b.journals)
     t0 = time.perf_counter()
     for _ in range(args.steps):
         st = ro.verify_batch(b.seals, b.image_ids, b.journals)
     dt = time.perf_counter() - t0
-    assert int((np.asarray(st) == 0).sum()) == m
+    assert np.asarray(st).tolist() == b.expect
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"status": np.asarray(st)})
     val = m * args.steps / dt
     line = {"impl": "reference", "metric": "groth16_verifies_per_sec", "value": val, "unit": "verifies/s", "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u256 (4x64-bit Montgomery)",
@@ -194,7 +231,11 @@ def main():
     ap.add_argument("--segments", type=int, default=0, help="Miller loop segments per chunk (0 = library default)")
     ap.add_argument("--chunks", type=int, default=0, help="stream-overlap chunks per device batch (0 = library default)")
     ap.add_argument("--layout", type=int, default=-1, help="1 = shared-memory-resident lazily reduced kernels (default), 0 = the round-1 thread-stack kernels (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the per-proof status bytes of the last step as DIR/<name>.npy "
+                                                          "(float32; status = device-resident path, e2e_status = host-buffer path; rank 0 only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, local_rank, world = dist_env()
     if args.impl == "reference":
         return run_reference(args, rank, world)
@@ -263,7 +304,8 @@ def main():
     for _ in range(max(args.warmup, 3)):
         launch(d_st, sp)
     torch.cuda.synchronize()
-    assert int((d_st == 0).sum().item()) == n, "a synthetic valid proof was rejected"
+    expect = torch.tensor(batch.expect, dtype=torch.uint8, device="cuda")
+    assert bool((d_st == expect).all()), "a status differs from the synthetic batch's expectation"
     imad_peak, fpmul_peak = Z.imad_peak(dev)
 
     # per-kernel durations for the roofline: one chain on one stream (no overlap between chunks), CUDA events around every stage
@@ -298,6 +340,7 @@ def main():
     with ClockSampler(dev) as clocks:
         for k in range(args.steps):
             flush.fill_(k)                                    # evict L2 between timed steps (not timed)
+            d_st.fill_(255)                                   # each step must write every status itself (not timed)
             ev[k][0].record(stream)
             launch(d_st, sp)
             ev[k][1].record(stream)
@@ -305,19 +348,22 @@ def main():
         barrier()
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     launches = Z.launch_count() - launches0          # counted by the library at its launch sites (all chunks, Miller segments, final-exp stages)
-    assert int((d_st == 0).sum().item()) == n
+    assert bool((d_st == expect).all())
 
     # ---- end to end through the C-ABI with host buffers
     out = np.zeros(n, dtype=np.uint8)
     for _ in range(2):
         e2e_call(out)
     barrier()
+    out.fill(255)                                     # the timed calls must write every status themselves
     t0 = time.perf_counter()
     for _ in range(args.steps):
         e2e_call(out)
     torch.cuda.synchronize()
     e2e_s = time.perf_counter() - t0
-    assert int((out == 0).sum()) == n
+    assert out.tolist() == batch.expect
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"status": d_st.cpu().numpy(), "e2e_status": out})
 
     t = torch.tensor([dev_ms, e2e_s], dtype=torch.float64, device="cuda")
     if use_dist:
