@@ -62,6 +62,33 @@ void zkv_vk_free(zkv_vk* vk);
  * ZKV_OK or ZKV_VERIFICATION_FAILED. */
 int zkv_groth16_verify_batch(const zkv_vk* vk, const uint8_t* proofs, const uint8_t* signals, int k, size_t n, uint8_t* status_out);
 
+/* ---- many keys in one batch: N independent verify_proof_with_key calls (common/groth16.rs:23-49) ---------
+ * A set of 1..256 loaded keys (borrowed: they must outlive the set).  Every key must be loaded on every device of the set
+ * (devices == NULL -> device 0); keys may differ in vm_type and n_ic.  zkv_vkset_create returns ZKV_ERR_ARG for a key missing on
+ * a set device, and for a valid key with finite gamma and delta whose normalised line tables could not be built (a vanishing line
+ * coefficient).  A set always runs the default schedule (shared-memory kernels, normalised lines, automatic chunking): the member
+ * keys' zkv_vk_tune settings do not apply to it.
+ *
+ * zkv_groth16_verify_batch_keys: proof i (256 B, the layout of zkv_groth16_verify_batch) is verified under keys[key_idx[i]] with
+ * the signals signals[sig_off[i] .. sig_off[i+1]) (offsets in 32-byte words, n+1 of them, non-decreasing).  status_out[i] =
+ * ZKV_OK or ZKV_VERIFICATION_FAILED in caller order: exactly what zkv_groth16_verify_batch returns for that proof alone under its
+ * own key, so a signal count other than that key's n_ic - 1 (groth16.rs:32) fails that proof only, the RISC Zero negation of A
+ * applies to proofs of ZKV_VM_RISC0 keys only, and a key with an invalid point fails all of its proofs.  A key index >= n_keys,
+ * decreasing offsets or a null pointer returns ZKV_ERR_ARG with status_out untouched; n == 0 does nothing.  A multi-device set splits
+ * the batch into contiguous caller ranges.  The proofs of a device pass (up to 2^20) are grouped by key on the device before any
+ * verification kernel runs; the kernel launches per pass do not depend on the number of keys (zkv_launch_count: 10 for a pass of
+ * one kernel chain, 41 once the pass's slot bound n + 31 x min(n_keys, n) reaches the automatic chunking threshold of ZKV_TUNE_OVERLAP).
+ * zkv_groth16_verify_batch_keys_device: the same on device-resident arrays of one set device (d_key_idx n x uint32, d_sig_off
+ * n+1 x uint64 indexing d_signals directly), n <= 2^23, enqueued on `stream` (a cudaStream_t), asynchronous.  The index and offset
+ * checks run on the device there: a key index >= n_keys or a decreasing offset fails that proof (ZKV_VERIFICATION_FAILED). */
+typedef struct zkv_vkset zkv_vkset;
+int zkv_vkset_create(const zkv_vk* const* keys, int n_keys, const int* devices, int n_dev, zkv_vkset** out);
+void zkv_vkset_destroy(zkv_vkset* s);
+int zkv_groth16_verify_batch_keys(const zkv_vkset* s, const uint32_t* key_idx, const uint8_t* proofs, const uint8_t* signals,
+                                  const uint64_t* sig_off, size_t n, uint8_t* status_out);
+int zkv_groth16_verify_batch_keys_device(const zkv_vkset* s, int device, const void* d_key_idx, const void* d_proofs,
+                                         const void* d_signals, const void* d_sig_off, size_t n, void* d_status_out, void* stream);
+
 /* ---- RISC Zero (risc0/verifier.rs) -------------------------------------------------------
  * zkv_risc0_create(vk = NULL) uses the reference's hard-coded key; a custom vk (synthetic
  * benchmarks) is borrowed, not owned.  A handle starts un-initialised, like the contract. */

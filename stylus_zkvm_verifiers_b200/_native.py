@@ -21,6 +21,10 @@ _SIGS = {
     "zkv_vk_load_sp1": (C.c_int, [_P, C.c_int, C.POINTER(_P)]),
     "zkv_vk_free": (None, [_P]),
     "zkv_groth16_verify_batch": (C.c_int, [_P, _P, _P, C.c_int, C.c_size_t, _P]),
+    "zkv_vkset_create": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(_P)]),
+    "zkv_vkset_destroy": (None, [_P]),
+    "zkv_groth16_verify_batch_keys": (C.c_int, [_P, _P, _P, _P, _P, C.c_size_t, _P]),
+    "zkv_groth16_verify_batch_keys_device": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, C.c_size_t, _P, _P]),
     "zkv_risc0_create": (C.c_int, [_P, _P, C.c_int, C.POINTER(_P)]),
     "zkv_risc0_destroy": (None, [_P]),
     "zkv_risc0_initialize": (C.c_int, [_P, _P, _P]),

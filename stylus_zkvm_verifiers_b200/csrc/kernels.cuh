@@ -57,26 +57,14 @@ __device__ __forceinline__ int g2_decode_bytes(fp2& x, fp2& y, const uint8_t* b)
 // the front checks of risc0/verifier.rs:151-170 / sp1/verifier.rs:64-83 happen HERE, in the reference's order: length < 4 ->
 // InvalidProofData, selector mismatch, length - 4 != 256 -> InvalidProofData (strict abi_decode of 8 x uint256).  rec + off points at
 // 8 x BE-32.  vm == RISC0 applies negate_g1 exactly as groth16.rs:75-84 does: on the raw 256-bit words, BEFORE any range check.
-__global__ void k_decode(int n, const uint8_t* recs, size_t stride, size_t off, uint32_t selector_le, int check_selector, int vm,
-                         const uint64_t* rec_off, uint64_t rec_base,
-                         fp* ax, fp* ay, fp2* bx, fp2* by, fp* cx, fp* cy, uint8_t* flags) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const uint8_t* rec = rec_off ? recs + (size_t)(rec_off[i] - rec_base) : recs + (size_t)i * stride;
-    const uint64_t len = rec_off ? rec_off[i + 1] - rec_off[i] : (uint64_t)stride;
+// a record that never reaches the Groth16 stage: harmless operands for the uniform kernels behind, and its reject flag
+__device__ __forceinline__ void decode_reject(int i, uint8_t fl, fp* ax, fp* ay, fp2* bx, fp2* by, fp* cx, fp* cy, uint8_t* flags) {
+    ax[i] = fp_zero(); ay[i] = fp_zero(); cx[i] = fp_zero(); cy[i] = fp_zero(); bx[i] = f2_zero(); by[i] = f2_zero();
+    flags[i] = fl | F_SKIP0 | F_SKIPC;
+}
+// (a, b, c) of the 8 x BE-32 words at p into slot i (k_decode and k_decode_keys)
+__device__ __forceinline__ void decode_points(int i, const uint8_t* p, int vm, fp* ax, fp* ay, fp2* bx, fp2* by, fp* cx, fp* cy, uint8_t* flags) {
     uint8_t fl = 0;
-    if (rec_off && len < 4) fl = F_BADDATA;
-    else if (check_selector) {
-        uint32_t s = (uint32_t)rec[0] | (uint32_t)rec[1] << 8 | (uint32_t)rec[2] << 16 | (uint32_t)rec[3] << 24;
-        if (s != selector_le) fl = F_SELMIS;
-    }
-    if (rec_off && !fl && len != off + 256) fl = F_BADDATA;
-    if (fl) {                                             // never reaches the Groth16 stage: leave harmless operands for the uniform kernels behind
-        ax[i] = fp_zero(); ay[i] = fp_zero(); cx[i] = fp_zero(); cy[i] = fp_zero(); bx[i] = f2_zero(); by[i] = f2_zero();
-        flags[i] = fl | F_SKIP0 | F_SKIPC;
-        return;
-    }
-    const uint8_t* p = rec + off;
     uint32_t rx[8], ry[8];
     be32_to_raw(rx, p); be32_to_raw(ry, p + 32);
     if (vm == 0) {
@@ -100,6 +88,23 @@ __global__ void k_decode(int n, const uint8_t* recs, size_t stride, size_t off, 
     if (ra == 1 || rb == 1) fl |= F_SKIP0;
     if (rc == 1) fl |= F_SKIPC;
     flags[i] = fl;
+}
+__global__ void k_decode(int n, const uint8_t* recs, size_t stride, size_t off, uint32_t selector_le, int check_selector, int vm,
+                         const uint64_t* rec_off, uint64_t rec_base,
+                         fp* ax, fp* ay, fp2* bx, fp2* by, fp* cx, fp* cy, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint8_t* rec = rec_off ? recs + (size_t)(rec_off[i] - rec_base) : recs + (size_t)i * stride;
+    const uint64_t len = rec_off ? rec_off[i + 1] - rec_off[i] : (uint64_t)stride;
+    uint8_t fl = 0;
+    if (rec_off && len < 4) fl = F_BADDATA;
+    else if (check_selector) {
+        uint32_t s = (uint32_t)rec[0] | (uint32_t)rec[1] << 8 | (uint32_t)rec[2] << 16 | (uint32_t)rec[3] << 24;
+        if (s != selector_le) fl = F_SELMIS;
+    }
+    if (rec_off && !fl && len != off + 256) fl = F_BADDATA;
+    if (fl) { decode_reject(i, fl, ax, ay, bx, by, cx, cy, flags); return; }
+    decode_points(i, rec + off, vm, ax, ay, bx, by, cx, cy, flags);
 }
 
 // K3: RISC Zero public signals 2 and 3 (risc0/verifier.rs:172-179 + crypto.rs:103-110 split_digest):
@@ -157,14 +162,13 @@ __global__ void k_generic_signals(int n, int k, const uint8_t* sig, uint32_t* sc
 
 // K5: vk_x = base + sum_t s_t * IC_t from 4-bit fixed-base window tables (compute_vk_x, groth16.rs:51-58,
 // i.e. the k ecMul + k ecAdd precompile calls).  tab[t][w][d-1] = d * 16^w * IC_t (affine, Montgomery).
-__global__ void k_vkx(int n, const uint32_t* scal, int ns, int nwin, const g1aff* tab, g1aff base, fp* vx, fp* vy, uint8_t* flags) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+// vk_x of slot i: its `ns` scalars start at scal + i * stride * 8 (k_vkx: stride = ns; k_vkx_keys: the set's widest key)
+__device__ __forceinline__ void vkx_one(int i, const uint32_t* scal, int stride, int ns, int nwin, const g1aff* tab, const g1aff& base, fp* vx, fp* vy, uint8_t* flags) {
     g1j acc;
     if (fp_is_zero(base.x) && fp_is_zero(base.y)) { acc.x = fp_one(); acc.y = fp_one(); acc.z = fp_zero(); }
     else { acc.x = base.x; acc.y = base.y; acc.z = fp_one(); }
     for (int t = 0; t < ns; t++) {
-        const uint32_t* s = scal + ((size_t)i * ns + t) * 8;
+        const uint32_t* s = scal + ((size_t)i * stride + t) * 8;
         const g1aff* tt = tab + (size_t)t * ZKV_WIN_PER_SCALAR * ZKV_WIN_ENTRIES;
         for (int w = 0; w < nwin; w++) {
             uint32_t d = (s[w >> 3] >> ((w & 7) * 4)) & 15u;
@@ -179,6 +183,11 @@ __global__ void k_vkx(int n, const uint32_t* scal, int ns, int nwin, const g1aff
     bool fin = g1_to_affine(x, y, acc);
     vx[i] = x; vy[i] = y;
     if (!fin && flags) flags[i] |= F_SKIPX;
+}
+__global__ void k_vkx(int n, const uint32_t* scal, int ns, int nwin, const g1aff* tab, g1aff base, fp* vx, fp* vy, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    vkx_one(i, scal, ns, ns, nwin, tab, base, vx, vy, flags);
 }
 
 // K2: order-r membership of B (EIP-197; the reference reaches it through ecPairing, groth16.rs:121-125)
@@ -404,16 +413,19 @@ __device__ __noinline__ void lz_slopes_to(fp* sl, const fp* x1, const fp* y1, co
     g1_slopes2(xy, iy, x12, y12, off);
     sl[0] = xy[0]; sl[1] = xy[1]; sl[2] = iy[0]; sl[3] = iy[1];
 }
-__global__ void __launch_bounds__(LZ_NT, 2) k_miller_lz(int n, MillerArgs a, const uint8_t* flags, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
+// body of k_miller_lz / k_miller_lz_keys; the key's tables (nt0, nt1: normalised gamma / delta lines, pre = Miller(alpha, beta)) and its
+// disabled pairs come in separately, the rest from `a`
+__device__ __forceinline__ void miller_lz(int n, const MillerArgs& a, const nline_t* nt0, const nline_t* nt1, const fp12* pre, uint8_t vk_skip,
+                                          const uint8_t* flags, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
     const int i0 = blockIdx.x * LZ_NT + threadIdx.x, i = i0 < n ? i0 : n - 1;
     const uint8_t fl = flags[i];
-    uint32_t skip = a.vk_skip;
+    uint32_t skip = vk_skip;
     for (int j = 0; j < 3; j++) if (fl & a.skip_bit[j]) skip |= 1u << j;
     if (fl & F_REJECT) skip = 0xF;
     fp* mysl = sl + 4 * (size_t)i0;
     if (first) lz_slopes_to(mysl, a.px[1] + i, a.py[1] + i, a.px[2] + i, a.py[2] + i, (skip & 2u) != 0, (skip & 4u) != 0);
     LzMillerIn in;
-    in.px0 = a.px[0] + i; in.py0 = a.py[0] + i; in.qx = a.qx + i; in.qy = a.qy + i; in.sl = mysl; in.nt[0] = a.ntabs[0]; in.nt[1] = a.ntabs[1]; in.var_off = (skip & 1u) != 0;
+    in.px0 = a.px[0] + i; in.py0 = a.py[0] + i; in.qx = a.qx + i; in.qy = a.qy + i; in.sl = mysl; in.nt[0] = nt0; in.nt[1] = nt1; in.var_off = (skip & 1u) != 0;
     const uint32_t tid = lz_tid();
     if (first) lz_miller_init(a.qx[i], a.qy[i]);
     else {
@@ -422,13 +434,16 @@ __global__ void __launch_bounds__(LZ_NT, 2) k_miller_lz(int n, MillerArgs a, con
         lz_st2(tid + LZ_R * LZ_SLOT, R->x); lz_st2(tid + (LZ_R + 2) * LZ_SLOT, R->y); lz_st2(tid + (LZ_R + 4) * LZ_SLOT, R->z);
     }
     lz_miller_norm_seg(in, d_hi, d_lo, last != 0);
-    if (last) { if (a.pre) lz_f12mul_g(tid + LZ_F * LZ_SLOT, tid + LZ_T * LZ_SLOT, tid + LZ_R * LZ_SLOT, a.pre, false); }      // x Miller(alpha, beta); T and R are free now
+    if (last) { if (pre) lz_f12mul_g(tid + LZ_F * LZ_SLOT, tid + LZ_T * LZ_SLOT, tid + LZ_R * LZ_SLOT, pre, false); }      // x Miller(alpha, beta); T and R are free now
     else if (i0 < n) { g2j* R = rst + i; R->x = lz_ld2(tid + LZ_R * LZ_SLOT); R->y = lz_ld2(tid + (LZ_R + 2) * LZ_SLOT); R->z = lz_ld2(tid + (LZ_R + 4) * LZ_SLOT); }
     if (i0 < n) lz_stg12(fio + i, tid + LZ_F * LZ_SLOT);
 }
+__global__ void __launch_bounds__(LZ_NT, 2) k_miller_lz(int n, MillerArgs a, const uint8_t* flags, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
+    miller_lz(n, a, a.ntabs[0], a.ntabs[1], a.pre, a.vk_skip, flags, fio, rst, sl, d_hi, d_lo, first, last);
+}
 // stages s_lo .. s_hi of the final exponentiation (0..3 = all of it in one launch); st = 6 Fp12 of state per LAUNCHED thread; the last stage writes the
 // status (pairing_mode: 1 product is one / 0 it is not / 2 the call reverts) and, if gt_out is set, the value (12 x BE-32, zeroed for rejected inputs)
-__global__ void __launch_bounds__(LZ_NT, 2) k_final_exp_lz(int n, int s_lo, int s_hi, const fp12* in, fp12* st, const uint8_t* flags, uint8_t* status, uint8_t* gt_out, int pairing_mode) {
+__device__ __forceinline__ void final_exp_lz(int n, int s_lo, int s_hi, const fp12* in, fp12* st, const uint8_t* flags, uint8_t* status, uint8_t* gt_out, int pairing_mode) {
     const int i0 = blockIdx.x * LZ_NT + threadIdx.x, i = i0 < n ? i0 : n - 1;
     for (int s = s_lo; s <= s_hi; s++) lz_final_exp_stage(s, in + i, st + 6 * (size_t)i0);
     if (s_hi < 3 || i0 >= n) return;
@@ -446,6 +461,9 @@ __global__ void __launch_bounds__(LZ_NT, 2) k_final_exp_lz(int n, int s_lo, int 
         if (gt_out) fp_to_be32(gt_out + (size_t)i * 384 + 32 * k, w);
     }
     status[i] = pairing_mode ? (t == 0 ? 1 : 0) : (t == 0 ? ST_OK : ST_VERIFICATION_FAILED);
+}
+__global__ void __launch_bounds__(LZ_NT, 2) k_final_exp_lz(int n, int s_lo, int s_hi, const fp12* in, fp12* st, const uint8_t* flags, uint8_t* status, uint8_t* gt_out, int pairing_mode) {
+    final_exp_lz(n, s_lo, s_hi, in, st, flags, status, gt_out, pairing_mode);
 }
 // General multi-Miller loop (lz_miller_gen_seg): nvar variable pairs + nfix tabled pairs per instance, pair-major arrays of `in.stride`
 // entries each (stride >= launched threads: surplus threads work on the padding, whose pskip bytes are 1).  iskip[i] != 0: the instance is
@@ -623,6 +641,158 @@ __global__ void k_ic_tables(const uint8_t* ic /* n_ic x 64, IC_0 first */, g1aff
         fp ex, ey; g1_to_affine(ex, ey, acc);
         o[d].x = ex; o[d].y = ey;
     }
+}
+
+// ---------------------------------------------------------------------------- key sets (zkv_groth16_verify_batch_keys)
+// A batch whose proofs name their own key is first GROUPED: slot s of the workspace holds caller record perm[s] of key slot_key[s], the
+// proofs of one key occupy consecutive slots in caller order, and each key's group is padded to a multiple of 32 slots, so every warp of
+// the Miller kernel works on ONE key (lz_fixed_lines stages a step's gamma / delta line entries once per warp).  Padding slots hold
+// ZKV_SLOT_EMPTY and their group's key; slots behind the last group (the host sizes the workspace for the bound n + 31 x keys present)
+// hold ZKV_SLOT_EMPTY and key 0, and the heavy kernels do not run them (the slot total is read on the device).
+#define ZKV_MAX_KEYS 256
+#define ZKV_GROUP_TILE 4096            /* caller records per block of the grouping kernels: 8 warps x 16 rounds of 32 */
+#define ZKV_SLOT_EMPTY 0xffffffffu
+struct KeyDesc {                       // one key of a set on one device (device memory)
+    g1aff base;                        // IC0
+    const g1aff* tab;                  // window tables of IC1..
+    const nline_t* nt[2];              // normalised gamma / delta line tables
+    const fp12* pre;                   // Miller(alpha, beta)
+    int ns, vm, reject;                // signals per proof (n_ic - 1), ZKV_VM_*, every proof fails (a key point is invalid)
+    uint8_t vk_skip;                   // pairs 1 / 2 disabled for every proof (gamma / delta at infinity), as MillerArgs::vk_skip
+};
+__device__ __forceinline__ uint32_t group_of(uint32_t k, int nk) { return k < (uint32_t)nk ? k : 0u; }   // out-of-range keys fail in group 0
+// per tile t of ZKV_GROUP_TILE records: cnt[t * nk + k] = records of key k
+__global__ void __launch_bounds__(256) k_group_count(int n, int nk, const uint32_t* key_idx, uint32_t* cnt) {
+    __shared__ uint32_t h[ZKV_MAX_KEYS];
+    for (int k = threadIdx.x; k < nk; k += blockDim.x) h[k] = 0;
+    __syncthreads();
+    const size_t t0 = (size_t)blockIdx.x * ZKV_GROUP_TILE;
+    for (int j = threadIdx.x; j < ZKV_GROUP_TILE; j += blockDim.x)
+        if (t0 + j < (size_t)n) atomicAdd(&h[group_of(key_idx[t0 + j], nk)], 1u);
+    __syncthreads();
+    for (int k = threadIdx.x; k < nk; k += blockDim.x) cnt[(size_t)blockIdx.x * nk + k] = h[k];
+}
+// one block of ZKV_MAX_KEYS threads, thread k = key k: group k starts at the exclusive sum of the padded group sizes before it;
+// cnt[t * nk + k] becomes the first slot of tile t's records of key k; the padding slots get their key; *total = slots in all groups
+__global__ void __launch_bounds__(ZKV_MAX_KEYS) k_group_scan(int ntiles, int nk, uint32_t* cnt, uint8_t* slot_key, uint32_t* total) {
+    __shared__ uint32_t sc[ZKV_MAX_KEYS];
+    const int k = threadIdx.x;
+    uint32_t c = 0;
+    if (k < nk) for (int t = 0; t < ntiles; t++) c += cnt[(size_t)t * nk + k];
+    const uint32_t padded = (c + 31u) & ~31u;
+    sc[k] = k < nk ? padded : 0u;
+    __syncthreads();
+    for (int d = 1; d < ZKV_MAX_KEYS; d <<= 1) {
+        const uint32_t v = k >= d ? sc[k - d] : 0u;
+        __syncthreads();
+        sc[k] += v;
+        __syncthreads();
+    }
+    if (k == ZKV_MAX_KEYS - 1) *total = sc[k];
+    if (k >= nk) return;
+    uint32_t s = sc[k] - padded;
+    for (uint32_t p = s + c; p < s + padded; p++) slot_key[p] = (uint8_t)k;
+    for (int t = 0; t < ntiles; t++) { const uint32_t v = cnt[(size_t)t * nk + k]; cnt[(size_t)t * nk + k] = s; s += v; }
+}
+// perm[slot] / slot_key[slot] of every record: warp w of a block takes records [w * 512, w * 512 + 512) of the block's tile in rounds of 32;
+// the rank of a record among its key's records is (tile base) + (that key's records in the tile's earlier warps) + (earlier rounds) + (earlier
+// lanes of its round, __match_any_sync): caller order inside every group, and the same slots on every run
+__global__ void __launch_bounds__(256) k_group_scatter(int n, int nk, const uint32_t* key_idx, const uint32_t* base, uint32_t* perm, uint8_t* slot_key) {
+    __shared__ uint32_t wc[8][ZKV_MAX_KEYS];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int k = lane; k < nk; k += 32) wc[w][k] = 0;
+    __syncwarp();
+    const size_t r0 = (size_t)blockIdx.x * ZKV_GROUP_TILE + (size_t)w * (ZKV_GROUP_TILE / 8);
+    const unsigned lt = (1u << lane) - 1u;
+    for (int r = 0; r < ZKV_GROUP_TILE / 8; r += 32) {
+        const size_t i = r0 + r + lane;
+        const uint32_t k = i < (size_t)n ? group_of(key_idx[i], nk) : ZKV_SLOT_EMPTY;
+        const unsigned peers = __match_any_sync(0xffffffffu, k);
+        if (k != ZKV_SLOT_EMPTY && (peers & lt) == 0) wc[w][k] += __popc(peers);
+        __syncwarp();
+    }
+    __syncthreads();
+    for (int k = threadIdx.x; k < nk; k += blockDim.x) {
+        uint32_t run = base[(size_t)blockIdx.x * nk + k];
+        for (int v = 0; v < 8; v++) { const uint32_t c = wc[v][k]; wc[v][k] = run; run += c; }
+    }
+    __syncthreads();
+    for (int r = 0; r < ZKV_GROUP_TILE / 8; r += 32) {
+        const size_t i = r0 + r + lane;
+        const uint32_t k = i < (size_t)n ? group_of(key_idx[i], nk) : ZKV_SLOT_EMPTY;
+        const unsigned peers = __match_any_sync(0xffffffffu, k);
+        if (k != ZKV_SLOT_EMPTY) { const uint32_t s = wc[w][k] + __popc(peers & lt); perm[s] = (uint32_t)i; slot_key[s] = (uint8_t)k; }
+        __syncwarp();
+        if (k != ZKV_SLOT_EMPTY && (peers & lt) == 0) wc[w][k] += __popc(peers);
+        __syncwarp();
+    }
+}
+// k_decode in slot order: record perm[s] of the 256-byte proofs, the vm of the slot's key; empty slots, out-of-range key indices and keys
+// with an invalid point get the reject flags of a malformed record
+__global__ void k_decode_keys(int n, const uint32_t* perm, const uint8_t* slot_key, const KeyDesc* keys, int nk, const uint32_t* key_idx, const uint8_t* proofs,
+                              fp* ax, fp* ay, fp2* bx, fp2* by, fp* cx, fp* cy, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t p = perm[i];
+    const KeyDesc* kd = keys + slot_key[i];
+    if (p == ZKV_SLOT_EMPTY || key_idx[p] >= (uint32_t)nk || kd->reject) { decode_reject(i, F_INVALID, ax, ay, bx, by, cx, cy, flags); return; }
+    decode_points(i, proofs + (size_t)p * 256, kd->vm, ax, ay, bx, by, cx, cy, flags);
+}
+// signals of record perm[s]: words sig_off[p] .. sig_off[p + 1] of `sig` (offsets relative to sig_base); a count other than the key's
+// n_ic - 1 (groth16.rs:32) or a signal >= R (groth16.rs:32-34) fails the proof.  Scalars at a stride of `stride` (the widest key) per slot.
+__global__ void k_signals_keys(int n, const uint32_t* perm, const uint8_t* slot_key, const KeyDesc* keys, const uint8_t* sig, const uint64_t* sig_off, uint64_t sig_base,
+                               int stride, uint32_t* scal, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t p = perm[i];
+    if (p == ZKV_SLOT_EMPTY) return;
+    const int k = keys[slot_key[i]].ns;
+    const uint64_t a = sig_off[p], b = sig_off[p + 1];
+    if (b < a || b - a != (uint64_t)k) { flags[i] |= F_INVALID; return; }
+    bool bad = false;
+    for (int j = 0; j < k; j++) {
+        uint32_t s[8];
+        be32_to_raw(s, sig + (a - sig_base + j) * 32);
+        bad |= u256_geq(s, C_R);
+        for (int t = 0; t < 8; t++) scal[((size_t)i * stride + j) * 8 + t] = s[t];
+    }
+    if (bad) flags[i] |= F_INVALID;
+}
+// k_vkx with the slot's key: its IC0, window tables and scalar count; empty slots get the point at infinity's encoding and no work
+__global__ void k_vkx_keys(int n, const uint32_t* perm, const uint8_t* slot_key, const KeyDesc* keys, const uint32_t* scal, int stride, fp* vx, fp* vy, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    if (perm[i] == ZKV_SLOT_EMPTY) { vx[i] = fp_zero(); vy[i] = fp_zero(); return; }
+    const KeyDesc* kd = keys + slot_key[i];
+    const g1aff base = kd->base;
+    vkx_one(i, scal, stride, kd->ns, ZKV_WIN_PER_SCALAR, kd->tab, base, vx, vy, flags);
+}
+// slots of a chunk [o, o + m) that lie in a group: the rest of the chunk is not run (whole blocks return; the last block's surplus threads
+// redo the chunk's last grouped slot, whose warp is of a single key since group sizes are multiples of 32)
+__device__ __forceinline__ int grouped_in_chunk(const uint32_t* total, size_t o, int m) {
+    const size_t t = *total;
+    return t <= o ? 0 : (int)(t - o < (size_t)m ? t - o : (size_t)m);
+}
+// k_miller_lz over slots: each warp reads its key's tables (one key per warp, see above)
+__global__ void __launch_bounds__(LZ_NT, 2) k_miller_lz_keys(const uint32_t* total, size_t o, int m, MillerArgs a, const uint8_t* slot_key, const KeyDesc* keys,
+                                                            const uint8_t* flags, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
+    const int n = grouped_in_chunk(total, o, m);
+    if ((int)blockIdx.x * LZ_NT >= n) return;
+    const int i0 = blockIdx.x * LZ_NT + threadIdx.x;
+    const KeyDesc* kd = keys + slot_key[i0 < n ? i0 : n - 1];
+    miller_lz(n, a, kd->nt[0], kd->nt[1], kd->pre, kd->vk_skip, flags, fio, rst, sl, d_hi, d_lo, first, last);
+}
+__global__ void __launch_bounds__(LZ_NT, 2) k_final_exp_lz_keys(const uint32_t* total, size_t o, int m, int s_lo, int s_hi, const fp12* in, fp12* st, const uint8_t* flags, uint8_t* status) {
+    const int n = grouped_in_chunk(total, o, m);
+    if ((int)blockIdx.x * LZ_NT >= n) return;
+    final_exp_lz(n, s_lo, s_hi, in, st, flags, status, nullptr, 0);
+}
+// slot statuses back to caller order
+__global__ void k_status_to_caller(int n, const uint32_t* total, const uint32_t* perm, const uint8_t* slot_status, uint8_t* status) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || (uint32_t)i >= *total) return;
+    const uint32_t p = perm[i];
+    if (p != ZKV_SLOT_EMPTY) status[p] = slot_status[i];
 }
 
 // ---------------------------------------------------------------------------- small services

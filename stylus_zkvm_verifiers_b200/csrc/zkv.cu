@@ -152,7 +152,8 @@ struct zkv_vk {
 };
 static DevCtx* vk_ctx(const zkv_vk* vk, int device) { for (auto* c : vk->devs) if (c->device == device) return c; return nullptr; }
 
-static int vk_build_on(zkv_vk* vk, DevCtx* c) {
+// streams, events and kernel attributes of a context on c->device (the workspace is allocated by the first batch)
+static int ctx_init(DevCtx* c) {
     CK(cudaSetDevice(c->device));
     CK(cudaDeviceGetAttribute(&c->sms, cudaDevAttrMultiProcessorCount, c->device));
     CK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
@@ -164,6 +165,12 @@ static int vk_build_on(zkv_vk* vk, DevCtx* c) {
     CK(cudaFuncSetAttribute(k_miller_lz, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_MILLER));
     CK(cudaFuncSetAttribute(k_final_exp_lz, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_BYTES));
     CK(cudaFuncSetAttribute(k_pairing_lz, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_BYTES));
+    CK(cudaFuncSetAttribute(k_miller_lz_keys, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_MILLER));
+    CK(cudaFuncSetAttribute(k_final_exp_lz_keys, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_BYTES));
+    return 0;
+}
+static int vk_build_on(zkv_vk* vk, DevCtx* c) {
+    int rc = ctx_init(c); if (rc) return rc;
     int nt = vk->n_ic - 1;
     CK(cudaMalloc(&c->d_vk, sizeof(VkDev))); CK(cudaMalloc(&c->d_lines, sizeof(line_t) * 3 * ZKV_LINES_PER_G2)); CK(cudaMalloc(&c->d_nlines, sizeof(nline_t) * 2 * ZKV_LINES_PER_G2)); CK(cudaMalloc(&c->d_pre, sizeof(fp12)));
     CK(cudaMalloc(&c->d_tab, sizeof(g1aff) * (size_t)nt * ZKV_WIN_PER_SCALAR * ZKV_WIN_ENTRIES)); CK(cudaMalloc(&c->d_ic0, sizeof(g1aff)));
@@ -511,12 +518,12 @@ static void collect_stage_ms(DevCtx* c) {
     for (int e = 0; e < 5; e++) { float ms = 0; if (cudaEventElapsedTime(&ms, c->ev[e], c->ev[e + 1]) != cudaSuccess) { cudaGetLastError(); ms = 0; } c->stage_ms[e] = ms; }
 }
 
-// Split `n` items over the vk's devices in contiguous ranges and run fn(ctx, begin, end) on one host thread per device.
+// Split `n` items over the contexts (one per device) in contiguous ranges and run fn(ctx, begin, end) on one host thread per device.
 template <class F>
-static int for_each_device(const zkv_vk* vk, size_t n, F fn) {
-    size_t nd = vk->devs.size();
+static int for_each_device(const std::vector<DevCtx*>& devs, size_t n, F fn) {
+    size_t nd = devs.size();
     if (nd == 1 || n < 4096) {
-        DevCtx* c = vk->devs[0];
+        DevCtx* c = devs[0];
         std::lock_guard<std::mutex> lk(c->mu);
         CK(cudaSetDevice(c->device));
         return fn(c, (size_t)0, n);
@@ -526,7 +533,7 @@ static int for_each_device(const zkv_vk* vk, size_t n, F fn) {
     for (size_t d = 0; d < nd; d++) {
         size_t b = n * d / nd, e = n * (d + 1) / nd;
         th.emplace_back([&, d, b, e]() {
-            DevCtx* c = vk->devs[d];
+            DevCtx* c = devs[d];
             std::lock_guard<std::mutex> lk(c->mu);
             if (cudaSetDevice(c->device) != cudaSuccess) { rcs[d] = ZKV_ERR_CUDA; errs[d] = "cudaSetDevice"; return; }
             rcs[d] = fn(c, b, e);
@@ -539,12 +546,13 @@ static int for_each_device(const zkv_vk* vk, size_t n, F fn) {
 }
 
 // ------------------------------------------------------------------------------------------ generic Groth16
+static bool offsets_ok(const uint64_t* off, size_t n) { for (size_t i = 0; i < n; i++) if (off[i + 1] < off[i]) return false; return true; }
 extern "C" int zkv_groth16_verify_batch(const zkv_vk* vk, const uint8_t* proofs, const uint8_t* signals, int k, size_t n, uint8_t* status_out) {
     if (!vk || (n && (!proofs || !status_out)) || k < 0 || (n && k && !signals)) return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch: bad argument");
     if (n == 0) return 0;
     if (k + 1 != vk->n_ic) { memset(status_out, ZKV_VERIFICATION_FAILED, n); return 0; }        // groth16.rs:32
     const bool direct = n >= 4096 && is_pinned(proofs) && (k == 0 || is_pinned(signals));      // page-locked caller arrays are uploaded in place
-    return for_each_device(vk, n, [&](DevCtx* c, size_t b, size_t e) -> int {
+    return for_each_device(vk->devs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
         for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
             size_t m = std::min(MAX_CHUNK, e - s0);
             int rc = host_pipeline(c, vk, m, m * (256 + (size_t)k * 32), k,
@@ -562,6 +570,196 @@ extern "C" int zkv_groth16_verify_batch(const zkv_vk* vk, const uint8_t* proofs,
         }
         return 0;
     });
+}
+
+// ------------------------------------------------------------------------------------------ key sets: N verify_proof_with_key calls (groth16.rs:23-49)
+// A set borrows its keys' device tables and owns, per device, a workspace context without key tables plus the grouping arrays.  A call groups
+// each device pass by key on the device (kernels.cuh, "key sets"), runs the front kernels over the pass in slot order and the heavy kernels
+// chunked like run_verify, then scatters the slot statuses back to caller order.
+struct SetDev {
+    DevCtx* c = nullptr;
+    KeyDesc* d_keys = nullptr;
+    uint32_t* perm = nullptr; uint8_t* slot_key = nullptr; uint8_t* slot_status = nullptr; size_t slot_cap = 0;
+    uint32_t* tile = nullptr; size_t tile_cap = 0; uint32_t* total = nullptr;
+};
+struct zkv_vkset {
+    std::vector<const zkv_vk*> keys;
+    std::vector<SetDev> devs;
+    std::vector<DevCtx*> ctxs;            // devs[d].c (for_each_device)
+    int ns_max = 1;                       // signals per proof of the widest key: the scalar stride of a slot
+};
+static SetDev* set_dev(const zkv_vkset* s, int device) {
+    for (auto& d : s->devs) if (d.c->device == device) return const_cast<SetDev*>(&d);
+    return nullptr;
+}
+extern "C" void zkv_vkset_destroy(zkv_vkset* s) {
+    if (!s) return;
+    for (auto& d : s->devs) {
+        if (!d.c) continue;
+        cudaSetDevice(d.c->device);
+        cudaFree(d.d_keys); cudaFree(d.perm); cudaFree(d.slot_key); cudaFree(d.slot_status); cudaFree(d.tile); cudaFree(d.total);
+        ctx_free(d.c);
+    }
+    delete s;
+}
+static int vkset_build_on(zkv_vkset* s, SetDev& sd) {
+    int rc = ctx_init(sd.c); if (rc) return rc;
+    std::vector<KeyDesc> h(s->keys.size());
+    for (size_t k = 0; k < h.size(); k++) {
+        const zkv_vk* vk = s->keys[k];
+        const DevCtx* kc = vk_ctx(vk, sd.c->device);
+        KeyDesc& q = h[k]; memset(&q, 0, sizeof q);
+        q.base = kc->h_ic0; q.tab = kc->d_tab; q.nt[0] = kc->d_nlines; q.nt[1] = kc->d_nlines + ZKV_LINES_PER_G2; q.pre = kc->d_pre;
+        q.ns = vk->n_ic - 1; q.vm = vk->vm; q.reject = !vk->valid;
+        q.vk_skip = (uint8_t)((kc->h_vk.g2_inf[1] ? 2 : 0) | (kc->h_vk.g2_inf[2] ? 4 : 0));
+    }
+    CK(cudaMalloc(&sd.d_keys, sizeof(KeyDesc) * h.size())); CK(cudaMalloc(&sd.total, sizeof(uint32_t)));
+    CK(cudaMemcpy(sd.d_keys, h.data(), sizeof(KeyDesc) * h.size(), cudaMemcpyHostToDevice));
+    return 0;
+}
+extern "C" int zkv_vkset_create(const zkv_vk* const* keys, int n_keys, const int* devices, int n_dev, zkv_vkset** out) {
+    if (!out || !keys) return fail(ZKV_ERR_ARG, "zkv_vkset_create: null argument");
+    if (n_keys < 1 || n_keys > ZKV_MAX_KEYS) return fail(ZKV_ERR_ARG, "zkv_vkset_create: n_keys must be 1..256");
+    for (int k = 0; k < n_keys; k++) if (!keys[k]) return fail(ZKV_ERR_ARG, "zkv_vkset_create: null key");
+    int ndev_sys = zkv_device_count();
+    if (ndev_sys <= 0) return fail(ZKV_ERR_CUDA, "zkv_vkset_create: no CUDA device (this library has no CPU path)");
+    std::vector<int> devs;
+    if (!devices || n_dev <= 0) devs.push_back(0); else devs.assign(devices, devices + n_dev);
+    for (int d : devs) if (d < 0 || d >= ndev_sys) return fail(ZKV_ERR_ARG, "zkv_vkset_create: bad device index");
+    for (int k = 0; k < n_keys; k++)
+        for (int d : devs) {
+            const DevCtx* kc = vk_ctx(keys[k], d);
+            if (!kc) return fail(ZKV_ERR_ARG, "zkv_vkset_create: key " + std::to_string(k) + " is not loaded on device " + std::to_string(d));
+            // a valid key whose gamma and delta are finite has normalised line tables unless a line coefficient vanished (not expected for
+            // points of G2); the set has no unscaled-line path for such a key
+            if (keys[k]->valid && !kc->h_vk.norm_ok && !kc->h_vk.g2_inf[1] && !kc->h_vk.g2_inf[2])
+                return fail(ZKV_ERR_ARG, "zkv_vkset_create: key " + std::to_string(k) + " has no normalised gamma / delta line tables (a vanishing line coefficient)");
+        }
+    zkv_vkset* s = new zkv_vkset();
+    s->keys.assign(keys, keys + n_keys);
+    for (auto* vk : s->keys) s->ns_max = std::max(s->ns_max, vk->n_ic - 1);
+    s->devs.resize(devs.size());
+    for (size_t j = 0; j < devs.size(); j++) {
+        SetDev& sd = s->devs[j];
+        sd.c = new DevCtx(); sd.c->device = devs[j]; s->ctxs.push_back(sd.c);
+        int rc = vkset_build_on(s, sd);
+        if (rc) { zkv_vkset_destroy(s); return rc; }
+    }
+    *out = s;
+    return 0;
+}
+// Slots of a pass of m records: each key present pads its group by at most 31 slots (a multiple of 32, so chunks keep whole warps)
+static size_t slot_bound(size_t m, size_t n_keys) { return (m + 31 * std::min(n_keys, m) + 31) / 32 * 32; }
+// One device pass of m records already in device memory (key_idx, 256-byte proofs, signal words with offsets relative to sig_base), enqueued
+// on c->stream; statuses in caller order to d_status.  Caller holds c->mu and has set the device.  Launches: 3 grouping kernels, decode,
+// signals, vk_x, G2 check, Miller loop, final exponentiation, status scatter = 10 for a pass of one chain; from chunk_count's threshold on,
+// + 1 (flag merge of the forked front) and 4 chunks x (4 Miller segments + 4 final-exponentiation stages) instead of 2: 41.
+static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t* d_key_idx, const uint8_t* d_proofs, const uint8_t* d_sig,
+                       const uint64_t* d_sig_off, uint64_t sig_base, uint8_t* d_status) {
+    DevCtx* c = sd->c;
+    cudaStream_t st = c->stream;
+    const int nk = (int)s->keys.size(), ns = s->ns_max;
+    const size_t S = slot_bound(m, (size_t)nk), ntiles = (m + ZKV_GROUP_TILE - 1) / ZKV_GROUP_TILE;
+    int rc = ctx_acquire(c, st); if (rc) return rc;
+    if (c->busy && (S > c->cap || S > c->fes_cap || S * (size_t)ns * 8 > c->scal_words || S > sd->slot_cap || ntiles * nk > sd->tile_cap)) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }
+    rc = ctx_reserve(c, S, (size_t)ns * 8); if (rc) return rc;
+    if (S > sd->slot_cap) {
+        cudaFree(sd->perm); cudaFree(sd->slot_key); cudaFree(sd->slot_status); sd->slot_cap = 0;
+        CK(cudaMalloc(&sd->perm, S * sizeof(uint32_t))); CK(cudaMalloc(&sd->slot_key, S)); CK(cudaMalloc(&sd->slot_status, S)); sd->slot_cap = S;
+    }
+    if (ntiles * nk > sd->tile_cap) { cudaFree(sd->tile); sd->tile_cap = 0; CK(cudaMalloc(&sd->tile, ntiles * nk * sizeof(uint32_t))); sd->tile_cap = ntiles * nk; }
+    CK(cudaMemsetAsync(sd->perm, 0xff, S * sizeof(uint32_t), st)); CK(cudaMemsetAsync(sd->slot_key, 0, S, st));
+    k_group_count<<<(int)ntiles, 256, 0, st>>>((int)m, nk, d_key_idx, sd->tile);
+    k_group_scan<<<1, ZKV_MAX_KEYS, 0, st>>>((int)ntiles, nk, sd->tile, sd->slot_key, sd->total);
+    k_group_scatter<<<(int)ntiles, 256, 0, st>>>((int)m, nk, d_key_idx, sd->tile, sd->perm, sd->slot_key);
+    const int n = (int)S;
+    uint8_t* flags = c->flags;
+    k_decode_keys<<<nblk(n), TPB, 0, st>>>(n, sd->perm, sd->slot_key, sd->d_keys, nk, d_key_idx, d_proofs, c->px[0], c->py[0], c->qx, c->qy, c->px[3], c->py[3], flags);
+    k_signals_keys<<<nblk(n), TPB, 0, st>>>(n, sd->perm, sd->slot_key, sd->d_keys, d_sig, d_sig_off, sig_base, ns, c->scal, flags);
+    const int chunks = chunk_count(c, S, 0);
+    int nl = 7;
+    if (chunks > 1) {                       // the front phase of run_verify's schedule: the G2 check beside vk_x, vk_x's flags merged afterwards
+        CK(cudaEventRecord(c->ev_fork, st)); CK(cudaStreamWaitEvent(c->aux[0], c->ev_fork, 0));
+        k_g2_check<<<nblk(n), TPB, 0, c->aux[0]>>>(n, c->qx, c->qy, flags);
+        CK(cudaMemsetAsync(c->status, 0, S, st));
+        k_vkx_keys<<<nblk(n), TPB, 0, st>>>(n, sd->perm, sd->slot_key, sd->d_keys, c->scal, ns, c->px[2], c->py[2], c->status);
+        CK(cudaEventRecord(c->ev_join[0], c->aux[0])); CK(cudaStreamWaitEvent(st, c->ev_join[0], 0));
+        k_or_flags<<<nblk(n, 256), 256, 0, st>>>(n, flags, c->status);
+        nl++;
+    } else {
+        k_vkx_keys<<<nblk(n), TPB, 0, st>>>(n, sd->perm, sd->slot_key, sd->d_keys, c->scal, ns, c->px[2], c->py[2], flags);
+        k_g2_check<<<nblk(n), TPB, 0, st>>>(n, c->qx, c->qy, flags);
+    }
+    auto heavy = [&](size_t o, int mm, cudaStream_t hs, int segs, bool staged) -> int {
+        MillerArgs a; memset(&a, 0, sizeof a);
+        a.px[0] = c->px[0] + o; a.py[0] = c->py[0] + o; a.px[1] = c->px[2] + o; a.py[1] = c->py[2] + o; a.px[2] = c->px[3] + o; a.py[2] = c->py[3] + o;
+        a.qx = c->qx + o; a.qy = c->qy + o; a.nfixed = 2;
+        a.skip_bit[0] = F_SKIP0; a.skip_bit[1] = F_SKIPX; a.skip_bit[2] = F_SKIPC;
+        const int top = ZKV_ATE_NAF_LEN - 2;
+        for (int k = 0; k < segs; k++) {
+            int hi = top - (top + 1) * k / segs, lo = top - (top + 1) * (k + 1) / segs + 1;
+            k_miller_lz_keys<<<nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_MILLER, hs>>>(sd->total, o, mm, a, sd->slot_key + o, sd->d_keys, flags + o, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == segs - 1);
+        }
+        if (staged) for (int q = 0; q < 4; q++) k_final_exp_lz_keys<<<nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs>>>(sd->total, o, mm, q, q, c->f + o, c->fes + 6 * o, flags + o, sd->slot_status + o);
+        else k_final_exp_lz_keys<<<nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs>>>(sd->total, o, mm, 0, 3, c->f + o, c->fes + 6 * o, flags + o, sd->slot_status + o);
+        nl += segs + (staged ? 4 : 1);
+        return 0;
+    };
+    if (chunks <= 1) rc = heavy(0, n, st, 1, false);
+    else rc = fork_join(c, st, S, chunks, [&](size_t o, int mm, cudaStream_t hs) { return heavy(o, mm, hs, 4, true); });
+    if (rc) return rc;
+    k_status_to_caller<<<nblk(n), TPB, 0, st>>>(n, sd->total, sd->perm, sd->slot_status, d_status);
+    g_launches += nl + 1;
+    CK(cudaGetLastError());
+    return 0;
+}
+extern "C" int zkv_groth16_verify_batch_keys(const zkv_vkset* s, const uint32_t* key_idx, const uint8_t* proofs, const uint8_t* signals,
+                                             const uint64_t* sig_off, size_t n, uint8_t* status_out) {
+    if (!s || (n && (!key_idx || !proofs || !sig_off || !status_out))) return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch_keys: null argument");
+    if (n == 0) return 0;
+    if (n > 0xffffffffull) return fail(ZKV_ERR_ARG, "batch too large");
+    for (size_t i = 0; i < n; i++) if (key_idx[i] >= s->keys.size()) return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch_keys: key index " + std::to_string(key_idx[i]) + " out of range");
+    if (!offsets_ok(sig_off, n)) return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch_keys: signal offsets must be non-decreasing");
+    const bool any_sig = sig_off[n] != sig_off[0];
+    if (any_sig && !signals) return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch_keys: null signals");
+    const bool direct = n >= 4096 && is_pinned(key_idx) && is_pinned(proofs) && is_pinned(sig_off) && (!any_sig || is_pinned(signals));   // page-locked caller arrays are uploaded in place
+    return for_each_device(s->ctxs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
+        SetDev* sd = set_dev(s, c->device);
+        if (c->busy) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }      // a host call blocks anyway: wait out an earlier asynchronous device call here
+        // A pass is grouped as a whole, so it is uploaded as a whole before its kernels run: [key_idx][signal offsets][proofs][signal words]
+        for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
+            const size_t m = std::min(MAX_CHUNK, e - s0), words = (size_t)(sig_off[s0 + m] - sig_off[s0]);
+            const size_t o_off = (m * 4 + 255) / 256 * 256, o_pr = o_off + ((m + 1) * 8 + 255) / 256 * 256, o_sig = o_pr + m * 256, bytes = o_sig + words * 32;
+            int rc = ctx_stage(c, bytes, m); if (rc) return rc;
+            Sink sk{direct ? nullptr : c->h_pin, c->d_in, c->stream, 0};
+            sk.put(0, key_idx + s0, m * 4, true); sk.put(o_off, sig_off + s0, (m + 1) * 8, true); sk.put(o_pr, proofs + s0 * 256, m * 256, true);
+            if (words) sk.put(o_sig, signals + sig_off[s0] * 32, words * 32, true);
+            if (sk.bad) return fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (page-locked caller memory to device)");
+            if (!direct) CK(cudaMemcpyAsync(c->d_in, c->h_pin, bytes, cudaMemcpyHostToDevice, c->stream));
+            rc = keyset_pass(s, sd, m, (const uint32_t*)c->d_in, c->d_in + o_pr, c->d_in + o_sig, (const uint64_t*)(c->d_in + o_off), sig_off[s0], c->d_out);
+            if (rc) return rc;
+            CK(cudaMemcpyAsync(c->h_out, c->d_out, m, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            memcpy(status_out + s0, c->h_out, m);
+        }
+        return 0;
+    });
+}
+extern "C" int zkv_groth16_verify_batch_keys_device(const zkv_vkset* s, int device, const void* d_key_idx, const void* d_proofs, const void* d_signals,
+                                                    const void* d_sig_off, size_t n, void* d_status_out, void* stream) {
+    if (!s || !d_key_idx || !d_proofs || !d_signals || !d_sig_off || !d_status_out) return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch_keys_device: null argument");
+    SetDev* sd = set_dev(s, device);
+    if (!sd) return fail(ZKV_ERR_ARG, "device not in the set's device list");
+    if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, "device batch too large");
+    if (n == 0) return 0;
+    DevCtx* c = sd->c;
+    std::lock_guard<std::mutex> lk(c->mu);
+    CK(cudaSetDevice(device));
+    cudaStream_t keep = c->stream; c->stream = (cudaStream_t)stream;          // NULL is the legacy default stream, as for any CUDA call
+    int rc = keyset_pass(s, sd, n, (const uint32_t*)d_key_idx, (const uint8_t*)d_proofs, (const uint8_t*)d_signals, (const uint64_t*)d_sig_off, 0, (uint8_t*)d_status_out);
+    if (!rc) rc = ctx_release_async(c, c->stream);
+    c->stream = keep;
+    return rc;
 }
 
 // ------------------------------------------------------------------------------------------ RISC Zero
@@ -651,7 +849,6 @@ extern "C" int zkv_risc0_get_bn254_control_id(const zkv_risc0* h, uint8_t out[32
 extern "C" int zkv_risc0_get_verifier_key_digest(const zkv_risc0* h, uint8_t out[32]) { if (!h || !out) return fail(ZKV_ERR_ARG, "null"); risc0_vk_digest(out, h->vk); return 0; }
 
 static uint32_t sel_le(const uint8_t s[4]) { return (uint32_t)s[0] | (uint32_t)s[1] << 8 | (uint32_t)s[2] << 16 | (uint32_t)s[3] << 24; }
-static bool offsets_ok(const uint64_t* off, size_t n) { for (size_t i = 0; i < n; i++) if (off[i + 1] < off[i]) return false; return true; }
 // Host-buffer batches upload the caller's arrays AS THEY ARE (four bulk copies per chunk into pinned staging: offsets, the two 32-byte
 // arrays, the seal bytes) and leave the front checks of verify_integrity_internal (risc0/verifier.rs:151-170) to k_decode; round 1
 // filtered and repacked proof by proof on the host, which cost 7 % of the end-to-end rate.
@@ -663,7 +860,7 @@ static int risc0_batch(const zkv_risc0* h, const uint8_t* seals, const uint64_t*
     if (!h->initialized) { memset(status_out, ZKV_INVALID_INITIALIZATION, n); return 0; }     // risc0/verifier.rs:84-86, 99-101
     const zkv_vk* vk = h->vk;
     const bool direct = n >= 4096 && is_pinned(seals) && is_pinned(seal_off) && is_pinned(a32) && (integrity || is_pinned(b32));      // page-locked caller arrays are uploaded in place
-    return for_each_device(vk, n, [&](DevCtx* c, size_t b, size_t e) -> int {
+    return for_each_device(vk->devs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
         for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
             size_t m = std::min(MAX_CHUNK, e - s0);
             const size_t per = integrity ? 32 : 64;
@@ -748,7 +945,7 @@ extern "C" int zkv_sp1_verify_batch(const zkv_sp1* h, const uint8_t* vkeys, cons
     if (!offsets_ok(proof_off, n) || !offsets_ok(pv_off, n)) return fail(ZKV_ERR_ARG, "proof / public-value offsets must be non-decreasing");
     const zkv_vk* vk = h->vk;
     const bool direct = n >= 4096 && is_pinned(proofs) && is_pinned(proof_off) && is_pinned(pv_off) && is_pinned(vkeys) && is_pinned(public_values);      // page-locked caller arrays are uploaded in place
-    return for_each_device(vk, n, [&](DevCtx* c, size_t b, size_t e) -> int {
+    return for_each_device(vk->devs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
         for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
             size_t m = std::min(MAX_CHUNK, e - s0);
             const size_t pvb = (size_t)(pv_off[s0 + m] - pv_off[s0]), prb = (size_t)(proof_off[s0 + m] - proof_off[s0]);
@@ -891,7 +1088,7 @@ extern "C" int zkv_pairing4_batch(const zkv_vk* vk, const uint8_t* g1s, const ui
     if (!vk || (n && (!g1s || !g2s || !ok_out))) return fail(ZKV_ERR_ARG, "zkv_pairing4_batch: null argument");
     if (n == 0) return 0;
     const size_t CH = (size_t)1 << 18;
-    return for_each_device(vk, n, [&](DevCtx* c, size_t b, size_t e) -> int {
+    return for_each_device(vk->devs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
         for (size_t s0 = b; s0 < e; s0 += CH) {
             size_t m = std::min(CH, e - s0);
             size_t ob = m + (gt_out ? m * 384 : 0) + (miller_out ? m * 384 : 0);

@@ -100,6 +100,31 @@ class VerificationKey:
         return _tune(self._h, option, value)
 
 
+class VerificationKeySet:
+    """1..256 loaded VerificationKeys for Groth16Verifier.verify_batch_keys (zkv_vkset_create).  Every key must be loaded on every
+    device of the set; the set keeps references to its keys so that they outlive it."""
+
+    def __init__(self, keys, devices=None):
+        self.keys = list(keys)
+        self._h = C.c_void_p()
+        handles = (C.c_void_p * max(len(self.keys), 1))(*[k._h for k in self.keys])
+        arr, nd = _dev_array(devices)
+        N.check(N.lib().zkv_vkset_create(handles, len(self.keys), arr, nd, C.byref(self._h)))
+
+    def __len__(self):
+        return len(self.keys)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            N.lib().zkv_vkset_destroy(self._h); self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class Groth16Verifier:
     """common/groth16.rs:16-49."""
 
@@ -117,6 +142,40 @@ class Groth16Verifier:
         st = np.zeros(n, dtype=np.uint8)
         N.check(N.lib().zkv_groth16_verify_batch(vk._h, N.buf(proofs), N.buf(signals) if k else None, k, n, st.ctypes.data))
         return st
+
+    @staticmethod
+    def verify_batch_keys(keyset, key_idx, proofs, signals):
+        """N verify_proof_with_key calls in one batch: proof i (256 B; `proofs` is one n x 256-byte blob or a list of 256-byte proofs) under
+        keyset.keys[key_idx[i]] with the integers signals[i] -> n status bytes.  A signal count other than that key's n_ic - 1 fails that proof."""
+        n = len(key_idx)
+        if len(signals) != n:
+            raise ValueError("signals: expected %d entries, got %d" % (n, len(signals)))
+        off = np.zeros(n + 1, dtype=np.uint64)
+        if n:
+            off[1:] = np.cumsum(np.fromiter((len(s) for s in signals), dtype=np.uint64, count=n))
+        blob = b"".join(int(v).to_bytes(32, "big") for s in signals for v in s)
+        return Groth16Verifier.verify_batch_keys_packed(keyset, key_idx, proofs if isinstance(proofs, (bytes, bytearray, np.ndarray)) else b"".join(proofs), blob, off)
+
+    @staticmethod
+    def verify_batch_keys_packed(keyset, key_idx, proofs, sig_blob, sig_off, status_out=None):
+        """Zero-copy form: key_idx (uint32), proofs n x 256 B, sig_blob = the signals as 32-byte words, sig_off = n + 1 uint64 word offsets."""
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        n = len(key_idx)
+        sig_off = np.ascontiguousarray(sig_off, dtype=np.uint64)
+        if (proofs.nbytes if isinstance(proofs, np.ndarray) else len(proofs)) != 256 * n:
+            raise ValueError("proofs: expected %d bytes" % (256 * n))
+        if len(sig_off) != n + 1:
+            raise ValueError("sig_off: expected %d offsets, got %d" % (n + 1, len(sig_off)))
+        st = status_out if status_out is not None else np.zeros(n, dtype=np.uint8)
+        N.check(N.lib().zkv_groth16_verify_batch_keys(keyset._h, key_idx.ctypes.data, N.buf(proofs) if n else None,
+                                                      N.buf(sig_blob) if len(sig_blob) else None, sig_off.ctypes.data, n, st.ctypes.data))
+        return st
+
+    @staticmethod
+    def verify_batch_keys_device(keyset, device, d_key_idx, d_proofs, d_signals, d_sig_off, n, d_status, stream=None):
+        """Inputs already in HBM (raw device pointers as ints: n uint32 key indices, n x 256-byte proofs, signal words, n + 1 uint64 offsets
+        into them); asynchronous on `stream`."""
+        N.check(N.lib().zkv_groth16_verify_batch_keys_device(keyset._h, device, d_key_idx, d_proofs, d_signals, d_sig_off, n, d_status, stream))
 
 
 class RiscZeroVerifier:
