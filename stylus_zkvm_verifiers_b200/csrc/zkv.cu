@@ -19,6 +19,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/zkv.h"
@@ -77,7 +78,7 @@ struct DevCtx {
     cudaEvent_t ev_fork = nullptr, ev_join[NAUX] = {};
     // The workspace above is shared by every call on this key and device.  Host-buffer calls return only when their work is done; the
     // *_device calls are asynchronous, so each records `ev_busy` behind its last kernel and every later user of the workspace, on whatever
-    // stream, first waits for it (ctx_acquire).
+    // stream, first waits for it (ctx_acquire); a host call, or a reserve about to free a buffer, waits for it on the host (ctx_wait_idle).
     cudaEvent_t ev_busy = nullptr; bool busy = false;
     std::mutex mu;
 };
@@ -91,7 +92,15 @@ struct Tuning {
     std::atomic<int> layout{1};             // 1: shared-memory-resident lazily reduced kernels (lazy.cuh); 0: the round-1 thread-stack kernels
 };
 static constexpr size_t PAD = 256;          // workspace slack behind a batch: surplus threads of the last block park their state there
+// wait on the host for the last asynchronous user of the workspace (caller holds c->mu)
+static int ctx_wait_idle(DevCtx* c) {
+    if (c->busy) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }
+    return 0;
+}
+// Grow the workspace to n proofs.  Growing frees buffers an earlier asynchronous call may still use, so it waits for that call first.
 static int ctx_reserve(DevCtx* c, size_t n, size_t scal_words_per_proof) {
+    size_t need = n * scal_words_per_proof;
+    if (n > c->cap || n > c->fes_cap || need > c->scal_words) { int rc = ctx_wait_idle(c); if (rc) return rc; }
     if (n > c->cap) {
         cudaFree(c->px[0]); cudaFree(c->py[0]); cudaFree(c->pskip);
         cudaFree(c->qx); cudaFree(c->qy); cudaFree(c->f); cudaFree(c->flags); cudaFree(c->status); cudaFree(c->rst); cudaFree(c->sl);
@@ -111,7 +120,6 @@ static int ctx_reserve(DevCtx* c, size_t n, size_t scal_words_per_proof) {
         cudaFree(c->fes); c->fes = nullptr; c->fes_cap = 0;
         CK(cudaMalloc(&c->fes, (n + PAD) * 6 * sizeof(fp12))); c->fes_cap = n;
     }
-    size_t need = n * scal_words_per_proof;
     if (need > c->scal_words) { cudaFree(c->scal); c->scal_words = 0; CK(cudaMalloc(&c->scal, need * 4)); c->scal_words = need; }
     return 0;
 }
@@ -125,6 +133,17 @@ static int ctx_stage(DevCtx* c, size_t in_bytes, size_t out_bytes) {
 // order stream `s` after the last asynchronous user of the workspace (caller holds c->mu)
 static int ctx_acquire(DevCtx* c, cudaStream_t s) { if (c->busy) CK(cudaStreamWaitEvent(s, c->ev_busy, 0)); return 0; }
 static int ctx_release_async(DevCtx* c, cudaStream_t s) { CK(cudaEventRecord(c->ev_busy, s)); c->busy = true; return 0; }
+// A *_device call: run(s) enqueues its work on the caller's stream s (NULL is the legacy default stream, as for any CUDA call), and later
+// users of the workspace are ordered behind it.
+template <class F>
+static int device_call(DevCtx* c, int device, void* stream, F run) {
+    std::lock_guard<std::mutex> lk(c->mu);
+    CK(cudaSetDevice(device));
+    cudaStream_t s = (cudaStream_t)stream;
+    int rc = run(s);
+    if (!rc) rc = ctx_release_async(c, s);
+    return rc;
+}
 static void ctx_free(DevCtx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
@@ -235,16 +254,16 @@ extern "C" int zkv_vk_load_sp1(const int* devices, int n_dev, zkv_vk** out) {
 // ------------------------------------------------------------------------------------------ the device pipeline
 enum SigMode { SIG_GENERIC, SIG_RISC0_VERIFY, SIG_RISC0_INTEGRITY, SIG_SP1 };
 struct Job {
-    const zkv_vk* vk; size_t n;
+    const zkv_vk* vk = nullptr; size_t n = 0;
     // proof records (device): rec i at recs + i*stride (or at recs + rec_off[i] - rec_base when rec_off is set: the caller's concatenated
     // blobs, front checks on the device), 8 x BE-32 at +off; selector (if any) in the first 4 bytes
-    const uint8_t* recs; size_t stride, off; int check_selector; uint32_t selector_le;
-    const uint64_t* rec_off; uint64_t rec_base, pv_base;
-    SigMode mode;
-    const uint8_t *sig_a, *sig_b;           // generic: signals | risc0: image_ids, journals (or claims) | sp1: vkeys, public values
-    const uint64_t* pv_off; size_t pv_stride; int k;
-    Risc0HashConsts hc; g1aff base; int all_fail;
-    uint8_t* d_status;
+    const uint8_t* recs = nullptr; size_t stride = 0, off = 0; int check_selector = 0; uint32_t selector_le = 0;
+    const uint64_t* rec_off = nullptr; uint64_t rec_base = 0, pv_base = 0;
+    SigMode mode = SIG_GENERIC;
+    const uint8_t *sig_a = nullptr, *sig_b = nullptr;     // generic: signals | risc0: image_ids, journals (or claims) | sp1: vkeys, public values
+    const uint64_t* pv_off = nullptr; size_t pv_stride = 0; int k = 0;
+    Risc0HashConsts hc = {}; g1aff base = {}; int all_fail = 0;
+    uint8_t* d_status = nullptr;
 };
 __global__ void k_status_all_fail(int n, const uint8_t* flags, uint8_t* status) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -252,6 +271,12 @@ __global__ void k_status_all_fail(int n, const uint8_t* flags, uint8_t* status) 
 }
 static std::atomic<unsigned long long> g_launches{0};   // kernels launched by the verification chains since load (bench.py's gpu_launches; a counter, not a setting)
 extern "C" unsigned long long zkv_launch_count(void) { return g_launches.load(); }
+// every kernel of a verification chain (enqueue_chain, keyset_pass) is launched through here, so the counter cannot miss one
+template <class... P, class... A>
+static void launch(void (*kernel)(P...), int grid, int block, size_t smem, cudaStream_t s, A&&... args) {
+    kernel<<<grid, block, smem, s>>>(std::forward<A>(args)...);
+    g_launches++;
+}
 extern "C" int zkv_vk_tune(const void* handle_vk, int option, int value) {
     const zkv_vk* vk = (const zkv_vk*)handle_vk;
     if (!vk) return fail(ZKV_ERR_ARG, "zkv_vk_tune: null key");
@@ -269,101 +294,110 @@ extern "C" int zkv_vk_tune(const void* handle_vk, int option, int value) {
     return f->exchange(value);
 }
 
-// the kernel chain for proofs [o, o+m) of job j on stream s; stage events only when `timed`
-// jo: offset of the first proof inside the job's buffers, o: offset inside the device workspace
 static const bool g_debug_sync = getenv("ZKV_DEBUG_SYNC") != nullptr;      // diagnostics: synchronise after every kernel of a chain and name the one that failed
 #define DBG(name) do { if (g_debug_sync) { cudaError_t e_ = cudaStreamSynchronize(s); if (e_ != cudaSuccess) return fail(ZKV_ERR_CUDA, std::string(name) + ": " + cudaGetErrorString(e_)); } } while (0)
+// The end of the front phase on workspace proofs [o, o+m): vk_x (vkx(flag array) enqueues it on s) and the G2 check.
+// fork: the front phase of a whole chunked batch on the call's main stream.  vk_x and the G2 check are independent (the check reads what the
+// decode kernel wrote, both touch disjoint flag bits of different proofs' bytes only through their own thread), and each is 1.7 waves of its
+// own block shape at 2^16 proofs: side by side on two streams they fill each other's partial waves.  F_SKIPX (vk_x = infinity) and F_INVALID
+// (B outside the subgroup) live in the same flag byte of a proof, so the two kernels must not write it concurrently: vk_x gets a flag array
+// of its own (the front-phase scratch c->status) that is OR-ed in by the G2 check's stream afterwards.
+template <class VkX>
+static int enqueue_vkx_g2(DevCtx* c, size_t o, int m, uint8_t* flags, cudaStream_t s, bool fork, bool timed, VkX vkx) {
+    if (fork) {
+        CK(cudaEventRecord(c->ev_fork, s)); CK(cudaStreamWaitEvent(c->aux[0], c->ev_fork, 0));
+        launch(k_g2_check, nblk(m), TPB, 0, c->aux[0], m, c->qx + o, c->qy + o, flags);
+        CK(cudaMemsetAsync(c->status + o, 0, m, s));
+        vkx(c->status + o);
+        CK(cudaEventRecord(c->ev_join[0], c->aux[0])); CK(cudaStreamWaitEvent(s, c->ev_join[0], 0));
+        launch(k_or_flags, nblk(m, 256), 256, 0, s, m, flags, c->status + o);
+        return 0;
+    }
+    vkx(flags);
+    if (timed) CK(cudaEventRecord(c->ev[2], s));
+    DBG("decode / signals / vk_x");
+    launch(k_g2_check, nblk(m), TPB, 0, s, m, c->qx + o, c->qy + o, flags);
+    DBG("k_g2_check");
+    if (timed) CK(cudaEventRecord(c->ev[3], s));
+    return 0;
+}
+// NAF digits hi .. lo (of top .. 0) that segment k of an S-segment Miller loop runs
+static std::pair<int, int> miller_segment(int k, int S) {
+    const int top = ZKV_ATE_NAF_LEN - 2;
+    return {top - (top + 1) * k / S, top - (top + 1) * (k + 1) / S + 1};
+}
+// MillerArgs of the verification path at workspace offset o: the pair (A, B), then (vk_x, gamma) and (C, delta) from tabled lines
+static MillerArgs verify_miller_args(const DevCtx* c, size_t o) {
+    MillerArgs a; memset(&a, 0, sizeof a);
+    a.px[0] = c->px[0] + o; a.py[0] = c->py[0] + o; a.px[1] = c->px[2] + o; a.py[1] = c->py[2] + o; a.px[2] = c->px[3] + o; a.py[2] = c->py[3] + o;
+    a.qx = c->qx + o; a.qy = c->qy + o; a.nfixed = 2;
+    a.skip_bit[0] = F_SKIP0; a.skip_bit[1] = F_SKIPX; a.skip_bit[2] = F_SKIPC;
+    return a;
+}
+// the kernel chain for proofs [o, o+m) of job j on stream s
+// jo: offset of the first proof inside the job's buffers, o: offset inside the device workspace
+// timed: record the per-stage events, and run the Miller loop and the final exponentiation as one launch each (no segments, no stages)
 // phases: 1 = the front kernels (decode, public-input hashing, vk_x, G2 check), 2 = the heavy ones (Miller loop, final exponentiation), 3 = both
-static int enqueue_chain(DevCtx* c, const Job& j, size_t jo, size_t o, int m, cudaStream_t s, bool timed, bool mono_kernels = false, int phases = 3) {
-    const bool mono = timed || mono_kernels;      // one-launch Miller loop / final exponentiation (no segments, no stages); `timed` also records the per-stage events
+// fork_front: phase 1 of a whole chunked batch on the call's main stream (enqueue_vkx_g2)
+static int enqueue_chain(DevCtx* c, const Job& j, size_t jo, size_t o, int m, cudaStream_t s, bool timed, int phases = 3, bool fork_front = false) {
     const zkv_vk* vk = j.vk;
     int ns = (j.mode == SIG_GENERIC) ? j.k : 2;
     uint32_t* scal = c->scal + o * (size_t)ns * 8;
     uint8_t* flags = c->flags + o;
     if (phases & 1) {
         if (timed) CK(cudaEventRecord(c->ev[0], s));
-        k_decode<<<nblk(m), TPB, 0, s>>>(m, j.rec_off ? j.recs : j.recs + jo * j.stride, j.stride, j.off, j.selector_le, j.check_selector, vk->vm, j.rec_off ? j.rec_off + jo : nullptr, j.rec_base, c->px[0] + o, c->py[0] + o, c->qx + o, c->qy + o, c->px[3] + o, c->py[3] + o, flags);
+        launch(k_decode, nblk(m), TPB, 0, s, m, j.rec_off ? j.recs : j.recs + jo * j.stride, j.stride, j.off, j.selector_le, j.check_selector, vk->vm, j.rec_off ? j.rec_off + jo : nullptr, j.rec_base, c->px[0] + o, c->py[0] + o, c->qx + o, c->qy + o, c->px[3] + o, c->py[3] + o, flags);
         const g1aff* tab = c->d_tab; int nwin = ZKV_WIN_PER_SCALAR;
         switch (j.mode) {
-            case SIG_GENERIC: k_generic_signals<<<nblk(m), TPB, 0, s>>>(m, j.k, j.sig_a + jo * (size_t)j.k * 32, scal, flags); break;
-            case SIG_RISC0_VERIFY: k_risc0_signals<<<nblk(m), TPB, 0, s>>>(m, j.sig_a + jo * 32, j.sig_b + jo * 32, nullptr, 0, j.hc, scal); break;
-            case SIG_RISC0_INTEGRITY: k_risc0_signals<<<nblk(m), TPB, 0, s>>>(m, nullptr, nullptr, j.sig_a + jo * 32, 1, j.hc, scal); break;
-            case SIG_SP1: k_sp1_signals<<<nblk(m), TPB, 0, s>>>(m, j.sig_a + jo * 32, j.pv_off ? j.sig_b : j.sig_b + jo * j.pv_stride, j.pv_off ? j.pv_off + jo : nullptr, j.pv_base, j.pv_stride, scal, flags); break;
+            case SIG_GENERIC: launch(k_generic_signals, nblk(m), TPB, 0, s, m, j.k, j.sig_a + jo * (size_t)j.k * 32, scal, flags); break;
+            case SIG_RISC0_VERIFY: launch(k_risc0_signals, nblk(m), TPB, 0, s, m, j.sig_a + jo * 32, j.sig_b + jo * 32, nullptr, 0, j.hc, scal); break;
+            case SIG_RISC0_INTEGRITY: launch(k_risc0_signals, nblk(m), TPB, 0, s, m, nullptr, nullptr, j.sig_a + jo * 32, 1, j.hc, scal); break;
+            case SIG_SP1: launch(k_sp1_signals, nblk(m), TPB, 0, s, m, j.sig_a + jo * 32, j.pv_off ? j.sig_b : j.sig_b + jo * j.pv_stride, j.pv_off ? j.pv_off + jo : nullptr, j.pv_base, j.pv_stride, scal, flags); break;
         }
         if (j.mode == SIG_RISC0_VERIFY || j.mode == SIG_RISC0_INTEGRITY) { tab = c->d_tab + (size_t)2 * ZKV_WIN_PER_SCALAR * ZKV_WIN_ENTRIES; nwin = 32; }   // claim_lo / claim_hi are 128-bit
         if (timed) CK(cudaEventRecord(c->ev[1], s));
         if (j.all_fail || !vk->valid) {
-            k_status_all_fail<<<nblk(m), TPB, 0, s>>>(m, flags, j.d_status + jo);
-            g_launches += 3;
+            launch(k_status_all_fail, nblk(m), TPB, 0, s, m, flags, j.d_status + jo);
             if (timed) for (int e = 2; e < 6; e++) CK(cudaEventRecord(c->ev[e], s));
             CK(cudaGetLastError());
             return 0;
         }
-        // Front phase of a whole chunked batch (run_verify): vk_x and the G2 check are independent (the check reads what k_decode wrote, both
-        // touch disjoint flag bits of different proofs' bytes only through their own thread), and each is 1.7 waves of its own block shape at 2^16
-        // proofs: side by side on two streams they fill each other's partial waves.  F_SKIPX (vk_x = infinity) and F_INVALID (B outside the
-        // subgroup) live in the same flag byte of a proof, so the two kernels must not write it concurrently: vk_x gets a flag array of its own
-        // (the front-phase scratch) that is OR-ed in by the G2 check's stream afterwards.
-        const bool fork_front = phases == 1 && !timed && s == c->stream && m >= 8192;
-        if (fork_front) {
-            CK(cudaEventRecord(c->ev_fork, s)); CK(cudaStreamWaitEvent(c->aux[0], c->ev_fork, 0));
-            k_g2_check<<<nblk(m), TPB, 0, c->aux[0]>>>(m, c->qx + o, c->qy + o, flags);
-            CK(cudaMemsetAsync(c->status + o, 0, m, s));
-            k_vkx<<<nblk(m), TPB, 0, s>>>(m, scal, ns, nwin, tab, j.base, c->px[2] + o, c->py[2] + o, c->status + o);
-            CK(cudaEventRecord(c->ev_join[0], c->aux[0])); CK(cudaStreamWaitEvent(s, c->ev_join[0], 0));
-            k_or_flags<<<nblk(m, 256), 256, 0, s>>>(m, flags, c->status + o);
-            g_launches += 1;
-        } else {
-            k_vkx<<<nblk(m), TPB, 0, s>>>(m, scal, ns, nwin, tab, j.base, c->px[2] + o, c->py[2] + o, flags);
-            if (timed) CK(cudaEventRecord(c->ev[2], s));
-            DBG("decode / signals / vk_x");
-            k_g2_check<<<nblk(m), TPB, 0, s>>>(m, c->qx + o, c->qy + o, flags);
-            DBG("k_g2_check");
-            if (timed) CK(cudaEventRecord(c->ev[3], s));
-        }
-        if (!(phases & 2)) { g_launches += 4; CK(cudaGetLastError()); return 0; }
+        int rc = enqueue_vkx_g2(c, o, m, flags, s, fork_front, timed, [&](uint8_t* fl) {
+            launch(k_vkx, nblk(m), TPB, 0, s, m, scal, ns, nwin, tab, j.base, c->px[2] + o, c->py[2] + o, fl);
+        });
+        if (rc) return rc;
+        if (!(phases & 2)) { CK(cudaGetLastError()); return 0; }
     }
-    MillerArgs a; memset(&a, 0, sizeof a);
-    a.px[0] = c->px[0] + o; a.py[0] = c->py[0] + o; a.px[1] = c->px[2] + o; a.py[1] = c->py[2] + o; a.px[2] = c->px[3] + o; a.py[2] = c->py[3] + o;
-    a.qx = c->qx + o; a.qy = c->qy + o;
-    a.tabs[0] = c->d_lines + 1 * ZKV_LINES_PER_G2; a.tabs[1] = c->d_lines + 2 * ZKV_LINES_PER_G2;
-    a.nfixed = 2; a.pre = c->d_pre;
+    MillerArgs a = verify_miller_args(c, o);
+    a.tabs[0] = c->d_lines + 1 * ZKV_LINES_PER_G2; a.tabs[1] = c->d_lines + 2 * ZKV_LINES_PER_G2; a.pre = c->d_pre;
     a.ntabs[0] = c->d_nlines; a.ntabs[1] = c->d_nlines + ZKV_LINES_PER_G2;
+    a.vk_skip = (uint8_t)((c->h_vk.g2_inf[1] ? 2 : 0) | (c->h_vk.g2_inf[2] ? 4 : 0));
     const bool norm = c->h_vk.norm_ok && vk->tune.normalised_lines.load();
     const bool lazy = norm && vk->tune.layout.load();
     const int segs = vk->tune.miller_segments.load(), stages = vk->tune.final_exp_stages.load();
-    int nl = (phases & 1) ? 4 : 0;          // decode, signals, vk_x, G2 check
-    a.skip_bit[0] = F_SKIP0; a.skip_bit[1] = F_SKIPX; a.skip_bit[2] = F_SKIPC;
-    a.vk_skip = (uint8_t)((c->h_vk.g2_inf[1] ? 2 : 0) | (c->h_vk.g2_inf[2] ? 4 : 0));
-    const int top = ZKV_ATE_NAF_LEN - 2;    // digits top .. 0 of the loop
     if (lazy) {                             // shared-memory-resident kernels (lazy.cuh): segments when chunked, one launch otherwise
-        const int S = (segs > 1 && !mono) ? segs : 1;
+        const int S = (segs > 1 && !timed) ? segs : 1;
         for (int k = 0; k < S; k++) {
-            int hi = top - (top + 1) * k / S, lo = top - (top + 1) * (k + 1) / S + 1;
-            k_miller_lz<<<nblk(m, LZ_NT), LZ_NT, LZ_SMEM_MILLER, s>>>(m, a, flags, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == S - 1);
+            auto [hi, lo] = miller_segment(k, S);
+            launch(k_miller_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_MILLER, s, m, a, flags, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == S - 1);
             DBG("k_miller_lz");
         }
-        nl += S - 1;
-    } else if (norm && segs > 1 && !mono) {      // a timed single chain (per-stage roofline pass, small batches) runs the one-kernel form
-        const int S = segs;
-        for (int k = 0; k < S; k++) {
-            int hi = top - (top + 1) * k / S, lo = top - (top + 1) * (k + 1) / S + 1;
-            k_miller_norm_seg<<<nblk(m, ZKV_HTPB_MILLER), ZKV_HTPB_MILLER, 0, s>>>(m, a, flags, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == S - 1);
+    } else if (norm && segs > 1 && !timed) {      // a timed single chain (per-stage roofline pass, small batches) runs the one-kernel form
+        for (int k = 0; k < segs; k++) {
+            auto [hi, lo] = miller_segment(k, segs);
+            launch(k_miller_norm_seg, nblk(m, ZKV_HTPB_MILLER), ZKV_HTPB_MILLER, 0, s, m, a, flags, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == segs - 1);
         }
-        nl += S - 1;
-    } else if (norm) k_miller_norm<<<nblk(m, ZKV_HTPB_MILLER), ZKV_HTPB_MILLER, 0, s>>>(m, a, flags, c->f + o);
-    else k_miller<<<nblk(m, ZKV_HTPB), ZKV_HTPB, 0, s>>>(m, a, flags, c->f + o);
+    } else if (norm) launch(k_miller_norm, nblk(m, ZKV_HTPB_MILLER), ZKV_HTPB_MILLER, 0, s, m, a, flags, c->f + o);
+    else launch(k_miller, nblk(m, ZKV_HTPB), ZKV_HTPB, 0, s, m, a, flags, c->f + o);
     if (timed) CK(cudaEventRecord(c->ev[4], s));
     if (vk->tune.layout.load()) {
-        if (stages && !mono) { for (int st = 0; st < 4; st++) k_final_exp_lz<<<nblk(m, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s>>>(m, st, st, c->f + o, c->fes + 6 * o, flags, j.d_status + jo, nullptr, 0); nl += 3; }
-        else k_final_exp_lz<<<nblk(m, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s>>>(m, 0, 3, c->f + o, c->fes + 6 * o, flags, j.d_status + jo, nullptr, 0);
-    } else if (stages && !mono) {
-        for (int st = 0; st < 4; st++) k_final_exp_stage<<<nblk(m, ZKV_HTPB_FE), ZKV_HTPB_FE, 0, s>>>(m, st, c->f + o, c->fes + 5 * o, flags, j.d_status + jo);
-        nl += 3;
-    } else k_final_exp<<<nblk(m, ZKV_HTPB_FE), ZKV_HTPB_FE, 0, s>>>(m, c->f + o, flags, j.d_status + jo, nullptr, 0);
+        if (stages && !timed) for (int st = 0; st < 4; st++) launch(k_final_exp_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s, m, st, st, c->f + o, c->fes + 6 * o, flags, j.d_status + jo, nullptr, 0);
+        else launch(k_final_exp_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s, m, 0, 3, c->f + o, c->fes + 6 * o, flags, j.d_status + jo, nullptr, 0);
+    } else if (stages && !timed) {
+        for (int st = 0; st < 4; st++) launch(k_final_exp_stage, nblk(m, ZKV_HTPB_FE), ZKV_HTPB_FE, 0, s, m, st, c->f + o, c->fes + 5 * o, flags, j.d_status + jo);
+    } else launch(k_final_exp, nblk(m, ZKV_HTPB_FE), ZKV_HTPB_FE, 0, s, m, c->f + o, flags, j.d_status + jo, nullptr, 0);
     DBG("final exponentiation");
     if (timed) CK(cudaEventRecord(c->ev[5], s));
-    g_launches += nl + 2;                   // + Miller loop (first or only kernel) + final exponentiation (first or only kernel)
     CK(cudaGetLastError());
     return 0;
 }
@@ -383,12 +417,15 @@ static int chunk_count(const DevCtx* c, size_t n, int setting) {
     if (setting >= 1) return setting;
     return n < wave_proofs_of(c) / 2 ? 1 : 4;
 }
+// Proofs per chunk when n proofs are cut into `chunks`: a multiple of the heavy kernels' block size, so no chunk carries a second partial block.
+static size_t chunk_size(size_t n, int chunks) {
+    size_t per = (n + chunks - 1) / chunks;
+    return (per + ZKV_HTPB - 1) / ZKV_HTPB * ZKV_HTPB;
+}
 // Fork `chunks` side streams off `main`, run fn(chunk_begin, chunk_len, stream) on them round-robin, join back into `main`.
-// Chunk boundaries are multiples of the heavy kernels' block size so no chunk carries a second partial block.
 template <class F>
 static int fork_join(DevCtx* c, cudaStream_t main, size_t n, int chunks, F fn) {
-    size_t per = (n + chunks - 1) / chunks;
-    per = (per + ZKV_HTPB - 1) / ZKV_HTPB * ZKV_HTPB;
+    const size_t per = chunk_size(n, chunks);
     CK(cudaEventRecord(c->ev_fork, main));
     int used = 0, k = 0;
     for (size_t o = 0; o < n; o += per, k++) {
@@ -399,19 +436,18 @@ static int fork_join(DevCtx* c, cudaStream_t main, size_t n, int chunks, F fn) {
     for (int a = 0; a < used; a++) { CK(cudaEventRecord(c->ev_join[a], c->aux[a])); CK(cudaStreamWaitEvent(main, c->ev_join[a], 0)); }
     return 0;
 }
-// enqueue all stages of one batch (asynchronous; completion is ordered on c->stream); caller holds c->mu and has set the device
-static int run_verify(DevCtx* c, const Job& j) {
+// enqueue all stages of one batch on stream s (asynchronous; completion is ordered on s); caller holds c->mu and has set the device
+static int run_verify(DevCtx* c, const Job& j, cudaStream_t s) {
     if (j.n == 0) return 0;
     int ns = (j.mode == SIG_GENERIC) ? j.k : 2;
-    int rc = ctx_acquire(c, c->stream); if (rc) return rc;
-    if (c->busy && (j.n > c->cap || j.n > c->fes_cap || j.n * (size_t)ns * 8 > c->scal_words)) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }   // growing frees buffers an earlier asynchronous call may still use
+    int rc = ctx_acquire(c, s); if (rc) return rc;
     rc = ctx_reserve(c, j.n, (size_t)ns * 8); if (rc) return rc;
     int chunks = chunk_count(c, j.n, j.vk->tune.overlap_chunks.load());
-    if (chunks <= 1) return enqueue_chain(c, j, 0, 0, (int)j.n, c->stream, true);
-    if (j.all_fail || !j.vk->valid) return enqueue_chain(c, j, 0, 0, (int)j.n, c->stream, false);
+    if (chunks <= 1) return enqueue_chain(c, j, 0, 0, (int)j.n, s, true);
+    if (j.all_fail || !j.vk->valid) return enqueue_chain(c, j, 0, 0, (int)j.n, s, false);
     // the front kernels run once over the whole batch (at their own full occupancy), only the heavy kernels are chunked over the side streams
-    rc = enqueue_chain(c, j, 0, 0, (int)j.n, c->stream, false, false, 1); if (rc) return rc;
-    return fork_join(c, c->stream, j.n, chunks, [&](size_t o, int m, cudaStream_t s) { return enqueue_chain(c, j, o, o, m, s, false, false, 2); });
+    rc = enqueue_chain(c, j, 0, 0, (int)j.n, s, false, 1, true); if (rc) return rc;
+    return fork_join(c, s, j.n, chunks, [&](size_t o, int m, cudaStream_t hs) { return enqueue_chain(c, j, o, o, m, hs, false, 2); });
 }
 static void collect_stage_ms(DevCtx* c);
 // memcpy of a large block by up to four threads (one thread moves 5 - 10 GB/s into pinned memory: a 45 MB piece would cost as much as a wave of kernels)
@@ -426,11 +462,11 @@ static void pcopy(void* dst, const void* src, size_t n) {
     for (auto& t : th) t.join();
 }
 
-// Host-buffer form of a batch on one device, pipelined: the batch is cut like run_verify cuts it, and every chunk gets its own
-// pack (into its slice of the pinned staging buffer) -> H2D -> kernel chain -> D2H on a side stream, so packing and copying chunk k+1
-// overlap the kernels of chunk k.  pack(first, count, dst) writes the chunk's input block and returns its size in bytes;
-// job(first, count, d_block) describes the chunk, with pointers into its device input block and d_status = c->d_out + first.
-// in_bytes: upper bound of the whole batch's input.  On return c->h_out[0..m) holds the status bytes.
+// Host-buffer form of proofs [b, e) on one device, in passes of up to MAX_CHUNK proofs, pipelined: a pass is cut like run_verify cuts a
+// batch, and every piece gets its own pack (into its slice of the pinned staging buffer) -> H2D -> kernel chain -> D2H on a side stream,
+// so packing and copying piece k+1 overlap the kernels of piece k.  pack(first, count, dst) writes the input block of proofs
+// [first, first + count) and returns its size in bytes; job(first, count, d_block) describes them, with pointers into their device input
+// block (host_pass fills in the key, the count and the status slice).  The status bytes go to status_out[b, e).
 // Where a piece's input block is assembled: in the pinned staging buffer (memcpy; large segments by several threads), or - when every source
 // array of the call already lives in page-locked memory (cudaHostAlloc / cudaHostRegister) - straight in device memory, one asynchronous
 // upload per segment from the caller's own arrays, with no host copy at all.
@@ -448,37 +484,32 @@ static bool is_pinned(const void* p) {
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
     return a.type == cudaMemoryTypeHost;
 }
+// one pass of proofs [s0, s0 + m); on return c->h_out[0..m) holds their status bytes
 template <class Pack, class MakeJob>
-static int host_pipeline(DevCtx* c, const zkv_vk* vk, size_t m, size_t in_bytes, int ns, Pack pack, MakeJob job, bool direct = false) {
-    if (c->busy) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }      // a host call blocks anyway: wait out an earlier asynchronous device call here
+static int host_pass(DevCtx* c, const zkv_vk* vk, size_t s0, size_t m, int ns, Pack& pack, MakeJob& job, bool direct) {
     int rc = ctx_reserve(c, m, (size_t)ns * 8); if (rc) return rc;
-    // Pieces of the batch, in upload order: `chunks` equal pieces (multiples of the heavy kernels' block size), each with its own side stream.
+    // Pieces of the pass, in upload order: `chunks` equal pieces (multiples of the heavy kernels' block size), each with its own side stream.
     // Every piece runs its front kernels first, side by side with the others', then the heavy ones (chunk_count above); with more pieces
     // than side streams (a forced setting) each piece simply runs its whole chain on stream k mod NAUX.
     struct Piece { size_t first, cnt; };
     std::vector<Piece> pcs;
-    int chunks = chunk_count(c, m, vk->tune.overlap_chunks.load());
-    {
-        size_t per = (m + chunks - 1) / chunks;
-        per = (per + ZKV_HTPB - 1) / ZKV_HTPB * ZKV_HTPB;
-        for (size_t f = 0; f < m; f += per) pcs.push_back({f, std::min(per, m - f)});
-    }
+    const size_t per = chunk_size(m, chunk_count(c, m, vk->tune.overlap_chunks.load()));
+    for (size_t f = 0; f < m; f += per) pcs.push_back({f, std::min(per, m - f)});
     const int np = (int)pcs.size();
     // pack(first, cnt, nullptr) returns the size of a piece's block, so every piece's region of the pinned staging buffer is known up front
     // and the pieces can be packed by concurrent host threads: piece 0 on this thread, the others on up to 6 helpers (helper h packs pieces
     // h + 1, h + 1 + H, ...); ready[k] flips when piece k's block is complete.  Packing is a handful of bulk memcpy per piece.
     std::vector<size_t> bytes(np, 0), offs(np + 1, 0);
-    for (int k = 0; k < np; k++) { bytes[k] = pack(pcs[k].first, pcs[k].cnt, (Sink*)nullptr); offs[k + 1] = offs[k] + (bytes[k] + 255) / 256 * 256; }
-    (void)in_bytes;
+    for (int k = 0; k < np; k++) { bytes[k] = pack(s0 + pcs[k].first, pcs[k].cnt, (Sink*)nullptr); offs[k + 1] = offs[k] + (bytes[k] + 255) / 256 * 256; }
     rc = ctx_stage(c, offs[np], m); if (rc) return rc;
     const int H = direct ? 0 : std::min(np - 1, 6);
     std::vector<std::atomic<int>> ready(np);
     for (auto& r : ready) r.store(direct ? 1 : 0);
     std::vector<std::thread> helpers;
     for (int h = 0; h < H; h++) helpers.emplace_back([&, h]() {
-        for (int k = h + 1; k < np; k += H) { Sink sk{c->h_pin + offs[k], nullptr, nullptr, 0}; pack(pcs[k].first, pcs[k].cnt, &sk); ready[k].store(1, std::memory_order_release); }
+        for (int k = h + 1; k < np; k += H) { Sink sk{c->h_pin + offs[k], nullptr, nullptr, 0}; pack(s0 + pcs[k].first, pcs[k].cnt, &sk); ready[k].store(1, std::memory_order_release); }
     });
-    if (!direct) { Sink sk{c->h_pin, nullptr, nullptr, 0}; pack(pcs[0].first, pcs[0].cnt, &sk); ready[0].store(1); }
+    if (!direct) { Sink sk{c->h_pin, nullptr, nullptr, 0}; pack(s0 + pcs[0].first, pcs[0].cnt, &sk); ready[0].store(1); }
     const bool split = np > 1 && np <= DevCtx::NAUX;
     std::vector<cudaEvent_t> evs;                    // front-done event per piece
     if (split) { evs.resize((size_t)np, nullptr); for (auto& e : evs) if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "cudaEventCreate"); }
@@ -486,25 +517,26 @@ static int host_pipeline(DevCtx* c, const zkv_vk* vk, size_t m, size_t in_bytes,
     auto kstream = [&](int k) { return np == 1 ? c->stream : c->aux[k % DevCtx::NAUX]; };
     for (int k = 0; k < np && !rc; k++) {
         const size_t first = pcs[k].first, cnt = pcs[k].cnt, in_off = offs[k];
-        cudaStream_t s = kstream(k), s_in = s, s_out = s;
+        cudaStream_t s = kstream(k);
         while (!ready[k].load(std::memory_order_acquire)) std::this_thread::yield();
-        if (direct) { Sink sk{nullptr, c->d_in + in_off, s_in, 0}; pack(first, cnt, &sk); rc = sk.bad ? fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (page-locked caller memory to device)") : 0; }
-        else rc = cudaMemcpyAsync(c->d_in + in_off, c->h_pin + in_off, bytes[k], cudaMemcpyHostToDevice, s_in) == cudaSuccess ? 0 : fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (host to device)");
+        if (direct) { Sink sk{nullptr, c->d_in + in_off, s, 0}; pack(s0 + first, cnt, &sk); rc = sk.bad ? fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (page-locked caller memory to device)") : 0; }
+        else rc = cudaMemcpyAsync(c->d_in + in_off, c->h_pin + in_off, bytes[k], cudaMemcpyHostToDevice, s) == cudaSuccess ? 0 : fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (host to device)");
         if (rc) break;
-        jobs[k] = job(first, cnt, c->d_in + in_off);
+        jobs[k] = job(s0 + first, cnt, c->d_in + in_off);
+        jobs[k].vk = vk; jobs[k].n = cnt; jobs[k].d_status = c->d_out + first;
         if (split && !(jobs[k].all_fail || !vk->valid)) {
-            rc = enqueue_chain(c, jobs[k], 0, first, (int)cnt, s, false, false, 1);
+            rc = enqueue_chain(c, jobs[k], 0, first, (int)cnt, s, false, 1);
             if (!rc && cudaEventRecord(evs[k], s) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "event (front done)");
             continue;
         }
         rc = enqueue_chain(c, jobs[k], 0, first, (int)cnt, s, np == 1);
-        if (!rc && cudaMemcpyAsync(c->h_out + first, c->d_out + first, cnt, cudaMemcpyDeviceToHost, s_out) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (device to host)");
+        if (!rc && cudaMemcpyAsync(c->h_out + first, c->d_out + first, cnt, cudaMemcpyDeviceToHost, s) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (device to host)");
     }
     for (int k = 0; split && k < np && !rc; k++) {
         if (jobs[k].all_fail || !vk->valid) continue;        // (that piece ran its whole chain above)
         cudaStream_t s = kstream(k);
         for (int o = 0; o < np && !rc; o++) if (o != k && !(jobs[o].all_fail || !vk->valid) && cudaStreamWaitEvent(s, evs[o], 0) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "event wait (front done)");
-        if (!rc) rc = enqueue_chain(c, jobs[k], 0, pcs[k].first, (int)pcs[k].cnt, s, false, false, 2);
+        if (!rc) rc = enqueue_chain(c, jobs[k], 0, pcs[k].first, (int)pcs[k].cnt, s, false, 2);
         if (!rc && cudaMemcpyAsync(c->h_out + pcs[k].first, c->d_out + pcs[k].first, pcs[k].cnt, cudaMemcpyDeviceToHost, s) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (device to host)");
     }
     for (auto& t : helpers) t.join();
@@ -513,6 +545,16 @@ static int host_pipeline(DevCtx* c, const zkv_vk* vk, size_t m, size_t in_bytes,
     else for (int a = 0; a < DevCtx::NAUX; a++) CK(cudaStreamSynchronize(c->aux[a]));
     for (auto e : evs) if (e) cudaEventDestroy(e);
     return 0;
+}
+template <class Pack, class MakeJob>
+static int host_pipeline(DevCtx* c, const zkv_vk* vk, size_t b, size_t e, int ns, uint8_t* status_out, Pack pack, MakeJob job, bool direct) {
+    int rc = ctx_wait_idle(c);      // a host call blocks anyway: wait out an earlier asynchronous device call here
+    for (size_t s0 = b; s0 < e && !rc; s0 += MAX_CHUNK) {
+        const size_t m = std::min(MAX_CHUNK, e - s0);
+        rc = host_pass(c, vk, s0, m, ns, pack, job, direct);
+        if (!rc) memcpy(status_out + s0, c->h_out, m);
+    }
+    return rc;
 }
 static void collect_stage_ms(DevCtx* c) {
     for (int e = 0; e < 5; e++) { float ms = 0; if (cudaEventElapsedTime(&ms, c->ev[e], c->ev[e + 1]) != cudaSuccess) { cudaGetLastError(); ms = 0; } c->stage_ms[e] = ms; }
@@ -553,22 +595,16 @@ extern "C" int zkv_groth16_verify_batch(const zkv_vk* vk, const uint8_t* proofs,
     if (k + 1 != vk->n_ic) { memset(status_out, ZKV_VERIFICATION_FAILED, n); return 0; }        // groth16.rs:32
     const bool direct = n >= 4096 && is_pinned(proofs) && (k == 0 || is_pinned(signals));      // page-locked caller arrays are uploaded in place
     return for_each_device(vk->devs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
-        for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
-            size_t m = std::min(MAX_CHUNK, e - s0);
-            int rc = host_pipeline(c, vk, m, m * (256 + (size_t)k * 32), k,
-                [&](size_t first, size_t cnt, Sink* dst) -> size_t {
-                    if (dst) { dst->put(0, proofs + (s0 + first) * 256, cnt * 256, true); dst->put(cnt * 256, signals + (s0 + first) * (size_t)k * 32, cnt * (size_t)k * 32, true); }
-                    return cnt * (256 + (size_t)k * 32);
-                },
-                [&](size_t first, size_t cnt, uint8_t* d) -> Job {
-                    Job j; memset(&j, 0, sizeof j);
-                    j.vk = vk; j.n = cnt; j.recs = d; j.stride = 256; j.off = 0; j.mode = SIG_GENERIC; j.sig_a = d + cnt * 256; j.k = k; j.base = c->h_ic0; j.d_status = c->d_out + first;
-                    return j;
-                }, direct);
-            if (rc) return rc;
-            memcpy(status_out + s0, c->h_out, m);
-        }
-        return 0;
+        return host_pipeline(c, vk, b, e, k, status_out,
+            [&](size_t first, size_t cnt, Sink* dst) -> size_t {
+                if (dst) { dst->put(0, proofs + first * 256, cnt * 256, true); dst->put(cnt * 256, signals + first * (size_t)k * 32, cnt * (size_t)k * 32, true); }
+                return cnt * (256 + (size_t)k * 32);
+            },
+            [&](size_t, size_t cnt, uint8_t* d) -> Job {
+                Job j;
+                j.recs = d; j.stride = 256; j.off = 0; j.mode = SIG_GENERIC; j.sig_a = d + cnt * 256; j.k = k; j.base = c->h_ic0;
+                return j;
+            }, direct);
     });
 }
 
@@ -650,66 +686,55 @@ extern "C" int zkv_vkset_create(const zkv_vk* const* keys, int n_keys, const int
 }
 // Slots of a pass of m records: each key present pads its group by at most 31 slots (a multiple of 32, so chunks keep whole warps)
 static size_t slot_bound(size_t m, size_t n_keys) { return (m + 31 * std::min(n_keys, m) + 31) / 32 * 32; }
-// One device pass of m records already in device memory (key_idx, 256-byte proofs, signal words with offsets relative to sig_base), enqueued
-// on c->stream; statuses in caller order to d_status.  Caller holds c->mu and has set the device.  Launches: 3 grouping kernels, decode,
-// signals, vk_x, G2 check, Miller loop, final exponentiation, status scatter = 10 for a pass of one chain; from chunk_count's threshold on,
-// + 1 (flag merge of the forked front) and 4 chunks x (4 Miller segments + 4 final-exponentiation stages) instead of 2: 41.
-static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t* d_key_idx, const uint8_t* d_proofs, const uint8_t* d_sig,
-                       const uint64_t* d_sig_off, uint64_t sig_base, uint8_t* d_status) {
-    DevCtx* c = sd->c;
-    cudaStream_t st = c->stream;
-    const int nk = (int)s->keys.size(), ns = s->ns_max;
-    const size_t S = slot_bound(m, (size_t)nk), ntiles = (m + ZKV_GROUP_TILE - 1) / ZKV_GROUP_TILE;
-    int rc = ctx_acquire(c, st); if (rc) return rc;
-    if (c->busy && (S > c->cap || S > c->fes_cap || S * (size_t)ns * 8 > c->scal_words || S > sd->slot_cap || ntiles * nk > sd->tile_cap)) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }
-    rc = ctx_reserve(c, S, (size_t)ns * 8); if (rc) return rc;
+// Grow the set's grouping arrays to S slots and ntk per-tile counters; like ctx_reserve, it waits for an asynchronous user before freeing.
+static int set_reserve(SetDev* sd, size_t S, size_t ntk) {
+    if (S > sd->slot_cap || ntk > sd->tile_cap) { int rc = ctx_wait_idle(sd->c); if (rc) return rc; }
     if (S > sd->slot_cap) {
         cudaFree(sd->perm); cudaFree(sd->slot_key); cudaFree(sd->slot_status); sd->slot_cap = 0;
         CK(cudaMalloc(&sd->perm, S * sizeof(uint32_t))); CK(cudaMalloc(&sd->slot_key, S)); CK(cudaMalloc(&sd->slot_status, S)); sd->slot_cap = S;
     }
-    if (ntiles * nk > sd->tile_cap) { cudaFree(sd->tile); sd->tile_cap = 0; CK(cudaMalloc(&sd->tile, ntiles * nk * sizeof(uint32_t))); sd->tile_cap = ntiles * nk; }
+    if (ntk > sd->tile_cap) { cudaFree(sd->tile); sd->tile_cap = 0; CK(cudaMalloc(&sd->tile, ntk * sizeof(uint32_t))); sd->tile_cap = ntk; }
+    return 0;
+}
+// One device pass of m records already in device memory (key_idx, 256-byte proofs, signal words with offsets relative to sig_base), enqueued
+// on stream st; statuses in caller order to d_status.  Caller holds c->mu and has set the device.  Launches: 3 grouping kernels, decode,
+// signals, vk_x, G2 check, Miller loop, final exponentiation, status scatter = 10 for a pass of one chain; from chunk_count's threshold on,
+// + 1 (flag merge of the forked front) and 4 chunks x (4 Miller segments + 4 final-exponentiation stages) instead of 2: 41.
+static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t* d_key_idx, const uint8_t* d_proofs, const uint8_t* d_sig,
+                       const uint64_t* d_sig_off, uint64_t sig_base, uint8_t* d_status, cudaStream_t st) {
+    DevCtx* c = sd->c;
+    const int nk = (int)s->keys.size(), ns = s->ns_max;
+    const size_t S = slot_bound(m, (size_t)nk), ntiles = (m + ZKV_GROUP_TILE - 1) / ZKV_GROUP_TILE;
+    int rc = ctx_acquire(c, st); if (rc) return rc;
+    rc = ctx_reserve(c, S, (size_t)ns * 8); if (rc) return rc;
+    rc = set_reserve(sd, S, ntiles * nk); if (rc) return rc;
     CK(cudaMemsetAsync(sd->perm, 0xff, S * sizeof(uint32_t), st)); CK(cudaMemsetAsync(sd->slot_key, 0, S, st));
-    k_group_count<<<(int)ntiles, 256, 0, st>>>((int)m, nk, d_key_idx, sd->tile);
-    k_group_scan<<<1, ZKV_MAX_KEYS, 0, st>>>((int)ntiles, nk, sd->tile, sd->slot_key, sd->total);
-    k_group_scatter<<<(int)ntiles, 256, 0, st>>>((int)m, nk, d_key_idx, sd->tile, sd->perm, sd->slot_key);
+    launch(k_group_count, (int)ntiles, 256, 0, st, (int)m, nk, d_key_idx, sd->tile);
+    launch(k_group_scan, 1, ZKV_MAX_KEYS, 0, st, (int)ntiles, nk, sd->tile, sd->slot_key, sd->total);
+    launch(k_group_scatter, (int)ntiles, 256, 0, st, (int)m, nk, d_key_idx, sd->tile, sd->perm, sd->slot_key);
     const int n = (int)S;
     uint8_t* flags = c->flags;
-    k_decode_keys<<<nblk(n), TPB, 0, st>>>(n, sd->perm, sd->slot_key, sd->d_keys, nk, d_key_idx, d_proofs, c->px[0], c->py[0], c->qx, c->qy, c->px[3], c->py[3], flags);
-    k_signals_keys<<<nblk(n), TPB, 0, st>>>(n, sd->perm, sd->slot_key, sd->d_keys, d_sig, d_sig_off, sig_base, ns, c->scal, flags);
+    launch(k_decode_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, nk, d_key_idx, d_proofs, c->px[0], c->py[0], c->qx, c->qy, c->px[3], c->py[3], flags);
+    launch(k_signals_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, d_sig, d_sig_off, sig_base, ns, c->scal, flags);
     const int chunks = chunk_count(c, S, 0);
-    int nl = 7;
-    if (chunks > 1) {                       // the front phase of run_verify's schedule: the G2 check beside vk_x, vk_x's flags merged afterwards
-        CK(cudaEventRecord(c->ev_fork, st)); CK(cudaStreamWaitEvent(c->aux[0], c->ev_fork, 0));
-        k_g2_check<<<nblk(n), TPB, 0, c->aux[0]>>>(n, c->qx, c->qy, flags);
-        CK(cudaMemsetAsync(c->status, 0, S, st));
-        k_vkx_keys<<<nblk(n), TPB, 0, st>>>(n, sd->perm, sd->slot_key, sd->d_keys, c->scal, ns, c->px[2], c->py[2], c->status);
-        CK(cudaEventRecord(c->ev_join[0], c->aux[0])); CK(cudaStreamWaitEvent(st, c->ev_join[0], 0));
-        k_or_flags<<<nblk(n, 256), 256, 0, st>>>(n, flags, c->status);
-        nl++;
-    } else {
-        k_vkx_keys<<<nblk(n), TPB, 0, st>>>(n, sd->perm, sd->slot_key, sd->d_keys, c->scal, ns, c->px[2], c->py[2], flags);
-        k_g2_check<<<nblk(n), TPB, 0, st>>>(n, c->qx, c->qy, flags);
-    }
+    rc = enqueue_vkx_g2(c, 0, n, flags, st, chunks > 1, false, [&](uint8_t* fl) {   // forked when chunked: the front phase of run_verify's schedule
+        launch(k_vkx_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, c->scal, ns, c->px[2], c->py[2], fl);
+    });
+    if (rc) return rc;
     auto heavy = [&](size_t o, int mm, cudaStream_t hs, int segs, bool staged) -> int {
-        MillerArgs a; memset(&a, 0, sizeof a);
-        a.px[0] = c->px[0] + o; a.py[0] = c->py[0] + o; a.px[1] = c->px[2] + o; a.py[1] = c->py[2] + o; a.px[2] = c->px[3] + o; a.py[2] = c->py[3] + o;
-        a.qx = c->qx + o; a.qy = c->qy + o; a.nfixed = 2;
-        a.skip_bit[0] = F_SKIP0; a.skip_bit[1] = F_SKIPX; a.skip_bit[2] = F_SKIPC;
-        const int top = ZKV_ATE_NAF_LEN - 2;
+        const MillerArgs a = verify_miller_args(c, o);
         for (int k = 0; k < segs; k++) {
-            int hi = top - (top + 1) * k / segs, lo = top - (top + 1) * (k + 1) / segs + 1;
-            k_miller_lz_keys<<<nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_MILLER, hs>>>(sd->total, o, mm, a, sd->slot_key + o, sd->d_keys, flags + o, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == segs - 1);
+            auto [hi, lo] = miller_segment(k, segs);
+            launch(k_miller_lz_keys, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_MILLER, hs, sd->total, o, mm, a, sd->slot_key + o, sd->d_keys, flags + o, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == segs - 1);
         }
-        if (staged) for (int q = 0; q < 4; q++) k_final_exp_lz_keys<<<nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs>>>(sd->total, o, mm, q, q, c->f + o, c->fes + 6 * o, flags + o, sd->slot_status + o);
-        else k_final_exp_lz_keys<<<nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs>>>(sd->total, o, mm, 0, 3, c->f + o, c->fes + 6 * o, flags + o, sd->slot_status + o);
-        nl += segs + (staged ? 4 : 1);
+        if (staged) for (int q = 0; q < 4; q++) launch(k_final_exp_lz_keys, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs, sd->total, o, mm, q, q, c->f + o, c->fes + 6 * o, flags + o, sd->slot_status + o);
+        else launch(k_final_exp_lz_keys, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs, sd->total, o, mm, 0, 3, c->f + o, c->fes + 6 * o, flags + o, sd->slot_status + o);
         return 0;
     };
     if (chunks <= 1) rc = heavy(0, n, st, 1, false);
     else rc = fork_join(c, st, S, chunks, [&](size_t o, int mm, cudaStream_t hs) { return heavy(o, mm, hs, 4, true); });
     if (rc) return rc;
-    k_status_to_caller<<<nblk(n), TPB, 0, st>>>(n, sd->total, sd->perm, sd->slot_status, d_status);
-    g_launches += nl + 1;
+    launch(k_status_to_caller, nblk(n), TPB, 0, st, n, sd->total, sd->perm, sd->slot_status, d_status);
     CK(cudaGetLastError());
     return 0;
 }
@@ -725,7 +750,7 @@ extern "C" int zkv_groth16_verify_batch_keys(const zkv_vkset* s, const uint32_t*
     const bool direct = n >= 4096 && is_pinned(key_idx) && is_pinned(proofs) && is_pinned(sig_off) && (!any_sig || is_pinned(signals));   // page-locked caller arrays are uploaded in place
     return for_each_device(s->ctxs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
         SetDev* sd = set_dev(s, c->device);
-        if (c->busy) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }      // a host call blocks anyway: wait out an earlier asynchronous device call here
+        if (int rc = ctx_wait_idle(c)) return rc;      // a host call blocks anyway: wait out an earlier asynchronous device call here
         // A pass is grouped as a whole, so it is uploaded as a whole before its kernels run: [key_idx][signal offsets][proofs][signal words]
         for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
             const size_t m = std::min(MAX_CHUNK, e - s0), words = (size_t)(sig_off[s0 + m] - sig_off[s0]);
@@ -736,7 +761,7 @@ extern "C" int zkv_groth16_verify_batch_keys(const zkv_vkset* s, const uint32_t*
             if (words) sk.put(o_sig, signals + sig_off[s0] * 32, words * 32, true);
             if (sk.bad) return fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (page-locked caller memory to device)");
             if (!direct) CK(cudaMemcpyAsync(c->d_in, c->h_pin, bytes, cudaMemcpyHostToDevice, c->stream));
-            rc = keyset_pass(s, sd, m, (const uint32_t*)c->d_in, c->d_in + o_pr, c->d_in + o_sig, (const uint64_t*)(c->d_in + o_off), sig_off[s0], c->d_out);
+            rc = keyset_pass(s, sd, m, (const uint32_t*)c->d_in, c->d_in + o_pr, c->d_in + o_sig, (const uint64_t*)(c->d_in + o_off), sig_off[s0], c->d_out, c->stream);
             if (rc) return rc;
             CK(cudaMemcpyAsync(c->h_out, c->d_out, m, cudaMemcpyDeviceToHost, c->stream));
             CK(cudaStreamSynchronize(c->stream));
@@ -752,14 +777,9 @@ extern "C" int zkv_groth16_verify_batch_keys_device(const zkv_vkset* s, int devi
     if (!sd) return fail(ZKV_ERR_ARG, "device not in the set's device list");
     if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, "device batch too large");
     if (n == 0) return 0;
-    DevCtx* c = sd->c;
-    std::lock_guard<std::mutex> lk(c->mu);
-    CK(cudaSetDevice(device));
-    cudaStream_t keep = c->stream; c->stream = (cudaStream_t)stream;          // NULL is the legacy default stream, as for any CUDA call
-    int rc = keyset_pass(s, sd, n, (const uint32_t*)d_key_idx, (const uint8_t*)d_proofs, (const uint8_t*)d_signals, (const uint64_t*)d_sig_off, 0, (uint8_t*)d_status_out);
-    if (!rc) rc = ctx_release_async(c, c->stream);
-    c->stream = keep;
-    return rc;
+    return device_call(sd->c, device, stream, [&](cudaStream_t st) {
+        return keyset_pass(s, sd, n, (const uint32_t*)d_key_idx, (const uint8_t*)d_proofs, (const uint8_t*)d_signals, (const uint64_t*)d_sig_off, 0, (uint8_t*)d_status_out, st);
+    });
 }
 
 // ------------------------------------------------------------------------------------------ RISC Zero
@@ -815,8 +835,8 @@ extern "C" int zkv_risc0_initialize(zkv_risc0* h, const uint8_t control_root[32]
     {
         std::lock_guard<std::mutex> lk(c->mu);
         CK(cudaSetDevice(c->device));
-        if (c->busy) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }
-        int rc = ctx_reserve(c, 1, 24); if (rc) return rc;
+        int rc = ctx_wait_idle(c); if (rc) return rc;
+        rc = ctx_reserve(c, 1, 24); if (rc) return rc;
         uint32_t sc[24]; memset(sc, 0, sizeof sc);
         uint8_t w32[32];
         memset(w32, 0, 32); memcpy(w32 + 16, h->control_root_0, 16); for (int k = 0; k < 8; k++) sc[k] = load_be32(w32 + 4 * (7 - k));
@@ -860,35 +880,28 @@ static int risc0_batch(const zkv_risc0* h, const uint8_t* seals, const uint64_t*
     if (!h->initialized) { memset(status_out, ZKV_INVALID_INITIALIZATION, n); return 0; }     // risc0/verifier.rs:84-86, 99-101
     const zkv_vk* vk = h->vk;
     const bool direct = n >= 4096 && is_pinned(seals) && is_pinned(seal_off) && is_pinned(a32) && (integrity || is_pinned(b32));      // page-locked caller arrays are uploaded in place
+    const size_t per = integrity ? 32 : 64;
     return for_each_device(vk->devs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
-        for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
-            size_t m = std::min(MAX_CHUNK, e - s0);
-            const size_t per = integrity ? 32 : 64;
-            const size_t blob = (size_t)(seal_off[s0 + m] - seal_off[s0]);
-            // chunk block layout: [offsets (cnt + 1) x 8][a32 cnt x 32][b32 cnt x 32][seal bytes][slack: k_decode never reads past a record's own length]
-            int rc = host_pipeline(c, vk, m, blob + m * (8 + per) + 64 * 8 + 64 * 320, 2,
-                [&](size_t first, size_t cnt, Sink* dst) -> size_t {
-                    const size_t i0 = s0 + first, bytes = (size_t)(seal_off[i0 + cnt] - seal_off[i0]);
-                    if (!dst) return (cnt + 1) * 8 + cnt * per + bytes + 320;
-                    size_t p = 0;
-                    dst->put(p, seal_off + i0, (cnt + 1) * 8); p += (cnt + 1) * 8;
-                    dst->put(p, a32 + i0 * 32, cnt * 32); p += cnt * 32;
-                    if (!integrity) { dst->put(p, b32 + i0 * 32, cnt * 32); p += cnt * 32; }
-                    dst->put(p, seals + seal_off[i0], bytes, true); p += bytes;
-                    return p + 320;
-                },
-                [&](size_t first, size_t cnt, uint8_t* d) -> Job {
-                    Job j; memset(&j, 0, sizeof j);
-                    j.vk = vk; j.n = cnt; j.rec_off = (const uint64_t*)d; j.rec_base = seal_off[s0 + first]; j.off = 4; j.stride = 260; j.check_selector = 1; j.selector_le = sel_le(h->selector);
-                    j.mode = integrity ? SIG_RISC0_INTEGRITY : SIG_RISC0_VERIFY;
-                    j.sig_a = d + (cnt + 1) * 8; j.sig_b = j.sig_a + cnt * 32; j.recs = j.sig_a + cnt * per;
-                    j.hc = h->hc; j.base = h->base; j.all_fail = h->all_fail; j.d_status = c->d_out + first;
-                    return j;
-                }, direct);
-            if (rc) return rc;
-            memcpy(status_out + s0, c->h_out, m);
-        }
-        return 0;
+        // piece block layout: [offsets (cnt + 1) x 8][a32 cnt x 32][b32 cnt x 32][seal bytes][slack: k_decode never reads past a record's own length]
+        return host_pipeline(c, vk, b, e, 2, status_out,
+            [&](size_t i0, size_t cnt, Sink* dst) -> size_t {
+                const size_t bytes = (size_t)(seal_off[i0 + cnt] - seal_off[i0]);
+                if (!dst) return (cnt + 1) * 8 + cnt * per + bytes + 320;
+                size_t p = 0;
+                dst->put(p, seal_off + i0, (cnt + 1) * 8); p += (cnt + 1) * 8;
+                dst->put(p, a32 + i0 * 32, cnt * 32); p += cnt * 32;
+                if (!integrity) { dst->put(p, b32 + i0 * 32, cnt * 32); p += cnt * 32; }
+                dst->put(p, seals + seal_off[i0], bytes, true); p += bytes;
+                return p + 320;
+            },
+            [&](size_t i0, size_t cnt, uint8_t* d) -> Job {
+                Job j;
+                j.rec_off = (const uint64_t*)d; j.rec_base = seal_off[i0]; j.off = 4; j.stride = 260; j.check_selector = 1; j.selector_le = sel_le(h->selector);
+                j.mode = integrity ? SIG_RISC0_INTEGRITY : SIG_RISC0_VERIFY;
+                j.sig_a = d + (cnt + 1) * 8; j.sig_b = j.sig_a + cnt * 32; j.recs = j.sig_a + cnt * per;
+                j.hc = h->hc; j.base = h->base; j.all_fail = h->all_fail;
+                return j;
+            }, direct);
     });
 }
 extern "C" int zkv_risc0_verify_batch(const zkv_risc0* h, const uint8_t* seals, const uint64_t* seal_off, const uint8_t* image_ids, const uint8_t* journal_digests, size_t n, uint8_t* status_out) {
@@ -909,19 +922,17 @@ extern "C" int zkv_risc0_verify_batch_device(const zkv_risc0* h, int device, con
     if (!h || !d_seals260 || !d_image_ids || !d_journal_digests || !d_status_out) return fail(ZKV_ERR_ARG, "zkv_risc0_verify_batch_device: null argument");
     DevCtx* c = vk_ctx(h->vk, device);
     if (!c) return fail(ZKV_ERR_ARG, "device not in the handle's device list");
-    std::lock_guard<std::mutex> lk(c->mu);
-    CK(cudaSetDevice(device));
     if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, "device batch too large");
-    if (!h->initialized) { CK(cudaMemsetAsync(d_status_out, ZKV_INVALID_INITIALIZATION, n, (cudaStream_t)stream)); return 0; }
-    Job j; memset(&j, 0, sizeof j);
+    if (!h->initialized) {      // no kernel, no use of the workspace
+        CK(cudaSetDevice(device));
+        CK(cudaMemsetAsync(d_status_out, ZKV_INVALID_INITIALIZATION, n, (cudaStream_t)stream));
+        return 0;
+    }
+    Job j;
     j.vk = h->vk; j.n = n; j.recs = (const uint8_t*)d_seals260; j.stride = 260; j.off = 4; j.check_selector = 1; j.selector_le = sel_le(h->selector);
     j.mode = SIG_RISC0_VERIFY; j.sig_a = (const uint8_t*)d_image_ids; j.sig_b = (const uint8_t*)d_journal_digests; j.hc = h->hc; j.base = h->base; j.all_fail = h->all_fail;
     j.d_status = (uint8_t*)d_status_out;
-    cudaStream_t keep = c->stream; c->stream = (cudaStream_t)stream;          // NULL is the legacy default stream, as for any CUDA call
-    int rc = run_verify(c, j);
-    if (!rc) rc = ctx_release_async(c, c->stream);
-    c->stream = keep;
-    return rc;
+    return device_call(c, device, stream, [&](cudaStream_t s) { return run_verify(c, j, s); });
 }
 
 // ------------------------------------------------------------------------------------------ SP1
@@ -946,35 +957,27 @@ extern "C" int zkv_sp1_verify_batch(const zkv_sp1* h, const uint8_t* vkeys, cons
     const zkv_vk* vk = h->vk;
     const bool direct = n >= 4096 && is_pinned(proofs) && is_pinned(proof_off) && is_pinned(pv_off) && is_pinned(vkeys) && is_pinned(public_values);      // page-locked caller arrays are uploaded in place
     return for_each_device(vk->devs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
-        for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
-            size_t m = std::min(MAX_CHUNK, e - s0);
-            const size_t pvb = (size_t)(pv_off[s0 + m] - pv_off[s0]), prb = (size_t)(proof_off[s0 + m] - proof_off[s0]);
-            // chunk block layout: [proof offsets (cnt + 1) x 8][public-value offsets (cnt + 1) x 8][vkeys cnt x 32][proof bytes][public values][slack]
-            int rc = host_pipeline(c, vk, m, prb + pvb + m * (16 + 32) + 64 * 16 + 64 * 320, 2,
-                [&](size_t first, size_t cnt, Sink* dst) -> size_t {
-                    const size_t i0 = s0 + first, pr = (size_t)(proof_off[i0 + cnt] - proof_off[i0]), pv = (size_t)(pv_off[i0 + cnt] - pv_off[i0]);
-                    if (!dst) return (cnt + 1) * 16 + cnt * 32 + pr + pv + 320;
-                    size_t p = 0;
-                    dst->put(p, proof_off + i0, (cnt + 1) * 8); p += (cnt + 1) * 8;
-                    dst->put(p, pv_off + i0, (cnt + 1) * 8); p += (cnt + 1) * 8;
-                    dst->put(p, vkeys + i0 * 32, cnt * 32); p += cnt * 32;
-                    dst->put(p, proofs + proof_off[i0], pr, true); p += pr;
-                    dst->put(p, public_values + pv_off[i0], pv, true); p += pv;
-                    return p + 320;
-                },
-                [&](size_t first, size_t cnt, uint8_t* d) -> Job {
-                    const size_t i0 = s0 + first;
-                    Job j; memset(&j, 0, sizeof j);
-                    j.vk = vk; j.n = cnt; j.rec_off = (const uint64_t*)d; j.rec_base = proof_off[i0]; j.off = 4; j.stride = 260; j.check_selector = 1; j.selector_le = sel_le(h->verifier_hash);
-                    j.mode = SIG_SP1; j.pv_off = (const uint64_t*)(d + (cnt + 1) * 8); j.pv_base = pv_off[i0];
-                    j.sig_a = d + (cnt + 1) * 16; j.recs = j.sig_a + cnt * 32; j.sig_b = j.recs + (size_t)(proof_off[i0 + cnt] - proof_off[i0]);
-                    j.base = c->h_ic0; j.d_status = c->d_out + first;
-                    return j;
-                }, direct);
-            if (rc) return rc;
-            memcpy(status_out + s0, c->h_out, m);
-        }
-        return 0;
+        // piece block layout: [proof offsets (cnt + 1) x 8][public-value offsets (cnt + 1) x 8][vkeys cnt x 32][proof bytes][public values][slack]
+        return host_pipeline(c, vk, b, e, 2, status_out,
+            [&](size_t i0, size_t cnt, Sink* dst) -> size_t {
+                const size_t pr = (size_t)(proof_off[i0 + cnt] - proof_off[i0]), pv = (size_t)(pv_off[i0 + cnt] - pv_off[i0]);
+                if (!dst) return (cnt + 1) * 16 + cnt * 32 + pr + pv + 320;
+                size_t p = 0;
+                dst->put(p, proof_off + i0, (cnt + 1) * 8); p += (cnt + 1) * 8;
+                dst->put(p, pv_off + i0, (cnt + 1) * 8); p += (cnt + 1) * 8;
+                dst->put(p, vkeys + i0 * 32, cnt * 32); p += cnt * 32;
+                dst->put(p, proofs + proof_off[i0], pr, true); p += pr;
+                dst->put(p, public_values + pv_off[i0], pv, true); p += pv;
+                return p + 320;
+            },
+            [&](size_t i0, size_t cnt, uint8_t* d) -> Job {
+                Job j;
+                j.rec_off = (const uint64_t*)d; j.rec_base = proof_off[i0]; j.off = 4; j.stride = 260; j.check_selector = 1; j.selector_le = sel_le(h->verifier_hash);
+                j.mode = SIG_SP1; j.pv_off = (const uint64_t*)(d + (cnt + 1) * 8); j.pv_base = pv_off[i0];
+                j.sig_a = d + (cnt + 1) * 16; j.recs = j.sig_a + cnt * 32; j.sig_b = j.recs + (size_t)(proof_off[i0 + cnt] - proof_off[i0]);
+                j.base = c->h_ic0;
+                return j;
+            }, direct);
     });
 }
 extern "C" int zkv_sp1_verify_proof(const zkv_sp1* h, const uint8_t vkey[32], const uint8_t* public_values, size_t pv_len, const uint8_t* proof, size_t proof_len, uint8_t* status_out) {
@@ -985,18 +988,12 @@ extern "C" int zkv_sp1_verify_batch_device(const zkv_sp1* h, int device, const v
     if (!h || !d_vkeys || !d_public_values || !d_proofs260 || !d_status_out) return fail(ZKV_ERR_ARG, "zkv_sp1_verify_batch_device: null argument");
     DevCtx* c = vk_ctx(h->vk, device);
     if (!c) return fail(ZKV_ERR_ARG, "device not in the handle's device list");
-    std::lock_guard<std::mutex> lk(c->mu);
-    CK(cudaSetDevice(device));
     if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, "device batch too large");
-    Job j; memset(&j, 0, sizeof j);
+    Job j;
     j.vk = h->vk; j.n = n; j.recs = (const uint8_t*)d_proofs260; j.stride = 260; j.off = 4; j.check_selector = 1; j.selector_le = sel_le(h->verifier_hash);
     j.mode = SIG_SP1; j.sig_a = (const uint8_t*)d_vkeys; j.sig_b = (const uint8_t*)d_public_values; j.pv_off = nullptr; j.pv_stride = pv_stride; j.base = c->h_ic0;
     j.d_status = (uint8_t*)d_status_out;
-    cudaStream_t keep = c->stream; c->stream = (cudaStream_t)stream;
-    int rc = run_verify(c, j);
-    if (!rc) rc = ctx_release_async(c, c->stream);
-    c->stream = keep;
-    return rc;
+    return device_call(c, device, stream, [&](cudaStream_t s) { return run_verify(c, j, s); });
 }
 
 
@@ -1066,12 +1063,10 @@ static int pairing4_chain(DevCtx* c, const zkv_vk* vk, size_t o, int n, const ui
     CK(cudaGetLastError());
     return 0;
 }
-static int run_pairing4(DevCtx* c, const zkv_vk* vk, size_t n_, const uint8_t* d_g1s, const uint8_t* d_g2s, uint8_t* d_ok, uint8_t* d_gt, uint8_t* d_miller) {
+static int run_pairing4(DevCtx* c, const zkv_vk* vk, size_t n_, const uint8_t* d_g1s, const uint8_t* d_g2s, uint8_t* d_ok, uint8_t* d_gt, uint8_t* d_miller, cudaStream_t s) {
     if (n_ == 0) return 0;
-    int rc = ctx_acquire(c, c->stream); if (rc) return rc;
-    if (c->busy && (n_ > c->cap || n_ > c->fes_cap)) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }
+    int rc = ctx_acquire(c, s); if (rc) return rc;
     rc = ctx_reserve(c, n_, 8); if (rc) return rc;
-    cudaStream_t s = c->stream;
     if (!vk->valid) {   // a fixed G2 point is invalid: every call reverts
         CK(cudaMemsetAsync(d_ok, 2, n_, s)); if (d_gt) CK(cudaMemsetAsync(d_gt, 0, n_ * 384, s)); if (d_miller) CK(cudaMemsetAsync(d_miller, 0, n_ * 384, s));
         for (int e = 0; e < 6; e++) CK(cudaEventRecord(c->ev[e], s));
@@ -1089,15 +1084,15 @@ extern "C" int zkv_pairing4_batch(const zkv_vk* vk, const uint8_t* g1s, const ui
     if (n == 0) return 0;
     const size_t CH = (size_t)1 << 18;
     return for_each_device(vk->devs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
+        if (int rc = ctx_wait_idle(c)) return rc;      // a host call blocks anyway: wait out an earlier asynchronous device call here
         for (size_t s0 = b; s0 < e; s0 += CH) {
             size_t m = std::min(CH, e - s0);
             size_t ob = m + (gt_out ? m * 384 : 0) + (miller_out ? m * 384 : 0);
-            if (c->busy) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }
             int rc = ctx_stage(c, m * 384, ob); if (rc) return rc;
             memcpy(c->h_pin, g1s + s0 * 256, m * 256); memcpy(c->h_pin + m * 256, g2s + s0 * 128, m * 128);
             CK(cudaMemcpyAsync(c->d_in, c->h_pin, m * 384, cudaMemcpyHostToDevice, c->stream));
             uint8_t* d_gt = gt_out ? c->d_out + m : nullptr; uint8_t* d_ml = miller_out ? c->d_out + m + (gt_out ? m * 384 : 0) : nullptr;
-            rc = run_pairing4(c, vk, m, c->d_in, c->d_in + m * 256, c->d_out, d_gt, d_ml); if (rc) return rc;
+            rc = run_pairing4(c, vk, m, c->d_in, c->d_in + m * 256, c->d_out, d_gt, d_ml, c->stream); if (rc) return rc;
             CK(cudaMemcpyAsync(c->h_out, c->d_out, ob, cudaMemcpyDeviceToHost, c->stream));
             CK(cudaStreamSynchronize(c->stream));
             collect_stage_ms(c);
@@ -1113,13 +1108,9 @@ extern "C" int zkv_pairing4_batch_device(const zkv_vk* vk, int device, const voi
     DevCtx* c = vk_ctx(vk, device);
     if (!c) return fail(ZKV_ERR_ARG, "device not in the key's device list");
     if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, "device batch too large");
-    std::lock_guard<std::mutex> lk(c->mu);
-    CK(cudaSetDevice(device));
-    cudaStream_t keep = c->stream; c->stream = (cudaStream_t)stream;
-    int rc = run_pairing4(c, vk, n, (const uint8_t*)d_g1s, (const uint8_t*)d_g2s, (uint8_t*)d_ok_out, (uint8_t*)d_gt_out, nullptr);
-    if (!rc) rc = ctx_release_async(c, c->stream);
-    c->stream = keep;
-    return rc;
+    return device_call(c, device, stream, [&](cudaStream_t s) {
+        return run_pairing4(c, vk, n, (const uint8_t*)d_g1s, (const uint8_t*)d_g2s, (uint8_t*)d_ok_out, (uint8_t*)d_gt_out, nullptr, s);
+    });
 }
 
 // ------------------------------------------------------------------------------------------ hooks and small services
@@ -1130,8 +1121,8 @@ extern "C" int zkv_vk_x_batch(const zkv_vk* vk, const uint8_t* signals, int k, s
     DevCtx* c = vk->devs[0];
     std::lock_guard<std::mutex> lk(c->mu);
     CK(cudaSetDevice(c->device));
-    if (c->busy) { CK(cudaEventSynchronize(c->ev_busy)); c->busy = false; }
-    int rc = ctx_reserve(c, n, (size_t)k * 8); if (rc) return rc;
+    int rc = ctx_wait_idle(c); if (rc) return rc;
+    rc = ctx_reserve(c, n, (size_t)k * 8); if (rc) return rc;
     rc = ctx_stage(c, n * (size_t)k * 32, n * 64); if (rc) return rc;
     CK(cudaMemcpyAsync(c->d_in, signals, n * (size_t)k * 32, cudaMemcpyHostToDevice, c->stream));
     CK(cudaMemsetAsync(c->flags, 0, n, c->stream));

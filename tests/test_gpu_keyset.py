@@ -154,6 +154,33 @@ def test_device_form_on_a_side_stream_matches_host_path(Z, mixed):
     assert d_st.cpu().numpy().tolist() == host.tolist() == mixed["want"].tolist()
 
 
+def test_set_workspace_growth_under_an_async_device_call(Z, S, gpu):
+    """On a fresh set (empty workspace), a small device call and at once, on another stream, a chunked one that grows every buffer of the
+    set: the second must wait for the first before it frees anything.  Both must give the host path's bytes, taken on a second set of the
+    same keys (its own workspace)."""
+    import torch
+    vks = [S.make_vk(gpu, k % 2, 3 + k, 0x5E7600 + k) for k in range(3)]
+    kvs = [_load(Z, vk) for vk in vks]
+    small, big = _tiled(S, gpu, vks, 100, 32, 0x5E7601), _tiled(S, gpu, vks, 3000, 64, 0x5E7602)
+    ref, ks = Z.VerificationKeySet(kvs), Z.VerificationKeySet(kvs)
+    dev = lambda a: torch.from_numpy(np.frombuffer(a, dtype=np.uint8).copy()).cuda()
+    calls = []
+    for key_idx, prs, sigs, _ in (small, big):
+        n = len(key_idx)
+        off = np.zeros(n + 1, dtype=np.uint64); off[1:] = np.cumsum([len(s) for s in sigs])
+        blob = b"".join(w32(v) for s in sigs for v in s)
+        want = Z.Groth16Verifier.verify_batch_keys_packed(ref, key_idx, b"".join(prs), blob, off)
+        calls.append((want, [dev(key_idx.tobytes()), dev(b"".join(prs)), dev(blob), dev(off.tobytes())], torch.full((n,), 255, dtype=torch.uint8, device="cuda")))
+    assert len(big[0]) > 8192 and 0 < int((calls[1][0] == 0).sum()) < len(big[0])
+    torch.cuda.synchronize()
+    streams = [torch.cuda.Stream(), torch.cuda.Stream()]
+    for (want, d, d_st), st in zip(calls, streams):
+        Z.Groth16Verifier.verify_batch_keys_device(ks, 0, *[x.data_ptr() for x in d], len(want), d_st.data_ptr(), st.cuda_stream)
+    torch.cuda.synchronize()
+    for want, _, d_st in calls:
+        assert d_st.cpu().numpy().tolist() == want.tolist()
+
+
 def test_argument_errors_leave_status_untouched(Z, mixed):
     from stylus_zkvm_verifiers_b200 import _native as N
     ks, n = mixed["ks"], 40

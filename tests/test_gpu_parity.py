@@ -739,6 +739,47 @@ def test_async_device_calls_share_the_workspace_safely(Z, gpu, fx):
     assert stB.cpu().numpy().tolist() == wantB.tolist()
 
 
+def test_workspace_growth_under_an_async_device_call(Z, gpu, fx):
+    """A device call that has to grow the workspace frees buffers an earlier, still running device call on another stream uses, so it must
+    wait for that call first.  On a fresh key handle (empty workspace): a small device call on stream X, at once a chunked one on stream Y
+    that grows every workspace buffer, then a still larger pairing-service device call on the same key.  Each must give the host path's
+    bytes, taken on a second handle of the same key so that its workspace does not pre-grow the first one's."""
+    import torch
+    from stylus_zkvm_verifiers_b200 import synth as S
+    from stylus_zkvm_verifiers_b200 import _native as N
+    vk = S.make_vk(gpu, 0, 6, 0xB2000071)
+    kref, kv = [Z.VerificationKey(0, vk.alpha, vk.beta, vk.gamma, vk.delta, vk.ic) for _ in range(2)]
+    ref, v = Z.RiscZeroVerifier(kref), Z.RiscZeroVerifier(kv)
+    for h in (ref, v):
+        h.initialize(fx["control_root"], fx["bn254_control_id"])
+    t = lambda blobs: torch.frombuffer(bytearray(b"".join(blobs)), dtype=torch.uint8).cuda()
+
+    def mk(n, seed):
+        b = S.make_risc0_batch(gpu, vk, v.get_selector(), fx["control_root"], fx["bn254_control_id"], fx["sys0"], n, seed, pool=64)
+        S.mutate_risc0(b, gpu, S.SplitMix64(seed + 7))
+        keep = [i for i in range(n) if len(b.seals[i]) == 260]
+        return [b.seals[i] for i in keep], [b.image_ids[i] for i in keep], [b.journals[i] for i in keep]
+    A, B = mk(300, 0xB2000072), mk(9500, 0xB2000073)
+    wantA, wantB = np.asarray(ref.verify_batch(*A)), np.asarray(ref.verify_batch(*B))
+    assert len(wantB) > 8192 and 0 < int((wantB == 0).sum()) < len(wantB)
+    npair = len(wantB) + 2000
+    g1s, g2s, _ = S.make_pairing4_batch(gpu, vk, npair, 0xB2000074, pool=16)
+    wantP = Z.pairing4_batch(kref, b"".join(g1s), b"".join(g2s), npair)[0]
+    assert 0 < int((wantP == 1).sum()) < npair
+    dA, dB, dg1, dg2 = [t(x) for x in A], [t(x) for x in B], t(g1s), t(g2s)
+    sx, sy = torch.cuda.Stream(), torch.cuda.Stream()
+    stA = torch.full((len(wantA),), 255, dtype=torch.uint8, device="cuda"); stB = torch.full((len(wantB),), 255, dtype=torch.uint8, device="cuda")
+    okP = torch.full((npair,), 255, dtype=torch.uint8, device="cuda")
+    torch.cuda.synchronize()
+    v.verify_batch_device(0, dA[0].data_ptr(), dA[1].data_ptr(), dA[2].data_ptr(), len(wantA), stA.data_ptr(), sx.cuda_stream)
+    v.verify_batch_device(0, dB[0].data_ptr(), dB[1].data_ptr(), dB[2].data_ptr(), len(wantB), stB.data_ptr(), sy.cuda_stream)
+    N.check(N.lib().zkv_pairing4_batch_device(kv._h, 0, dg1.data_ptr(), dg2.data_ptr(), npair, okP.data_ptr(), None, sx.cuda_stream))
+    torch.cuda.synchronize()
+    assert stA.cpu().numpy().tolist() == wantA.tolist()
+    assert stB.cpu().numpy().tolist() == wantB.tolist()
+    assert okP.cpu().numpy().tolist() == wantP.tolist()
+
+
 def test_staging_copy_covers_every_byte(Z, gpu, fx):
     """Regression (round 2): large blocks are gathered into the pinned staging buffer by several copy threads; slicing by floor(n / parts)
     once left the last n mod parts bytes of a chunk's seal blob uncopied whenever floor(n / parts) was a multiple of 64 - five valid proofs in
