@@ -246,6 +246,15 @@ __global__ void k_g2_check(int n, const fp2* bx, const fp2* by, uint8_t* flags) 
     if (f2_is_zero(x) && f2_is_zero(y)) return;      // infinity is a member
     if (!g2v_in_subgroup(x, y)) flags[i] = fl | F_INVALID;
 }
+// K2 of the shared-memory verification path (k_miller_lz, k_miller_lz_keys): T = -psi^3(B), against which the last Miller segment compares
+// its R (lz_r_is), so the subgroup test costs a Frobenius map here and two Fp2 products there instead of k_g2_check's ~1 800 Fp products
+__global__ void k_g2_target(int n, const fp2* bx, const fp2* by, fp2* tx, fp2* ty) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    fp2 x = bx[i], y = by[i];
+    g2_neg_psi3(x, y);
+    tx[i] = x; ty[i] = y;
+}
 
 // flags[i] |= extra[i] (vk_x's flag bits when it ran beside the G2 check on a scratch array)
 __global__ void k_or_flags(int n, uint8_t* flags, const uint8_t* extra) {
@@ -414,9 +423,10 @@ __device__ __noinline__ void lz_slopes_to(fp* sl, const fp* x1, const fp* y1, co
     sl[0] = xy[0]; sl[1] = xy[1]; sl[2] = iy[0]; sl[3] = iy[1];
 }
 // body of k_miller_lz / k_miller_lz_keys; the key's tables (nt0, nt1: normalised gamma / delta lines, pre = Miller(alpha, beta)) and its
-// disabled pairs come in separately, the rest from `a`
+// disabled pairs come in separately, the rest from `a`.  The last segment also finishes the subgroup test of B against T = (tx, ty)
+// (k_g2_target) and ORs F_INVALID into the proof's flag byte when it fails; R runs through every step whatever the skip bits say.
 __device__ __forceinline__ void miller_lz(int n, const MillerArgs& a, const nline_t* nt0, const nline_t* nt1, const fp12* pre, uint8_t vk_skip,
-                                          const uint8_t* flags, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
+                                          uint8_t* flags, const fp2* tx, const fp2* ty, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
     const int i0 = blockIdx.x * LZ_NT + threadIdx.x, i = i0 < n ? i0 : n - 1;
     const uint8_t fl = flags[i];
     uint32_t skip = vk_skip;
@@ -434,12 +444,13 @@ __device__ __forceinline__ void miller_lz(int n, const MillerArgs& a, const nlin
         lz_st2(tid + LZ_R * LZ_SLOT, R->x); lz_st2(tid + (LZ_R + 2) * LZ_SLOT, R->y); lz_st2(tid + (LZ_R + 4) * LZ_SLOT, R->z);
     }
     lz_miller_norm_seg(in, d_hi, d_lo, last != 0);
+    if (last && !lz_r_is(tid + LZ_R * LZ_SLOT, tx[i], ty[i]) && i0 < n) flags[i] = fl | F_INVALID;
     if (last) { if (pre) lz_f12mul_g(tid + LZ_F * LZ_SLOT, tid + LZ_T * LZ_SLOT, tid + LZ_R * LZ_SLOT, pre, false); }      // x Miller(alpha, beta); T and R are free now
     else if (i0 < n) { g2j* R = rst + i; R->x = lz_ld2(tid + LZ_R * LZ_SLOT); R->y = lz_ld2(tid + (LZ_R + 2) * LZ_SLOT); R->z = lz_ld2(tid + (LZ_R + 4) * LZ_SLOT); }
     if (i0 < n) lz_stg12(fio + i, tid + LZ_F * LZ_SLOT);
 }
-__global__ void __launch_bounds__(LZ_NT, 2) k_miller_lz(int n, MillerArgs a, const uint8_t* flags, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
-    miller_lz(n, a, a.ntabs[0], a.ntabs[1], a.pre, a.vk_skip, flags, fio, rst, sl, d_hi, d_lo, first, last);
+__global__ void __launch_bounds__(LZ_NT, 2) k_miller_lz(int n, MillerArgs a, uint8_t* flags, const fp2* tx, const fp2* ty, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
+    miller_lz(n, a, a.ntabs[0], a.ntabs[1], a.pre, a.vk_skip, flags, tx, ty, fio, rst, sl, d_hi, d_lo, first, last);
 }
 // stages s_lo .. s_hi of the final exponentiation (0..3 = all of it in one launch); st = 6 Fp12 of state per LAUNCHED thread; the last stage writes the
 // status (pairing_mode: 1 product is one / 0 it is not / 2 the call reverts) and, if gt_out is set, the value (12 x BE-32, zeroed for rejected inputs)
@@ -775,12 +786,12 @@ __device__ __forceinline__ int grouped_in_chunk(const uint32_t* total, size_t o,
 }
 // k_miller_lz over slots: each warp reads its key's tables (one key per warp, see above)
 __global__ void __launch_bounds__(LZ_NT, 2) k_miller_lz_keys(const uint32_t* total, size_t o, int m, MillerArgs a, const uint8_t* slot_key, const KeyDesc* keys,
-                                                            const uint8_t* flags, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
+                                                            uint8_t* flags, const fp2* tx, const fp2* ty, fp12* fio, g2j* rst, fp* sl, int d_hi, int d_lo, int first, int last) {
     const int n = grouped_in_chunk(total, o, m);
     if ((int)blockIdx.x * LZ_NT >= n) return;
     const int i0 = blockIdx.x * LZ_NT + threadIdx.x;
     const KeyDesc* kd = keys + slot_key[i0 < n ? i0 : n - 1];
-    miller_lz(n, a, kd->nt[0], kd->nt[1], kd->pre, kd->vk_skip, flags, fio, rst, sl, d_hi, d_lo, first, last);
+    miller_lz(n, a, kd->nt[0], kd->nt[1], kd->pre, kd->vk_skip, flags, tx, ty, fio, rst, sl, d_hi, d_lo, first, last);
 }
 __global__ void __launch_bounds__(LZ_NT, 2) k_final_exp_lz_keys(const uint32_t* total, size_t o, int m, int s_lo, int s_hi, const fp12* in, fp12* st, const uint8_t* flags, uint8_t* status) {
     const int n = grouped_in_chunk(total, o, m);

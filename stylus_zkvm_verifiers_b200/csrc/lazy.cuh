@@ -302,6 +302,22 @@ LZ_FN2 void lz_miller_norm_seg(LzMillerIn in, int d_hi, int d_lo, bool last) {
         li++;
     }
 }
+// The order-r test of B, finished at the end of the verification Miller loop (DESIGN.md section 4).  The loop above leaves
+// R = [6u+2]B + psi(B) - psi^2(B), and 6u+2 + p - p^2 + p^3 = 0 (mod r), so R = -psi^3(B) = T for B in G2 (psi acts as p there).  For B on
+// the twist but outside G2 the sum is not T (the endomorphism 6u+2 + psi - psi^2 + psi^3 has no kernel in the cofactor group: its norm is
+// prime to 2p - r), or an exceptional case of the homogeneous formulas (R = B or R = O before an addition) left Z_R = 0 for good.
+// T in affine coordinates; B = (0, 0), the encoding of infinity, gives T = (0, 0).
+LZ_INL void g2_neg_psi3(fp2& x, fp2& y) {
+    f2_conj(x, x); f2_conj(y, y);
+    x = f2v_mul(x, f2_const(C_FROB3[2])); y = f2v_neg(f2v_mul(y, f2_const(C_FROB3[3])));
+}
+// R (the three Fp2 slots at `r`) equals T: Z_R != 0, X_R = x_T Z_R, Y_R = y_T Z_R.  T = (0, 0) (B = infinity, a member) passes; no point
+// of the twist has x = y = 0.
+LZ_INL bool lz_r_is(uint32_t r, const fp2& tx, const fp2& ty) {
+    const fp2 Z = lz_ld2(r + 4 * LZ_SLOT);
+    const fp2 dx = f2v_sub(lz_ld2(r), f2v_mul(tx, Z)), dy = f2v_sub(lz_ld2(r + 2 * LZ_SLOT), f2v_mul(ty, Z));
+    return (!f2_is_zero(Z) && f2_is_zero(dx) && f2_is_zero(dy)) || (f2_is_zero(tx) && f2_is_zero(ty));
+}
 // General multi-Miller loop on slots (pairing services): `nvar` pairs with their own variable G2 point, then `nfix` pairs whose G2 points
 // have tabled (unscaled) lines; unscaled line products throughout, so the value is the oracle's Miller value bit for bit.  Arrays are
 // pair-major (pair j of instance i at [j * stride + i]).  With more than one variable pair the accumulators R_j do not fit in the slots:

@@ -65,7 +65,7 @@ struct DevCtx {
     size_t cap = 0;
     fp* px[4] = {nullptr, nullptr, nullptr, nullptr}; fp* py[4] = {nullptr, nullptr, nullptr, nullptr};   // four slices of ONE allocation each, `stride` entries apart (pair-major: the general Miller kernel indexes [j * stride + i])
     size_t stride = 0; uint8_t* pskip = nullptr;                                                          // pairing service: per-pair skip bytes, 4 x stride
-    fp2 *qx = nullptr, *qy = nullptr; fp12* f = nullptr; g2j* rst = nullptr; fp* sl = nullptr; fp12* fes = nullptr; size_t fes_cap = 0; uint8_t *flags = nullptr, *status = nullptr;      /* status: scratch flag bytes of vk_x when it runs beside the G2 check */ uint32_t* scal = nullptr; size_t scal_words = 0;
+    fp2 *qx = nullptr, *qy = nullptr, *tx = nullptr, *ty = nullptr; fp12* f = nullptr; g2j* rst = nullptr; fp* sl = nullptr; fp12* fes = nullptr; size_t fes_cap = 0; uint8_t *flags = nullptr, *status = nullptr;      /* status: scratch flag bytes of vk_x when it runs beside the G2 check */ uint32_t* scal = nullptr; size_t scal_words = 0;
     // staging
     uint8_t* d_in = nullptr; size_t d_in_cap = 0; uint8_t* d_out = nullptr; size_t d_out_cap = 0;
     uint8_t* h_pin = nullptr; size_t h_pin_cap = 0; uint8_t* h_out = nullptr; size_t h_out_cap = 0;
@@ -103,7 +103,7 @@ static int ctx_reserve(DevCtx* c, size_t n, size_t scal_words_per_proof) {
     if (n > c->cap || n > c->fes_cap || need > c->scal_words) { int rc = ctx_wait_idle(c); if (rc) return rc; }
     if (n > c->cap) {
         cudaFree(c->px[0]); cudaFree(c->py[0]); cudaFree(c->pskip);
-        cudaFree(c->qx); cudaFree(c->qy); cudaFree(c->f); cudaFree(c->flags); cudaFree(c->status); cudaFree(c->rst); cudaFree(c->sl);
+        cudaFree(c->qx); cudaFree(c->qy); cudaFree(c->tx); cudaFree(c->ty); cudaFree(c->f); cudaFree(c->flags); cudaFree(c->status); cudaFree(c->rst); cudaFree(c->sl);
         c->cap = 0;
         const size_t st = n + PAD;
         CK(cudaMalloc(&c->px[0], 4 * st * sizeof(fp))); CK(cudaMalloc(&c->py[0], 4 * st * sizeof(fp))); CK(cudaMalloc(&c->pskip, 4 * st));
@@ -112,6 +112,7 @@ static int ctx_reserve(DevCtx* c, size_t n, size_t scal_words_per_proof) {
         c->stride = st;
         CK(cudaMalloc(&c->qx, st * sizeof(fp2))); CK(cudaMalloc(&c->qy, st * sizeof(fp2))); CK(cudaMalloc(&c->f, st * sizeof(fp12)));
         CK(cudaMemset(c->qx, 0, st * sizeof(fp2))); CK(cudaMemset(c->qy, 0, st * sizeof(fp2)));
+        CK(cudaMalloc(&c->tx, st * sizeof(fp2))); CK(cudaMalloc(&c->ty, st * sizeof(fp2)));      // T = -psi^3(B) of the fused subgroup test (k_g2_target)
         CK(cudaMalloc(&c->rst, st * sizeof(g2j))); CK(cudaMalloc(&c->sl, st * 4 * sizeof(fp)));
         CK(cudaMalloc(&c->flags, n)); CK(cudaMalloc(&c->status, n));
         c->cap = n;
@@ -148,7 +149,7 @@ static void ctx_free(DevCtx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaFree(c->px[0]); cudaFree(c->py[0]); cudaFree(c->pskip);
-    cudaFree(c->qx); cudaFree(c->qy); cudaFree(c->f); cudaFree(c->flags); cudaFree(c->status); cudaFree(c->scal); cudaFree(c->rst); cudaFree(c->sl); cudaFree(c->fes);
+    cudaFree(c->qx); cudaFree(c->qy); cudaFree(c->tx); cudaFree(c->ty); cudaFree(c->f); cudaFree(c->flags); cudaFree(c->status); cudaFree(c->scal); cudaFree(c->rst); cudaFree(c->sl); cudaFree(c->fes);
     cudaFree(c->d_in); cudaFree(c->d_out); cudaFreeHost(c->h_pin); cudaFreeHost(c->h_out);
     cudaFree(c->d_vk); cudaFree(c->d_lines); cudaFree(c->d_nlines); cudaFree(c->d_pre); cudaFree(c->d_tab); cudaFree(c->d_ic0);
     for (auto& e : c->ev) if (e) cudaEventDestroy(e);
@@ -264,10 +265,14 @@ struct Job {
     const uint64_t* pv_off = nullptr; size_t pv_stride = 0; int k = 0;
     Risc0HashConsts hc = {}; g1aff base = {}; int all_fail = 0;
     uint8_t* d_status = nullptr;
+    bool lz_miller = false;     // the Miller loop runs k_miller_lz and finishes the G2 subgroup test (decided once per batch: lz_miller_of)
 };
 __global__ void k_status_all_fail(int n, const uint8_t* flags, uint8_t* status) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) status[i] = reject_status(flags[i]);
+}
+static bool lz_miller_of(const DevCtx* c, const zkv_vk* vk) {
+    return c->h_vk.norm_ok && vk->tune.normalised_lines.load() && vk->tune.layout.load();
 }
 static std::atomic<unsigned long long> g_launches{0};   // kernels launched by the verification chains since load (bench.py's gpu_launches; a counter, not a setting)
 extern "C" unsigned long long zkv_launch_count(void) { return g_launches.load(); }
@@ -296,17 +301,23 @@ extern "C" int zkv_vk_tune(const void* handle_vk, int option, int value) {
 
 static const bool g_debug_sync = getenv("ZKV_DEBUG_SYNC") != nullptr;      // diagnostics: synchronise after every kernel of a chain and name the one that failed
 #define DBG(name) do { if (g_debug_sync) { cudaError_t e_ = cudaStreamSynchronize(s); if (e_ != cudaSuccess) return fail(ZKV_ERR_CUDA, std::string(name) + ": " + cudaGetErrorString(e_)); } } while (0)
-// The end of the front phase on workspace proofs [o, o+m): vk_x (vkx(flag array) enqueues it on s) and the G2 check.
+// The end of the front phase on workspace proofs [o, o+m): vk_x (vkx(flag array) enqueues it on s) and the G2 check.  fused: the Miller loop
+// will be k_miller_lz / k_miller_lz_keys, which finish the subgroup test in their last segment; the check's slot then holds k_g2_target,
+// which writes the point T = -psi^3(B) that test compares against, and leaves the flags alone.
 // fork: the front phase of a whole chunked batch on the call's main stream.  vk_x and the G2 check are independent (the check reads what the
 // decode kernel wrote, both touch disjoint flag bits of different proofs' bytes only through their own thread), and each is 1.7 waves of its
 // own block shape at 2^16 proofs: side by side on two streams they fill each other's partial waves.  F_SKIPX (vk_x = infinity) and F_INVALID
 // (B outside the subgroup) live in the same flag byte of a proof, so the two kernels must not write it concurrently: vk_x gets a flag array
 // of its own (the front-phase scratch c->status) that is OR-ed in by the G2 check's stream afterwards.
 template <class VkX>
-static int enqueue_vkx_g2(DevCtx* c, size_t o, int m, uint8_t* flags, cudaStream_t s, bool fork, bool timed, VkX vkx) {
+static int enqueue_vkx_g2(DevCtx* c, size_t o, int m, uint8_t* flags, cudaStream_t s, bool fork, bool timed, bool fused, VkX vkx) {
+    auto g2 = [&](cudaStream_t gs) {
+        if (fused) launch(k_g2_target, nblk(m), TPB, 0, gs, m, c->qx + o, c->qy + o, c->tx + o, c->ty + o);
+        else launch(k_g2_check, nblk(m), TPB, 0, gs, m, c->qx + o, c->qy + o, flags);
+    };
     if (fork) {
         CK(cudaEventRecord(c->ev_fork, s)); CK(cudaStreamWaitEvent(c->aux[0], c->ev_fork, 0));
-        launch(k_g2_check, nblk(m), TPB, 0, c->aux[0], m, c->qx + o, c->qy + o, flags);
+        g2(c->aux[0]);
         CK(cudaMemsetAsync(c->status + o, 0, m, s));
         vkx(c->status + o);
         CK(cudaEventRecord(c->ev_join[0], c->aux[0])); CK(cudaStreamWaitEvent(s, c->ev_join[0], 0));
@@ -316,8 +327,8 @@ static int enqueue_vkx_g2(DevCtx* c, size_t o, int m, uint8_t* flags, cudaStream
     vkx(flags);
     if (timed) CK(cudaEventRecord(c->ev[2], s));
     DBG("decode / signals / vk_x");
-    launch(k_g2_check, nblk(m), TPB, 0, s, m, c->qx + o, c->qy + o, flags);
-    DBG("k_g2_check");
+    g2(s);
+    DBG("G2 check");
     if (timed) CK(cudaEventRecord(c->ev[3], s));
     return 0;
 }
@@ -362,7 +373,7 @@ static int enqueue_chain(DevCtx* c, const Job& j, size_t jo, size_t o, int m, cu
             CK(cudaGetLastError());
             return 0;
         }
-        int rc = enqueue_vkx_g2(c, o, m, flags, s, fork_front, timed, [&](uint8_t* fl) {
+        int rc = enqueue_vkx_g2(c, o, m, flags, s, fork_front, timed, j.lz_miller, [&](uint8_t* fl) {
             launch(k_vkx, nblk(m), TPB, 0, s, m, scal, ns, nwin, tab, j.base, c->px[2] + o, c->py[2] + o, fl);
         });
         if (rc) return rc;
@@ -373,13 +384,12 @@ static int enqueue_chain(DevCtx* c, const Job& j, size_t jo, size_t o, int m, cu
     a.ntabs[0] = c->d_nlines; a.ntabs[1] = c->d_nlines + ZKV_LINES_PER_G2;
     a.vk_skip = (uint8_t)((c->h_vk.g2_inf[1] ? 2 : 0) | (c->h_vk.g2_inf[2] ? 4 : 0));
     const bool norm = c->h_vk.norm_ok && vk->tune.normalised_lines.load();
-    const bool lazy = norm && vk->tune.layout.load();
     const int segs = vk->tune.miller_segments.load(), stages = vk->tune.final_exp_stages.load();
-    if (lazy) {                             // shared-memory-resident kernels (lazy.cuh): segments when chunked, one launch otherwise
+    if (j.lz_miller) {                      // shared-memory-resident kernels (lazy.cuh): segments when chunked, one launch otherwise
         const int S = (segs > 1 && !timed) ? segs : 1;
         for (int k = 0; k < S; k++) {
             auto [hi, lo] = miller_segment(k, S);
-            launch(k_miller_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_MILLER, s, m, a, flags, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == S - 1);
+            launch(k_miller_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_MILLER, s, m, a, flags, c->tx + o, c->ty + o, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == S - 1);
             DBG("k_miller_lz");
         }
     } else if (norm && segs > 1 && !timed) {      // a timed single chain (per-stage roofline pass, small batches) runs the one-kernel form
@@ -437,8 +447,9 @@ static int fork_join(DevCtx* c, cudaStream_t main, size_t n, int chunks, F fn) {
     return 0;
 }
 // enqueue all stages of one batch on stream s (asynchronous; completion is ordered on s); caller holds c->mu and has set the device
-static int run_verify(DevCtx* c, const Job& j, cudaStream_t s) {
-    if (j.n == 0) return 0;
+static int run_verify(DevCtx* c, const Job& job, cudaStream_t s) {
+    if (job.n == 0) return 0;
+    Job j = job; j.lz_miller = lz_miller_of(c, j.vk);
     int ns = (j.mode == SIG_GENERIC) ? j.k : 2;
     int rc = ctx_acquire(c, s); if (rc) return rc;
     rc = ctx_reserve(c, j.n, (size_t)ns * 8); if (rc) return rc;
@@ -514,6 +525,7 @@ static int host_pass(DevCtx* c, const zkv_vk* vk, size_t s0, size_t m, int ns, P
     std::vector<cudaEvent_t> evs;                    // front-done event per piece
     if (split) { evs.resize((size_t)np, nullptr); for (auto& e : evs) if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "cudaEventCreate"); }
     std::vector<Job> jobs(np);
+    const bool lz_miller = lz_miller_of(c, vk);
     auto kstream = [&](int k) { return np == 1 ? c->stream : c->aux[k % DevCtx::NAUX]; };
     for (int k = 0; k < np && !rc; k++) {
         const size_t first = pcs[k].first, cnt = pcs[k].cnt, in_off = offs[k];
@@ -523,7 +535,7 @@ static int host_pass(DevCtx* c, const zkv_vk* vk, size_t s0, size_t m, int ns, P
         else rc = cudaMemcpyAsync(c->d_in + in_off, c->h_pin + in_off, bytes[k], cudaMemcpyHostToDevice, s) == cudaSuccess ? 0 : fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (host to device)");
         if (rc) break;
         jobs[k] = job(s0 + first, cnt, c->d_in + in_off);
-        jobs[k].vk = vk; jobs[k].n = cnt; jobs[k].d_status = c->d_out + first;
+        jobs[k].vk = vk; jobs[k].n = cnt; jobs[k].d_status = c->d_out + first; jobs[k].lz_miller = lz_miller;
         if (split && !(jobs[k].all_fail || !vk->valid)) {
             rc = enqueue_chain(c, jobs[k], 0, first, (int)cnt, s, false, 1);
             if (!rc && cudaEventRecord(evs[k], s) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "event (front done)");
@@ -717,7 +729,7 @@ static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t*
     launch(k_decode_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, nk, d_key_idx, d_proofs, c->px[0], c->py[0], c->qx, c->qy, c->px[3], c->py[3], flags);
     launch(k_signals_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, d_sig, d_sig_off, sig_base, ns, c->scal, flags);
     const int chunks = chunk_count(c, S, 0);
-    rc = enqueue_vkx_g2(c, 0, n, flags, st, chunks > 1, false, [&](uint8_t* fl) {   // forked when chunked: the front phase of run_verify's schedule
+    rc = enqueue_vkx_g2(c, 0, n, flags, st, chunks > 1, false, true, [&](uint8_t* fl) {   // forked when chunked: the front phase of run_verify's schedule
         launch(k_vkx_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, c->scal, ns, c->px[2], c->py[2], fl);
     });
     if (rc) return rc;
@@ -725,7 +737,7 @@ static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t*
         const MillerArgs a = verify_miller_args(c, o);
         for (int k = 0; k < segs; k++) {
             auto [hi, lo] = miller_segment(k, segs);
-            launch(k_miller_lz_keys, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_MILLER, hs, sd->total, o, mm, a, sd->slot_key + o, sd->d_keys, flags + o, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == segs - 1);
+            launch(k_miller_lz_keys, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_MILLER, hs, sd->total, o, mm, a, sd->slot_key + o, sd->d_keys, flags + o, c->tx + o, c->ty + o, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == segs - 1);
         }
         if (staged) for (int q = 0; q < 4; q++) launch(k_final_exp_lz_keys, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs, sd->total, o, mm, q, q, c->f + o, c->fes + 6 * o, flags + o, sd->slot_status + o);
         else launch(k_final_exp_lz_keys, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs, sd->total, o, mm, 0, 3, c->f + o, c->fes + 6 * o, flags + o, sd->slot_status + o);
