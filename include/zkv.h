@@ -49,7 +49,9 @@ int zkv_device_count(void);
  * Replaces `VerificationKey` construction (risc0/crypto.rs:81-89, sp1/crypto.rs:83-91).
  * Uploads the key to every listed device and builds, on the GPU, the fixed-base window tables
  * for the IC points, the optimal-ate line tables for beta/gamma/delta and Miller(alpha,beta).
- * n_ic = number of IC points (public inputs + 1), 2..16.  devices == NULL -> device 0 only. */
+ * n_ic = number of IC points (public inputs + 1), 2..16.  devices == NULL -> device 0 only.
+ * ZKV_ERR_ARG also for a valid key with a finite gamma or delta whose normalised line table could not be built (a vanishing line
+ * coefficient, which no point of G2 has). */
 int zkv_vk_load(int vm_type, const uint8_t alpha[64], const uint8_t beta[128], const uint8_t gamma[128],
                 const uint8_t delta[128], const uint8_t* ic, int n_ic, const int* devices, int n_dev, zkv_vk** out);
 int zkv_vk_load_risc0(const int* devices, int n_dev, zkv_vk** out); /* the constants of risc0/crypto.rs:16-79 */
@@ -65,9 +67,8 @@ int zkv_groth16_verify_batch(const zkv_vk* vk, const uint8_t* proofs, const uint
 /* ---- many keys in one batch: N independent verify_proof_with_key calls (common/groth16.rs:23-49) ---------
  * A set of 1..256 loaded keys (borrowed: they must outlive the set).  Every key must be loaded on every device of the set
  * (devices == NULL -> device 0); keys may differ in vm_type and n_ic.  zkv_vkset_create returns ZKV_ERR_ARG for a key missing on
- * a set device, and for a valid key with finite gamma and delta whose normalised line tables could not be built (a vanishing line
- * coefficient).  A set always runs the default schedule (shared-memory kernels, normalised lines, automatic chunking): the member
- * keys' zkv_vk_tune settings do not apply to it.
+ * a set device.  A set always runs the default schedule (automatic chunking, four Miller segments, staged final exponentiation): the
+ * member keys' zkv_vk_tune settings do not apply to it.
  *
  * zkv_groth16_verify_batch_keys: proof i (256 B, the layout of zkv_groth16_verify_batch) is verified under keys[key_idx[i]] with
  * the signals signals[sig_off[i] .. sig_off[i+1]) (offsets in 32-byte words, n+1 of them, non-decreasing).  status_out[i] =
@@ -193,13 +194,14 @@ int zkv_last_stage_ms(const void* handle_vk, int device, float* out, int cap);
  *     front kernels of all pieces run first.  Automatic: one chain below half a wave of the heavy kernels (SMs x 128 proofs), four pieces
  *     above (measured best at every size from 2^16 to 2^20); batches under 8192 proofs are never cut; 1 = one chain on the main stream with
  *     the per-stage events zkv_last_stage_ms reads.
- *   ZKV_TUNE_NORMALISED_LINES (0/1, default 1): verification path uses the per-key normalised gamma / delta line tables (first
- *     coefficient scaled to 1 by a subfield element: 10 instead of 13 Fp2 products per line); 0 = the unscaled lines of the pairing service.
+ *   ZKV_TUNE_NORMALISED_LINES (fixed at 1): the verification path uses the per-key normalised gamma / delta line tables (first
+ *     coefficient scaled to 1 by a subfield element: 10 instead of 13 Fp2 products per line).  A query or setting 1 returns 1;
+ *     setting 0 returns ZKV_ERR_ARG (the unscaled-line verification kernels were removed).
  *   ZKV_TUNE_MILLER_SEGMENTS (1..16, default 4): chunked batches run the Miller loop as that many kernels (f, R carried in HBM).
  *   ZKV_TUNE_FINAL_EXP_STAGES (0/1, default 1): chunked batches run the final exponentiation as four stage kernels (state in HBM).
- *   ZKV_TUNE_LAYOUT (0/1, default 1): 1 = shared-memory-resident lazily reduced Miller / final-exponentiation kernels (two blocks of
- *     128 threads per SM, 28 Fp slots of shared memory per proof), 0 = the round-1 kernels (thread stack, three / two blocks per SM);
- *     kept for A/B measurements (DESIGN.md section 5). */
+ *   ZKV_TUNE_LAYOUT (fixed at 1): shared-memory-resident lazily reduced Miller / final-exponentiation kernels (two blocks of 128
+ *     threads per SM, 28 Fp slots of shared memory per proof).  A query or setting 1 returns 1; setting 0 returns ZKV_ERR_ARG (the
+ *     round-1 thread-stack kernels were removed, DESIGN.md section 5). */
 #define ZKV_TUNE_OVERLAP 0
 #define ZKV_TUNE_NORMALISED_LINES 1
 #define ZKV_TUNE_MILLER_SEGMENTS 2
@@ -211,8 +213,8 @@ int zkv_vk_tune(const void* handle_vk, int option, int value);
  * loaded; bench.py reports the difference over its timed region as gpu_launches. */
 unsigned long long zkv_launch_count(void);
 /* Proofs in one full wave of a heavy kernel on `device` (SM count x resident blocks per SM x 128 threads): kernel 0 = the verification
- * Miller loop, 1 = the final exponentiation (shared-memory layout); 2, 3 = the same two in the round-1 layout.  bench.py times
- * whole-wave launches for its roofline figures.  Negative = error. */
+ * Miller loop, 1 = the final exponentiation (shared-memory layout).  bench.py times whole-wave launches for its roofline figures.
+ * Negative = error (ZKV_ERR_ARG for any other kernel number). */
 long long zkv_wave_proofs(int device, int kernel);
 /* integer-pipe microbenchmark (roofline denominator): returns measured IMAD.WIDE.U32 results/s and
  * Fp-multiplications/s on `device` */
@@ -227,7 +229,7 @@ void zkv_host_free(void* p);
 void zkv_test_parallel_copy(void* dst, const void* src, size_t n);
 /* Known-answer self test of the production kernels on `device`: the reference's two golden proofs (the RISC Zero seal and the SP1 proof
  * of examples/{risc0,sp1}-verifier/examples/interact.rs, with the embedded keys of risc0/crypto.rs:16-79 and sp1/crypto.rs:7-81) must be
- * accepted and a one-bit tamper of each rejected with VerificationFailed, in both kernel layouts.  0 = pass, ZKV_ERR_STATE = a kernel
+ * accepted and a one-bit tamper of each rejected with VerificationFailed.  0 = pass, ZKV_ERR_STATE = a kernel
  * returned a wrong status (a miscompiled build: DESIGN.md section 5), other negatives as usual.  The Python mirror runs it once per
  * process on the first device before the first call (ZKV_SKIP_SELFTEST=1 skips it). */
 int zkv_self_test(int device);

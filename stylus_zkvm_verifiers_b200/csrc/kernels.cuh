@@ -262,157 +262,31 @@ __global__ void k_or_flags(int n, uint8_t* flags, const uint8_t* extra) {
     if (i < n && extra[i]) flags[i] |= extra[i];
 }
 
-// K6: multi-Miller loop.  Pair 0 = (px[0], variable G2); pairs 1..nfixed = (px[j], fixed G2 with line table tabs[j-1]).
+// K6 arguments: pair 0 = (px[0], variable G2); pairs 1..nfixed = (px[j], fixed G2 with line table tabs[j-1]).
 // If pre != nullptr the result is multiplied by that constant (Miller(alpha, beta), precomputed per vk).
 struct MillerArgs {
     const fp* px[4]; const fp* py[4];
     const fp2* qx; const fp2* qy;
     const line_t* tabs[3];
     int nfixed;
-    const nline_t* ntabs[2];  // verification path: normalised tables of gamma and delta (bn254.cuh), used by k_miller_norm
+    const nline_t* ntabs[2];  // verification path: normalised tables of gamma and delta (bn254.cuh), used by k_miller_lz
     const fp12* pre;
     uint8_t skip_bit[4];      // which flag bit disables pair j (0 = never)
     uint8_t vk_skip;          // pairs disabled for the whole batch (a vk G2 point at infinity)
 };
-// Launch shape of the two heavy kernels: blocks whose warps start together, run the same instruction stream and meet at the
-// rendezvous points of bn254.cuh, so they share instruction-cache lines; two such blocks per SM run out of phase with each
-// other, which lets one block's integer-multiply bursts overlap the other's carry / load phases.
+// Launch shape of the thread-stack tower kernels (k_fp12_op) and the granularity of a batch's chunks: blocks whose warps start together,
+// run the same instruction stream and meet at the rendezvous points of bn254.cuh, two blocks per SM (the same wave as the LZ_NT kernels).
 #ifndef ZKV_HTPB
 #define ZKV_HTPB 128
 #endif
 #ifndef ZKV_MINBLOCKS
 #define ZKV_MINBLOCKS 2
 #endif
-// The verification Miller-loop kernels (k_miller_norm, k_miller_norm_seg) run three blocks per SM (168 registers): measured on whole
-// waves, -4 % per proof against two blocks; the final exponentiation (more live Fp12 values) is 6 % slower at three and stays at two.
-#ifndef ZKV_MINBLOCKS_MILLER
-#define ZKV_MINBLOCKS_MILLER 3
-#endif
-#ifndef ZKV_HTPB_MILLER
-#define ZKV_HTPB_MILLER ZKV_HTPB
-#endif
-#ifndef ZKV_HTPB_FE
-#define ZKV_HTPB_FE ZKV_HTPB
-#endif
-#ifndef ZKV_MINBLOCKS_FE
-#define ZKV_MINBLOCKS_FE ZKV_MINBLOCKS
-#endif
-__global__ void __launch_bounds__(ZKV_HTPB, ZKV_MINBLOCKS) k_miller(int n, MillerArgs a, const uint8_t* flags, fp12* out) {
-    int i0 = blockIdx.x * blockDim.x + threadIdx.x;
-    int i = i0 < n ? i0 : n - 1;                      // surplus threads redo the last proof (every thread reaches every rendezvous)
-    uint8_t fl = flags[i];
-    uint32_t skip = a.vk_skip;
-    for (int j = 0; j <= a.nfixed; j++) if (fl & a.skip_bit[j]) skip |= 1u << j;
-    if (fl & (F_INVALID | F_SELMIS)) skip = 0xF;      // result is never used: every factor is replaced by 1 (the work is still done: uniform control flow)
-    fp px[4], py[4];
-    for (int j = 0; j <= a.nfixed; j++) { px[j] = a.px[j][i]; py[j] = a.py[j][i]; }
-    fp2 qx = a.qx[i], qy = a.qy[i];
-    fp12 f;
-    miller_loop(f, px, py, qx, qy, a.tabs, a.nfixed, skip);
-    if (a.pre) { fp12 p = *a.pre; f12_mul(f, f, p); }
-    if (i0 < n) out[i] = f;
-}
-
-// K6 for the verification entry points: pairs (A', B), (vk_x, gamma), (C, delta) with the NORMALISED gamma / delta tables (bn254.cuh),
-// times the per-key constant Miller(alpha, beta).  Same launch shape and flag conventions as k_miller.
-__global__ void __launch_bounds__(ZKV_HTPB_MILLER, ZKV_MINBLOCKS_MILLER) k_miller_norm(int n, MillerArgs a, const uint8_t* flags, fp12* out) {
-    int i0 = blockIdx.x * blockDim.x + threadIdx.x;
-    int i = i0 < n ? i0 : n - 1;
-    uint8_t fl = flags[i];
-    uint32_t skip = a.vk_skip;
-    for (int j = 0; j < 3; j++) if (fl & a.skip_bit[j]) skip |= 1u << j;
-    if (fl & F_REJECT) skip = 0xF;
-    fp x12[2] = {a.px[1][i], a.px[2][i]}, y12[2] = {a.py[1][i], a.py[2][i]}, xy[2], iy[2];
-    bool off[2] = {(skip & 2u) != 0, (skip & 4u) != 0};
-    g1_slopes2(xy, iy, x12, y12, off);
-    fp px0 = a.px[0][i], py0 = a.py[0][i];
-    fp2 qx = a.qx[i], qy = a.qy[i];
-    fp12 f;
-    miller_loop_norm(f, px0, py0, qx, qy, a.ntabs, xy, iy, (skip & 1u) != 0);
-    if (a.pre) { fp12 p = *a.pre; f12_mul(f, f, p); }
-    if (i0 < n) out[i] = f;
-}
-
-// Segment form of k_miller_norm: digits d_hi .. d_lo of the loop; f (in `fio`) and R (in `rst`) are carried in HBM between segments, the
-// slopes of the two fixed pairs are computed by the first segment and kept in `sl` (4 Fp per proof).
-__global__ void __launch_bounds__(ZKV_HTPB_MILLER, ZKV_MINBLOCKS_MILLER) k_miller_norm_seg(int n, MillerArgs a, const uint8_t* flags, fp12* fio, g2j* rst, fp* sl,
-                                                                              int d_hi, int d_lo, int first, int last) {
-    int i0 = blockIdx.x * blockDim.x + threadIdx.x;
-    int i = i0 < n ? i0 : n - 1;
-    uint8_t fl = flags[i];
-    uint32_t skip = a.vk_skip;
-    for (int j = 0; j < 3; j++) if (fl & a.skip_bit[j]) skip |= 1u << j;
-    if (fl & F_REJECT) skip = 0xF;
-    fp xy[2], iy[2];
-    if (first) {
-        fp x12[2] = {a.px[1][i], a.px[2][i]}, y12[2] = {a.py[1][i], a.py[2][i]};
-        bool off[2] = {(skip & 2u) != 0, (skip & 4u) != 0};
-        g1_slopes2(xy, iy, x12, y12, off);
-        if (i0 < n && !last) { sl[4 * (size_t)i] = xy[0]; sl[4 * (size_t)i + 1] = xy[1]; sl[4 * (size_t)i + 2] = iy[0]; sl[4 * (size_t)i + 3] = iy[1]; }
-    } else {
-        xy[0] = sl[4 * (size_t)i]; xy[1] = sl[4 * (size_t)i + 1]; iy[0] = sl[4 * (size_t)i + 2]; iy[1] = sl[4 * (size_t)i + 3];
-    }
-    fp px0 = a.px[0][i], py0 = a.py[0][i];
-    fp2 qx = a.qx[i], qy = a.qy[i];
-    fp12 f; g2j R;
-    if (first) { f = f12_one(); R.x = qx; R.y = qy; R.z = f2_one(); }
-    else { f = fio[i]; R = rst[i]; }
-    miller_loop_norm_seg(f, R, px0, py0, qx, qy, a.ntabs, xy, iy, (skip & 1u) != 0, d_hi, d_lo, last != 0);
-    if (last) { if (a.pre) { fp12 p = *a.pre; f12_mul(f, f, p); } }
-    else if (i0 < n) rst[i] = R;
-    if (i0 < n) fio[i] = f;
-}
-
-// K7 + K8: final exponentiation, is-one test and status byte
-__global__ void __launch_bounds__(ZKV_HTPB_FE, ZKV_MINBLOCKS_FE) k_final_exp(int n, const fp12* in, const uint8_t* flags, uint8_t* status, uint8_t* gt_out, int pairing_mode) {
-    int i0 = blockIdx.x * blockDim.x + threadIdx.x;
-    int i = i0 < n ? i0 : n - 1;
-    uint8_t fl = flags[i];
-    fp12 m = in[i], gt;
-    final_exp(gt, m);                                 // every thread runs it (k_miller left a harmless value for rejected inputs): uniform control flow
-    if (i0 >= n) return;
-    if (fl & (pairing_mode ? (F_INVALID | F_SELMIS) : F_REJECT)) {
-        status[i] = pairing_mode ? 2 : reject_status(fl);
-        if (gt_out) for (int k = 0; k < 384; k++) gt_out[(size_t)i * 384 + k] = 0;
-        return;
-    }
-    bool one = f12_is_one(gt);
-    status[i] = pairing_mode ? (one ? 1 : 0) : (one ? ST_OK : ST_VERIFICATION_FAILED);
-    if (gt_out) f12_to_bytes(gt_out + (size_t)i * 384, gt);
-}
-// Staged form of k_final_exp (bn254.cuh final_exp_stage0..3): the state (f, x, y, z, t1; slot 1 first holds t = f^u) lives in `st`, five
-// Fp12 per proof, so that the three exponentiations by u of different chunks can interleave.  Stage 3 writes the status like k_final_exp.
-__global__ void __launch_bounds__(ZKV_HTPB_FE, ZKV_MINBLOCKS_FE) k_final_exp_stage(int n, int stage, const fp12* in, fp12* st, const uint8_t* flags, uint8_t* status) {
-    int i0 = blockIdx.x * blockDim.x + threadIdx.x;
-    int i = i0 < n ? i0 : n - 1;
-    const bool w = i0 < n;
-    fp12* s = st + 5 * (size_t)i;
-    if (stage == 0) {
-        fp12 m = in[i], f, t;
-        final_exp_stage0(f, t, m);
-        if (w) { s[0] = f; s[1] = t; }
-    } else if (stage == 1) {
-        fp12 t = s[1], x, y, z;
-        final_exp_stage1(x, y, z, t);
-        if (w) { s[1] = x; s[2] = y; s[3] = z; }
-    } else if (stage == 2) {
-        fp12 z = s[3], t1;
-        final_exp_stage2(t1, z);
-        if (w) s[4] = t1;
-    } else {
-        fp12 f = s[0], x = s[1], y = s[2], z = s[3], t1 = s[4], gt;
-        final_exp_stage3(gt, f, x, y, z, t1);
-        if (!w) return;
-        uint8_t fl = flags[i];
-        if (fl & F_REJECT) { status[i] = reject_status(fl); return; }
-        status[i] = f12_is_one(gt) ? ST_OK : ST_VERIFICATION_FAILED;
-    }
-}
 // ---------------------------------------------------------------------------- shared-memory-resident forms of K6 / K7 (csrc/lazy.cuh)
-// Same inputs, outputs and flag conventions as k_miller_norm_seg / k_final_exp_stage; the working set of a proof (f, R, temporaries: 28 Fp
-// slots = 896 B) lives in shared memory, two blocks of LZ_NT = 128 threads per SM, the Fp6-level products are lazily reduced.  The state
-// between segments / stages travels through HBM exactly as in the round-1 kernels.  `sl` must have room for 4 Fp per LAUNCHED thread
-// (surplus threads of the last block park their slopes behind the batch).
+// The Miller loop runs in segments (digits d_hi .. d_lo), the final exponentiation in stages; the working set of a proof (f, R, temporaries:
+// 28 Fp slots = 896 B) lives in shared memory, two blocks of LZ_NT = 128 threads per SM, the Fp6-level products are lazily reduced.  The
+// state between segments / stages travels through HBM: f in `fio`, R in `rst`, the slopes of the two fixed pairs in `sl`, which must have
+// room for 4 Fp per LAUNCHED thread (surplus threads of the last block park their slopes behind the batch).
 #define LZ_SMEM_BYTES (LZ_SLOTS * 32 * LZ_NT)
 #define LZ_SMEM_MILLER (LZ_SMEM_BYTES + 1024)      /* + the per-warp line staging areas of lz_fixed_lines: 2 x (112 KB + 1 KB + 1 KB reserved) = the SM's 228 KB */
 // slopes of the two fixed pairs (g1_slopes2) written to sl[0..3] = xy0, xy1, iy0, iy1; out of line so that its arrays have a frame of their own
@@ -596,7 +470,7 @@ struct VkDev {                 // device-resident, Montgomery form
     fp alpha_x, alpha_y;
     int valid;                 // all key points decode under EIP-196/197 rules (else every verify fails)
     int g2_inf[3]; int alpha_inf;
-    int norm_ok;               // the normalised gamma / delta line tables exist (no vanishing l0)
+    int norm_ok;               // no finite gamma / delta has a vanishing l0 (its normalised line table exists)
 };
 // block j<3 (one thread each) validates + tabulates G2 point j; block 3 validates alpha
 __global__ void k_vk_setup(const uint8_t* alpha, const uint8_t* g2bytes /* 3 x 128 */, VkDev* vk, line_t* lines /* 3 x LINES */, nline_t* nlines /* 2 x LINES: gamma, delta */) {
@@ -608,7 +482,8 @@ __global__ void k_vk_setup(const uint8_t* alpha, const uint8_t* g2bytes /* 3 x 1
         vk->g2x[j] = x; vk->g2y[j] = y; vk->g2_inf[j] = (r == 1);
         if (r == 2) atomicAnd(&vk->valid, 0);
         if (r == 0) g2_precompute_lines(lines + (size_t)j * ZKV_LINES_PER_G2, x, y);
-        if (j >= 1 && (r != 0 || !g2_normalise_lines(nlines + (size_t)(j - 1) * ZKV_LINES_PER_G2, lines + (size_t)j * ZKV_LINES_PER_G2, ZKV_LINES_PER_G2))) atomicAnd(&vk->norm_ok, 0);
+        // gamma / delta at infinity keep their all-zero normalised table: the Miller loop switches that pair off (vk_skip)
+        if (j >= 1 && r == 0 && !g2_normalise_lines(nlines + (size_t)(j - 1) * ZKV_LINES_PER_G2, lines + (size_t)j * ZKV_LINES_PER_G2, ZKV_LINES_PER_G2)) atomicAnd(&vk->norm_ok, 0);
     } else if (j == 3) {
         uint32_t rx[8], ry[8]; be32_to_raw(rx, alpha); be32_to_raw(ry, alpha + 32);
         fp x, y; int r = g1_decode_raw(x, y, rx, ry);

@@ -86,10 +86,8 @@ struct DevCtx {
 // Tuning of one key handle (zkv_vk_tune): no process-wide mutable state (SURVEY.md section 8b).  Read once per batch call.
 struct Tuning {
     std::atomic<int> overlap_chunks{0};     // a device batch is cut into this many kernel chains on side streams; 0 = automatic (chunk_count)
-    std::atomic<int> normalised_lines{1};   // verification path: gamma / delta lines scaled to (1, n3, n4)
     std::atomic<int> miller_segments{4};    // chunked batches: segment kernels per Miller loop (state in HBM between them); 4 measured best (profiles/r2_chunk_sweep.txt)
     std::atomic<int> final_exp_stages{1};   // chunked batches: the final exponentiation as four stage kernels
-    std::atomic<int> layout{1};             // 1: shared-memory-resident lazily reduced kernels (lazy.cuh); 0: the round-1 thread-stack kernels
 };
 static constexpr size_t PAD = 256;          // workspace slack behind a batch: surplus threads of the last block park their state there
 // wait on the host for the last asynchronous user of the workspace (caller holds c->mu)
@@ -238,6 +236,9 @@ extern "C" int zkv_vk_load(int vm_type, const uint8_t alpha[64], const uint8_t b
     for (int d : devs) {
         DevCtx* c = new DevCtx(); c->device = d; vk->devs.push_back(c);
         int rc = vk_build_on(vk, c);
+        // the Miller loop needs the normalised line table of every finite gamma / delta of a valid key: a line coefficient l0 vanishes for
+        // no point of G2 (DESIGN.md section 4), but key bytes come from outside
+        if (!rc && c->h_vk.valid && !c->h_vk.norm_ok) rc = fail(ZKV_ERR_ARG, "zkv_vk_load: the key has no normalised gamma / delta line tables (a vanishing line coefficient)");
         if (rc) { zkv_vk_free(vk); return rc; }
     }
     *out = vk;
@@ -265,14 +266,10 @@ struct Job {
     const uint64_t* pv_off = nullptr; size_t pv_stride = 0; int k = 0;
     Risc0HashConsts hc = {}; g1aff base = {}; int all_fail = 0;
     uint8_t* d_status = nullptr;
-    bool lz_miller = false;     // the Miller loop runs k_miller_lz and finishes the G2 subgroup test (decided once per batch: lz_miller_of)
 };
 __global__ void k_status_all_fail(int n, const uint8_t* flags, uint8_t* status) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) status[i] = reject_status(flags[i]);
-}
-static bool lz_miller_of(const DevCtx* c, const zkv_vk* vk) {
-    return c->h_vk.norm_ok && vk->tune.normalised_lines.load() && vk->tune.layout.load();
 }
 static std::atomic<unsigned long long> g_launches{0};   // kernels launched by the verification chains since load (bench.py's gpu_launches; a counter, not a setting)
 extern "C" unsigned long long zkv_launch_count(void) { return g_launches.load(); }
@@ -288,10 +285,11 @@ extern "C" int zkv_vk_tune(const void* handle_vk, int option, int value) {
     std::atomic<int>* f; int lo, hi;
     switch (option) {
         case ZKV_TUNE_OVERLAP: f = &vk->tune.overlap_chunks; lo = 0; hi = 64; break;
-        case ZKV_TUNE_NORMALISED_LINES: f = &vk->tune.normalised_lines; lo = 0; hi = 1; break;
         case ZKV_TUNE_MILLER_SEGMENTS: f = &vk->tune.miller_segments; lo = 1; hi = 16; break;
         case ZKV_TUNE_FINAL_EXP_STAGES: f = &vk->tune.final_exp_stages; lo = 0; hi = 1; break;
-        case ZKV_TUNE_LAYOUT: f = &vk->tune.layout; lo = 0; hi = 1; break;
+        case ZKV_TUNE_NORMALISED_LINES: case ZKV_TUNE_LAYOUT:          // fixed at 1: the shared-memory kernels with normalised lines are the only ones
+            if (value == ZKV_TUNE_QUERY || value == 1) return 1;
+            return fail(ZKV_ERR_ARG, "zkv_vk_tune: the round-1 kernels and the unscaled verification lines were removed; this option is fixed at 1");
         default: return fail(ZKV_ERR_ARG, "zkv_vk_tune: unknown option");
     }
     if (value == ZKV_TUNE_QUERY) return f->load();
@@ -301,20 +299,17 @@ extern "C" int zkv_vk_tune(const void* handle_vk, int option, int value) {
 
 static const bool g_debug_sync = getenv("ZKV_DEBUG_SYNC") != nullptr;      // diagnostics: synchronise after every kernel of a chain and name the one that failed
 #define DBG(name) do { if (g_debug_sync) { cudaError_t e_ = cudaStreamSynchronize(s); if (e_ != cudaSuccess) return fail(ZKV_ERR_CUDA, std::string(name) + ": " + cudaGetErrorString(e_)); } } while (0)
-// The end of the front phase on workspace proofs [o, o+m): vk_x (vkx(flag array) enqueues it on s) and the G2 check.  fused: the Miller loop
-// will be k_miller_lz / k_miller_lz_keys, which finish the subgroup test in their last segment; the check's slot then holds k_g2_target,
-// which writes the point T = -psi^3(B) that test compares against, and leaves the flags alone.
+// The end of the front phase on workspace proofs [o, o+m): vk_x (vkx(flag array) enqueues it on s) and the G2 check.  The Miller loop
+// (k_miller_lz / k_miller_lz_keys) finishes the subgroup test in its last segment; the check's slot holds k_g2_target, which writes the
+// point T = -psi^3(B) that test compares against, and leaves the flags alone.
 // fork: the front phase of a whole chunked batch on the call's main stream.  vk_x and the G2 check are independent (the check reads what the
 // decode kernel wrote, both touch disjoint flag bits of different proofs' bytes only through their own thread), and each is 1.7 waves of its
 // own block shape at 2^16 proofs: side by side on two streams they fill each other's partial waves.  F_SKIPX (vk_x = infinity) and F_INVALID
 // (B outside the subgroup) live in the same flag byte of a proof, so the two kernels must not write it concurrently: vk_x gets a flag array
 // of its own (the front-phase scratch c->status) that is OR-ed in by the G2 check's stream afterwards.
 template <class VkX>
-static int enqueue_vkx_g2(DevCtx* c, size_t o, int m, uint8_t* flags, cudaStream_t s, bool fork, bool timed, bool fused, VkX vkx) {
-    auto g2 = [&](cudaStream_t gs) {
-        if (fused) launch(k_g2_target, nblk(m), TPB, 0, gs, m, c->qx + o, c->qy + o, c->tx + o, c->ty + o);
-        else launch(k_g2_check, nblk(m), TPB, 0, gs, m, c->qx + o, c->qy + o, flags);
-    };
+static int enqueue_vkx_g2(DevCtx* c, size_t o, int m, uint8_t* flags, cudaStream_t s, bool fork, bool timed, VkX vkx) {
+    auto g2 = [&](cudaStream_t gs) { launch(k_g2_target, nblk(m), TPB, 0, gs, m, c->qx + o, c->qy + o, c->tx + o, c->ty + o); };
     if (fork) {
         CK(cudaEventRecord(c->ev_fork, s)); CK(cudaStreamWaitEvent(c->aux[0], c->ev_fork, 0));
         g2(c->aux[0]);
@@ -373,7 +368,7 @@ static int enqueue_chain(DevCtx* c, const Job& j, size_t jo, size_t o, int m, cu
             CK(cudaGetLastError());
             return 0;
         }
-        int rc = enqueue_vkx_g2(c, o, m, flags, s, fork_front, timed, j.lz_miller, [&](uint8_t* fl) {
+        int rc = enqueue_vkx_g2(c, o, m, flags, s, fork_front, timed, [&](uint8_t* fl) {
             launch(k_vkx, nblk(m), TPB, 0, s, m, scal, ns, nwin, tab, j.base, c->px[2] + o, c->py[2] + o, fl);
         });
         if (rc) return rc;
@@ -383,29 +378,17 @@ static int enqueue_chain(DevCtx* c, const Job& j, size_t jo, size_t o, int m, cu
     a.tabs[0] = c->d_lines + 1 * ZKV_LINES_PER_G2; a.tabs[1] = c->d_lines + 2 * ZKV_LINES_PER_G2; a.pre = c->d_pre;
     a.ntabs[0] = c->d_nlines; a.ntabs[1] = c->d_nlines + ZKV_LINES_PER_G2;
     a.vk_skip = (uint8_t)((c->h_vk.g2_inf[1] ? 2 : 0) | (c->h_vk.g2_inf[2] ? 4 : 0));
-    const bool norm = c->h_vk.norm_ok && vk->tune.normalised_lines.load();
     const int segs = vk->tune.miller_segments.load(), stages = vk->tune.final_exp_stages.load();
-    if (j.lz_miller) {                      // shared-memory-resident kernels (lazy.cuh): segments when chunked, one launch otherwise
-        const int S = (segs > 1 && !timed) ? segs : 1;
-        for (int k = 0; k < S; k++) {
-            auto [hi, lo] = miller_segment(k, S);
-            launch(k_miller_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_MILLER, s, m, a, flags, c->tx + o, c->ty + o, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == S - 1);
-            DBG("k_miller_lz");
-        }
-    } else if (norm && segs > 1 && !timed) {      // a timed single chain (per-stage roofline pass, small batches) runs the one-kernel form
-        for (int k = 0; k < segs; k++) {
-            auto [hi, lo] = miller_segment(k, segs);
-            launch(k_miller_norm_seg, nblk(m, ZKV_HTPB_MILLER), ZKV_HTPB_MILLER, 0, s, m, a, flags, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == segs - 1);
-        }
-    } else if (norm) launch(k_miller_norm, nblk(m, ZKV_HTPB_MILLER), ZKV_HTPB_MILLER, 0, s, m, a, flags, c->f + o);
-    else launch(k_miller, nblk(m, ZKV_HTPB), ZKV_HTPB, 0, s, m, a, flags, c->f + o);
+    // shared-memory-resident kernels (lazy.cuh): segments / stages when chunked, one launch each in a timed single chain
+    const int S = (segs > 1 && !timed) ? segs : 1;
+    for (int k = 0; k < S; k++) {
+        auto [hi, lo] = miller_segment(k, S);
+        launch(k_miller_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_MILLER, s, m, a, flags, c->tx + o, c->ty + o, c->f + o, c->rst + o, c->sl + 4 * o, hi, lo, k == 0, k == S - 1);
+        DBG("k_miller_lz");
+    }
     if (timed) CK(cudaEventRecord(c->ev[4], s));
-    if (vk->tune.layout.load()) {
-        if (stages && !timed) for (int st = 0; st < 4; st++) launch(k_final_exp_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s, m, st, st, c->f + o, c->fes + 6 * o, flags, j.d_status + jo, nullptr, 0);
-        else launch(k_final_exp_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s, m, 0, 3, c->f + o, c->fes + 6 * o, flags, j.d_status + jo, nullptr, 0);
-    } else if (stages && !timed) {
-        for (int st = 0; st < 4; st++) launch(k_final_exp_stage, nblk(m, ZKV_HTPB_FE), ZKV_HTPB_FE, 0, s, m, st, c->f + o, c->fes + 5 * o, flags, j.d_status + jo);
-    } else launch(k_final_exp, nblk(m, ZKV_HTPB_FE), ZKV_HTPB_FE, 0, s, m, c->f + o, flags, j.d_status + jo, nullptr, 0);
+    if (stages && !timed) for (int st = 0; st < 4; st++) launch(k_final_exp_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s, m, st, st, c->f + o, c->fes + 6 * o, flags, j.d_status + jo, nullptr, 0);
+    else launch(k_final_exp_lz, nblk(m, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s, m, 0, 3, c->f + o, c->fes + 6 * o, flags, j.d_status + jo, nullptr, 0);
     DBG("final exponentiation");
     if (timed) CK(cudaEventRecord(c->ev[5], s));
     CK(cudaGetLastError());
@@ -447,9 +430,8 @@ static int fork_join(DevCtx* c, cudaStream_t main, size_t n, int chunks, F fn) {
     return 0;
 }
 // enqueue all stages of one batch on stream s (asynchronous; completion is ordered on s); caller holds c->mu and has set the device
-static int run_verify(DevCtx* c, const Job& job, cudaStream_t s) {
-    if (job.n == 0) return 0;
-    Job j = job; j.lz_miller = lz_miller_of(c, j.vk);
+static int run_verify(DevCtx* c, const Job& j, cudaStream_t s) {
+    if (j.n == 0) return 0;
     int ns = (j.mode == SIG_GENERIC) ? j.k : 2;
     int rc = ctx_acquire(c, s); if (rc) return rc;
     rc = ctx_reserve(c, j.n, (size_t)ns * 8); if (rc) return rc;
@@ -525,7 +507,6 @@ static int host_pass(DevCtx* c, const zkv_vk* vk, size_t s0, size_t m, int ns, P
     std::vector<cudaEvent_t> evs;                    // front-done event per piece
     if (split) { evs.resize((size_t)np, nullptr); for (auto& e : evs) if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "cudaEventCreate"); }
     std::vector<Job> jobs(np);
-    const bool lz_miller = lz_miller_of(c, vk);
     auto kstream = [&](int k) { return np == 1 ? c->stream : c->aux[k % DevCtx::NAUX]; };
     for (int k = 0; k < np && !rc; k++) {
         const size_t first = pcs[k].first, cnt = pcs[k].cnt, in_off = offs[k];
@@ -535,7 +516,7 @@ static int host_pass(DevCtx* c, const zkv_vk* vk, size_t s0, size_t m, int ns, P
         else rc = cudaMemcpyAsync(c->d_in + in_off, c->h_pin + in_off, bytes[k], cudaMemcpyHostToDevice, s) == cudaSuccess ? 0 : fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (host to device)");
         if (rc) break;
         jobs[k] = job(s0 + first, cnt, c->d_in + in_off);
-        jobs[k].vk = vk; jobs[k].n = cnt; jobs[k].d_status = c->d_out + first; jobs[k].lz_miller = lz_miller;
+        jobs[k].vk = vk; jobs[k].n = cnt; jobs[k].d_status = c->d_out + first;
         if (split && !(jobs[k].all_fail || !vk->valid)) {
             rc = enqueue_chain(c, jobs[k], 0, first, (int)cnt, s, false, 1);
             if (!rc && cudaEventRecord(evs[k], s) != cudaSuccess) rc = fail(ZKV_ERR_CUDA, "event (front done)");
@@ -678,10 +659,6 @@ extern "C" int zkv_vkset_create(const zkv_vk* const* keys, int n_keys, const int
         for (int d : devs) {
             const DevCtx* kc = vk_ctx(keys[k], d);
             if (!kc) return fail(ZKV_ERR_ARG, "zkv_vkset_create: key " + std::to_string(k) + " is not loaded on device " + std::to_string(d));
-            // a valid key whose gamma and delta are finite has normalised line tables unless a line coefficient vanished (not expected for
-            // points of G2); the set has no unscaled-line path for such a key
-            if (keys[k]->valid && !kc->h_vk.norm_ok && !kc->h_vk.g2_inf[1] && !kc->h_vk.g2_inf[2])
-                return fail(ZKV_ERR_ARG, "zkv_vkset_create: key " + std::to_string(k) + " has no normalised gamma / delta line tables (a vanishing line coefficient)");
         }
     zkv_vkset* s = new zkv_vkset();
     s->keys.assign(keys, keys + n_keys);
@@ -729,7 +706,7 @@ static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t*
     launch(k_decode_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, nk, d_key_idx, d_proofs, c->px[0], c->py[0], c->qx, c->qy, c->px[3], c->py[3], flags);
     launch(k_signals_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, d_sig, d_sig_off, sig_base, ns, c->scal, flags);
     const int chunks = chunk_count(c, S, 0);
-    rc = enqueue_vkx_g2(c, 0, n, flags, st, chunks > 1, false, true, [&](uint8_t* fl) {   // forked when chunked: the front phase of run_verify's schedule
+    rc = enqueue_vkx_g2(c, 0, n, flags, st, chunks > 1, false, [&](uint8_t* fl) {   // forked when chunked: the front phase of run_verify's schedule
         launch(k_vkx_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, c->scal, ns, c->px[2], c->py[2], fl);
     });
     if (rc) return rc;
@@ -1024,11 +1001,10 @@ extern "C" int zkv_self_test(int device) {
     int rc = zkv_risc0_create(nullptr, &device, 1, &r0);
     if (!rc) rc = zkv_risc0_initialize(r0, ZKV_RISC0_FIXTURE_CONTROL_ROOT, ZKV_RISC0_FIXTURE_BN254_CONTROL_ID);
     if (!rc) rc = zkv_sp1_create(nullptr, &device, 1, &s1);
-    for (int layout = 1; !rc && layout >= 0; layout--) {
+    if (!rc) {
         uint8_t st[4] = {255, 255, 255, 255};
         uint8_t seal[sizeof ZKV_RISC0_FIXTURE_SEAL], proof[sizeof ZKV_SP1_FIXTURE_PROOF];
         memcpy(seal, ZKV_RISC0_FIXTURE_SEAL, sizeof seal); memcpy(proof, ZKV_SP1_FIXTURE_PROOF, sizeof proof);
-        zkv_vk_tune(zkv_risc0_vk(r0), ZKV_TUNE_LAYOUT, layout); zkv_vk_tune(zkv_sp1_vk(s1), ZKV_TUNE_LAYOUT, layout);
         rc = zkv_risc0_verify(r0, seal, sizeof seal, ZKV_RISC0_FIXTURE_IMAGE_ID, ZKV_RISC0_FIXTURE_JOURNAL_DIGEST, &st[0]);
         seal[4 + 100] ^= 0x04;                               // one bit of B: still a field element, no longer a valid proof
         if (!rc) rc = zkv_risc0_verify(r0, seal, sizeof seal, ZKV_RISC0_FIXTURE_IMAGE_ID, ZKV_RISC0_FIXTURE_JOURNAL_DIGEST, &st[1]);
@@ -1036,7 +1012,7 @@ extern "C" int zkv_self_test(int device) {
         uint8_t vkey[32]; memcpy(vkey, ZKV_SP1_FIXTURE_VKEY, 32); vkey[31] ^= 1;      // another program key: a different public input
         if (!rc) rc = zkv_sp1_verify_proof(s1, vkey, ZKV_SP1_FIXTURE_PUBLIC_VALUES, sizeof ZKV_SP1_FIXTURE_PUBLIC_VALUES, proof, sizeof proof, &st[3]);
         if (!rc && !(st[0] == ZKV_OK && st[2] == ZKV_OK && st[1] != ZKV_OK && st[1] != 255 && st[3] == ZKV_VERIFICATION_FAILED)) {
-            char msg[160]; snprintf(msg, sizeof msg, "zkv_self_test: kernels (layout %d) returned statuses %d %d %d %d for the reference's golden proofs and their tampers; expected 0, reject, 0, 1", layout, st[0], st[1], st[2], st[3]);
+            char msg[160]; snprintf(msg, sizeof msg, "zkv_self_test: kernels returned statuses %d %d %d %d for the reference's golden proofs and their tampers; expected 0, reject, 0, 1", st[0], st[1], st[2], st[3]);
             rc = fail(ZKV_ERR_STATE, msg);
         }
     }
@@ -1045,32 +1021,23 @@ extern "C" int zkv_self_test(int device) {
     return rc;
 }
 // ------------------------------------------------------------------------------------------ pairing service (0x08 seam)
-static int pairing4_chain(DevCtx* c, const zkv_vk* vk, size_t o, int n, const uint8_t* d_g1s, const uint8_t* d_g2s, uint8_t* d_ok, uint8_t* d_gt, uint8_t* d_miller, cudaStream_t s, bool timed) {
+static int pairing4_chain(DevCtx* c, size_t o, int n, const uint8_t* d_g1s, const uint8_t* d_g2s, uint8_t* d_ok, uint8_t* d_gt, uint8_t* d_miller, cudaStream_t s, bool timed) {
     uint8_t* flags = c->flags + o;
     if (timed) CK(cudaEventRecord(c->ev[0], s));
     k_g1_decode4<<<nblk(n), TPB, 0, s>>>(n, d_g1s + o * 256, d_g2s + o * 128, c->px[0] + o, c->py[0] + o, c->px[1] + o, c->py[1] + o, c->px[2] + o, c->py[2] + o, c->px[3] + o, c->py[3] + o, c->qx + o, c->qy + o, flags);
     if (timed) { CK(cudaEventRecord(c->ev[1], s)); CK(cudaEventRecord(c->ev[2], s)); }
     k_g2_check<<<nblk(n), TPB, 0, s>>>(n, c->qx + o, c->qy + o, flags);
     if (timed) CK(cudaEventRecord(c->ev[3], s));
-    MillerArgs a; memset(&a, 0, sizeof a);
-    for (int j = 0; j < 4; j++) { a.px[j] = c->px[j] + o; a.py[j] = c->py[j] + o; }
-    a.qx = c->qx + o; a.qy = c->qy + o;
-    for (int j = 0; j < 3; j++) a.tabs[j] = c->d_lines + (size_t)j * ZKV_LINES_PER_G2;
-    a.nfixed = 3; a.pre = nullptr;
-    a.skip_bit[0] = F_SKIP0; a.skip_bit[1] = 0x20; a.skip_bit[2] = 0x40; a.skip_bit[3] = 0x80;
-    a.vk_skip = (uint8_t)((c->h_vk.g2_inf[0] ? 2 : 0) | (c->h_vk.g2_inf[1] ? 4 : 0) | (c->h_vk.g2_inf[2] ? 8 : 0));
-    const bool lazy = vk->tune.layout.load() != 0;
-    if (lazy) {                 // shared-memory-resident general Miller loop: one variable pair + the three tabled key points, unscaled lines (the oracle's Miller value)
-        k_pairing4_skip<<<nblk(n), TPB, 0, s>>>(n, c->stride, flags, a.vk_skip, c->pskip + o);
-        LzGenIn gi; memset(&gi, 0, sizeof gi);
-        gi.px = c->px[0] + o; gi.py = c->py[0] + o; gi.qx = c->qx + o; gi.qy = c->qy + o; gi.rst = c->rst + o; gi.pskip = c->pskip + o; gi.stride = c->stride; gi.nvar = 1; gi.nfix = 3;
-        for (int j = 0; j < 3; j++) gi.tabs[j] = a.tabs[j];
-        k_pairing_lz<<<nblk(n, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s>>>(n, gi, c->f + o, ZKV_ATE_NAF_LEN - 2, 0, 1, 1);
-    } else k_miller<<<nblk(n, ZKV_HTPB), ZKV_HTPB, 0, s>>>(n, a, flags, c->f + o);
+    // shared-memory-resident general Miller loop: one variable pair + the three tabled key points, unscaled lines (the oracle's Miller value)
+    const uint8_t vk_skip = (uint8_t)((c->h_vk.g2_inf[0] ? 2 : 0) | (c->h_vk.g2_inf[1] ? 4 : 0) | (c->h_vk.g2_inf[2] ? 8 : 0));
+    k_pairing4_skip<<<nblk(n), TPB, 0, s>>>(n, c->stride, flags, vk_skip, c->pskip + o);
+    LzGenIn gi; memset(&gi, 0, sizeof gi);
+    gi.px = c->px[0] + o; gi.py = c->py[0] + o; gi.qx = c->qx + o; gi.qy = c->qy + o; gi.rst = c->rst + o; gi.pskip = c->pskip + o; gi.stride = c->stride; gi.nvar = 1; gi.nfix = 3;
+    for (int j = 0; j < 3; j++) gi.tabs[j] = c->d_lines + (size_t)j * ZKV_LINES_PER_G2;
+    k_pairing_lz<<<nblk(n, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s>>>(n, gi, c->f + o, ZKV_ATE_NAF_LEN - 2, 0, 1, 1);
     if (timed) CK(cudaEventRecord(c->ev[4], s));
     if (d_miller) k_f12_to_bytes<<<nblk(n), TPB, 0, s>>>(n, c->f + o, d_miller + o * 384);
-    if (lazy) k_final_exp_lz<<<nblk(n, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s>>>(n, 0, 3, c->f + o, c->fes + 6 * o, flags, d_ok + o, d_gt ? d_gt + o * 384 : nullptr, 1);
-    else k_final_exp<<<nblk(n, ZKV_HTPB_FE), ZKV_HTPB_FE, 0, s>>>(n, c->f + o, flags, d_ok + o, d_gt ? d_gt + o * 384 : nullptr, 1);
+    k_final_exp_lz<<<nblk(n, LZ_NT), LZ_NT, LZ_SMEM_BYTES, s>>>(n, 0, 3, c->f + o, c->fes + 6 * o, flags, d_ok + o, d_gt ? d_gt + o * 384 : nullptr, 1);
     if (timed) CK(cudaEventRecord(c->ev[5], s));
     CK(cudaGetLastError());
     return 0;
@@ -1088,8 +1055,8 @@ static int run_pairing4(DevCtx* c, const zkv_vk* vk, size_t n_, const uint8_t* d
     // the pairing service's chunks carry their own decode / G2-check kernels: from two waves on one serial chain is the faster schedule here
     // (2^22 instances: 1.70 M against 1.63 M instances/s with four chunks)
     if (vk->tune.overlap_chunks.load() == 0 && n_ >= 2 * wave_proofs_of(c)) chunks = 1;
-    if (chunks <= 1) return pairing4_chain(c, vk, 0, (int)n_, d_g1s, d_g2s, d_ok, d_gt, d_miller, s, true);
-    return fork_join(c, s, n_, chunks, [&](size_t o, int m, cudaStream_t st) { return pairing4_chain(c, vk, o, m, d_g1s, d_g2s, d_ok, d_gt, d_miller, st, false); });
+    if (chunks <= 1) return pairing4_chain(c, 0, (int)n_, d_g1s, d_g2s, d_ok, d_gt, d_miller, s, true);
+    return fork_join(c, s, n_, chunks, [&](size_t o, int m, cudaStream_t st) { return pairing4_chain(c, o, m, d_g1s, d_g2s, d_ok, d_gt, d_miller, st, false); });
 }
 extern "C" int zkv_pairing4_batch(const zkv_vk* vk, const uint8_t* g1s, const uint8_t* g2s, size_t n, uint8_t* ok_out, uint8_t* gt_out, uint8_t* miller_out) {
     if (!vk || (n && (!g1s || !g2s || !ok_out))) return fail(ZKV_ERR_ARG, "zkv_pairing4_batch: null argument");
@@ -1293,7 +1260,7 @@ extern "C" int zkv_last_stage_ms(const void* handle_vk, int device, float* out, 
 extern "C" const void* zkv_risc0_vk(const zkv_risc0* h) { return h ? h->vk : nullptr; }
 extern "C" const void* zkv_sp1_vk(const zkv_sp1* h) { return h ? h->vk : nullptr; }
 
-// proofs in one full wave of a heavy kernel on `device` (SMs x resident blocks per SM x threads per block): 0 = k_miller_norm, 1 = k_final_exp
+// proofs in one full wave of a heavy kernel on `device` (SMs x resident blocks per SM x threads per block): 0 = k_miller_lz, 1 = k_final_exp_lz
 extern "C" long long zkv_wave_proofs(int device, int kernel) {
     if (zkv_device_count() <= device || device < 0) return fail(ZKV_ERR_CUDA, "no such CUDA device");
     if (cudaSetDevice(device) != cudaSuccess) return fail(ZKV_ERR_CUDA, "cudaSetDevice failed");
@@ -1303,9 +1270,7 @@ extern "C" long long zkv_wave_proofs(int device, int kernel) {
     switch (kernel) {
         case 0: tpb = LZ_NT; cudaFuncSetAttribute(k_miller_lz, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_MILLER); e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_miller_lz, LZ_NT, LZ_SMEM_MILLER); break;
         case 1: tpb = LZ_NT; cudaFuncSetAttribute(k_final_exp_lz, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_BYTES); e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_final_exp_lz, LZ_NT, LZ_SMEM_BYTES); break;
-        case 2: tpb = ZKV_HTPB_MILLER; e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_miller_norm, ZKV_HTPB_MILLER, 0); break;
-        case 3: tpb = ZKV_HTPB_FE; e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_final_exp, ZKV_HTPB_FE, 0); break;
-        default: return fail(ZKV_ERR_ARG, "zkv_wave_proofs: kernel");
+        default: return fail(ZKV_ERR_ARG, "zkv_wave_proofs: kernel must be 0 or 1 (2 and 3, the round-1 kernels, were removed)");
     }
     if (e != cudaSuccess) return fail(ZKV_ERR_CUDA, cudaGetErrorString(e));
     return (long long)prop.multiProcessorCount * per_sm * tpb;

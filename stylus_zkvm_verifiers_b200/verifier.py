@@ -96,7 +96,8 @@ class VerificationKey:
         return dict(zip(("decode_hash", "vk_x", "g2_check", "miller", "final_exp"), list(out)[:max(n, 0)]))
 
     def tune(self, option, value=None):
-        """Per-key tuning (overlap, normalised_lines, miller_segments, final_exp_stages, layout); returns the previous value."""
+        """Per-key tuning (overlap, miller_segments, final_exp_stages); returns the previous value.  normalised_lines and layout are
+        fixed at 1: they read 1, and setting 0 raises ZkvError (the round-1 kernels and the unscaled verification lines were removed)."""
         return _tune(self._h, option, value)
 
 
@@ -446,8 +447,7 @@ def device_count():
 
 
 def wave_proofs(device, kernel):
-    """Proofs in one full wave of the verification Miller-loop kernel (kernel 0) or the final exponentiation (kernel 1) on `device`;
-    2 / 3 = the same for the round-1 layout."""
+    """Proofs in one full wave of the verification Miller-loop kernel (kernel 0) or the final exponentiation (kernel 1) on `device`."""
     w = int(N.lib().zkv_wave_proofs(int(device), int(kernel)))
     if w <= 0:
         N.check(w if w < 0 else N.ZKV_ERR_CUDA)

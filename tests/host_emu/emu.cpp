@@ -25,7 +25,7 @@ int emu_final_exp_staged(const uint8_t* a, uint8_t* out) {
 }
 // 1 = in G2, 0 = on twist but not in G2, 2 = not on twist / bad encoding
 int emu_g2_check(const uint8_t* q) { fp2 x, y; if (!dec_g2(x, y, q)) return 2; if (!g2_on_curve(x, y)) return 2; return g2_in_subgroup(x, y) ? 1 : 0; }
-// 4-pair Miller loop + final exp the way k_miller does it: pair 0 variable G2, pairs 1..3 from line tables of the three fixed points
+// 4-pair Miller loop + final exp with bn254.cuh's thread-stack routines: pair 0 variable G2, pairs 1..3 from line tables of the three fixed points
 int emu_pairing4(const uint8_t* g1s /*4x64*/, const uint8_t* g2 /*128*/, const uint8_t* fixed /*3x128*/, uint8_t* miller_out, uint8_t* gt_out) {
     static line_t tabs_store[3][ZKV_LINES_PER_G2];
     fp px[4], py[4];

@@ -1,7 +1,7 @@
 """The G2 subgroup test finished by the shared-memory Miller kernels (k_g2_target + the last segment of k_miller_lz / k_miller_lz_keys)
 against the CPU oracle: 2^16 proofs under a RISC Zero-shape and an SP1-shape key, a part of them with B on the twist but outside G2
 (random points, G2 + small-order points, small-order points), some of those with A or vk_x at infinity, through the single chain, the
-chunked schedule, the key-set calls (host buffers and device form) and the round-1 layout, which keeps the stand-alone k_g2_check."""
+chunked schedule and the key-set calls (host buffers and device form)."""
 import numpy as np
 import pytest
 
@@ -90,10 +90,9 @@ def _single(Z, kv, key):
     return Z.Groth16Verifier.verify_batch(kv, b"".join(key["prs"]), b"".join(w32(v) for s in key["sigs"] for v in s), vk.k, len(key["prs"]))
 
 
-@pytest.mark.parametrize("overlap,layout", [(1, 1), (4, 1), (0, 1), (1, 0), (4, 0)])
+@pytest.mark.parametrize("overlap,layout", [(1, 1), (4, 1), (0, 1)])
 def test_single_key_paths(Z, batch, overlap, layout):
-    """overlap 1: one chain (k_g2_target, one Miller launch); 4 / 0 (automatic at 2^15): four chunks, four Miller segments each;
-    layout 0: the round-1 kernels behind the stand-alone k_g2_check"""
+    """overlap 1: one chain (k_g2_target, one Miller launch); 4 / 0 (automatic at 2^15): four chunks, four Miller segments each"""
     for key in batch:
         kv = _load(Z, key["vk"])
         kv.tune("overlap", overlap)

@@ -255,9 +255,9 @@ def test_risc0_shape_mixed_batch_vs_oracle(Z, gpu, fx, seed):
     assert len(set(got)) >= 4          # OK, INVALID_PROOF_DATA, SELECTOR_MISMATCH, VERIFICATION_FAILED all occur
 
 
-def test_normalised_and_unscaled_lines_agree(Z, gpu, fx):
+def test_normalised_lines_match_oracle(Z, gpu, fx):
     """The verification path scales the gamma / delta lines by subfield elements (10 instead of 13 Fp2 products per line): every status
-    byte must equal both the oracle's and the one obtained with the unscaled lines of the pairing service."""
+    byte must equal the oracle's.  The unscaled-line and round-1 kernels are gone: their options read 1 and refuse 0."""
     from stylus_zkvm_verifiers_b200 import synth as S
     vk = S.make_vk(gpu, 0, 6, 0xB2000009)
     kv = Z.VerificationKey(0, vk.alpha, vk.beta, vk.gamma, vk.delta, vk.ic)
@@ -267,17 +267,19 @@ def test_normalised_and_unscaled_lines_agree(Z, gpu, fx):
     S.mutate_risc0(batch, gpu, S.SplitMix64(0xB200000A))
     ro = O.Risc0Oracle(oracle_vk(vk)); ro.initialize(fx["control_root"], fx["bn254_control_id"])
     want = ro.verify_batch(batch.seals, batch.image_ids, batch.journals)
-    assert v.tune("normalised_lines") == 1 and v.tune("layout") == 1          # the defaults; tuning is per key, not process-wide
+    assert v.tune("normalised_lines") == 1 and v.tune("layout") == 1          # fixed at 1
+    assert v.tune("normalised_lines", 1) == 1 and v.tune("layout", 1) == 1
     a = v.verify_batch(batch.seals, batch.image_ids, batch.journals)          # shared-memory kernels, normalised lines
-    v.tune("layout", 0)
-    a0 = v.verify_batch(batch.seals, batch.image_ids, batch.journals)         # round-1 kernels, normalised lines
-    v.tune("normalised_lines", 0)
-    b = v.verify_batch(batch.seals, batch.image_ids, batch.journals)          # round-1 kernels, unscaled lines (the pairing service's loop)
-    v.tune("layout", 1)
-    b1 = v.verify_batch(batch.seals, batch.image_ids, batch.journals)         # unscaled lines + shared-memory final exponentiation
-    assert a.tolist() == want.tolist() and b.tolist() == want.tolist() and a0.tolist() == want.tolist() and b1.tolist() == want.tolist()
+    assert a.tolist() == want.tolist()
+    for opt in ("layout", "normalised_lines"):
+        with pytest.raises(Z.ZkvError) as e:
+            v.tune(opt, 0)
+        assert e.value.code == -1
+        assert v.tune(opt) == 1
+        assert v.verify_batch(batch.seals, batch.image_ids, batch.journals).tolist() == want.tolist()
+    v.tune("miller_segments", 2)                                              # tuning is per key, not process-wide
     other = Z.RiscZeroVerifier(Z.VerificationKey(0, vk.alpha, vk.beta, vk.gamma, vk.delta, vk.ic))
-    assert other.tune("normalised_lines") == 1                                # another key handle keeps its own settings
+    assert other.tune("miller_segments") == 4 and v.tune("miller_segments") == 2   # another key handle keeps its own settings
     assert 0 < int((want == 0).sum()) < n
 
 
@@ -444,28 +446,28 @@ def test_segmented_miller_loop_matches(Z, gpu, fx):
     ro = O.Risc0Oracle(oracle_vk(vk)); ro.initialize(fx["control_root"], fx["bn254_control_id"])
     sub = 600
     want = ro.verify_batch(batch.seals[:sub], batch.image_ids[:sub], batch.journals[:sub])
-    for layout in (1, 0):                                  # shared-memory kernels (default), round-1 kernels
-        v.tune("layout", layout)
-        v.tune("miller_segments", 1)
-        base = v.verify_batch(batch.seals, batch.image_ids, batch.journals)
-        assert base[:sub].tolist() == want.tolist(), layout
-        for segs in (2, 4, 7):
-            v.tune("miller_segments", segs)
-            assert v.verify_batch(batch.seals, batch.image_ids, batch.journals).tolist() == base.tolist(), (layout, segs)
-        for fe in (0, 1):                                  # one-kernel / staged final exponentiation
-            v.tune("final_exp_stages", fe)
-            assert v.verify_batch(batch.seals, batch.image_ids, batch.journals).tolist() == base.tolist(), (layout, "fe", fe)
+    v.tune("miller_segments", 1)                           # the shared-memory kernels k_miller_lz / k_final_exp_lz
+    base = v.verify_batch(batch.seals, batch.image_ids, batch.journals)
+    assert base[:sub].tolist() == want.tolist()
+    for segs in (2, 4, 7):
+        v.tune("miller_segments", segs)
+        assert v.verify_batch(batch.seals, batch.image_ids, batch.journals).tolist() == base.tolist(), segs
+    for fe in (0, 1):                                      # one-kernel / staged final exponentiation
+        v.tune("final_exp_stages", fe)
+        assert v.verify_batch(batch.seals, batch.image_ids, batch.journals).tolist() == base.tolist(), ("fe", fe)
 
 
 @pytest.mark.gpu
 def test_launch_counter_and_wave_size(Z, gpu, fx):
     """zkv_launch_count counts every kernel of the verification chains (bench.py's gpu_launches); zkv_wave_proofs is SMs x resident blocks
-    x 128 threads: two blocks per SM for the shared-memory Miller / final-exponentiation kernels, three / two for the round-1 kernels."""
+    x 128 threads: two blocks per SM for the shared-memory Miller / final-exponentiation kernels; 2 and 3 (the round-1 kernels) are gone."""
     import torch
     from stylus_zkvm_verifiers_b200 import synth as S
     sms = torch.cuda.get_device_properties(0).multi_processor_count
     assert Z.wave_proofs(0, 0) == sms * 2 * 128 and Z.wave_proofs(0, 1) == sms * 2 * 128
-    assert Z.wave_proofs(0, 2) == sms * 3 * 128 and Z.wave_proofs(0, 3) == sms * 2 * 128
+    for kernel in (2, 3):
+        with pytest.raises(Z.ZkvError):
+            Z.wave_proofs(0, kernel)
     vk = S.make_vk(gpu, 0, 6, 0xB200000D)
     kv = Z.VerificationKey(0, vk.alpha, vk.beta, vk.gamma, vk.delta, vk.ic)
     v = Z.RiscZeroVerifier(kv); v.initialize(fx["control_root"], fx["bn254_control_id"])
