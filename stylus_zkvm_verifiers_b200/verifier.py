@@ -402,7 +402,9 @@ def fp_mul_batch(a, b, n, device=0):
 
 
 def fp12_op_batch(op, a, b, n, device=0):
-    """Fp12 tower operation `op` (see zkv.h) on n operands of 384 bytes; b may be None for unary operations."""
+    """Fp12 tower operation `op` (see zkv.h) on n operands of 384 bytes; b may be None for unary operations.  Ops 0-9 run the round-1
+    tower (bn254.cuh); op 16 + k runs operation k on the shared-memory, lazily reduced tower of the verification kernels (lazy.cuh), plus
+    op 25 (the normalised-line product) and op 26 (the verification Miller loop on the single pair of op 9)."""
     out = C.create_string_buffer(384 * n)
     N.check(N.lib().zkv_fp12_op_batch(op, N.buf(a), N.buf(b) if b is not None else None, n, out, device))
     return out.raw

@@ -153,6 +153,108 @@ def fp12_cyc_sqr(a):
     return bytes(out.raw)
 
 
+P = 0x30644E72E131A029B85045B68181585D97816A916871CA8D3C208C16D87CFD47
+FP12_ONE = w32(1) + bytes(352)
+
+
+def fp12_words(a):
+    return [int.from_bytes(a[32 * i:32 * i + 32], "big") for i in range(12)]
+
+
+def fp12_from_words(ws):
+    return b"".join(w32(x) for x in ws)
+
+
+def fp12_conj(a):
+    """a^(p^6): c1 -> -c1 (the inverse of a unitary element)"""
+    ws = fp12_words(a)
+    return fp12_from_words(ws[:6] + [(P - x) % P for x in ws[6:]])
+
+
+def fp12_pow(a, e):
+    """a^e by left-to-right square-and-multiply over the oracle's Fp12 product (independent of every Frobenius routine)"""
+    r = FP12_ONE
+    for bit in bin(e)[2:]:
+        r = fp12_mul(r, r)
+        if bit == "1":
+            r = fp12_mul(r, a)
+    return r
+
+
+def fp12_frob(a, k):
+    """a^(p^k), k = 1, 2, 3, as k successive p-th powers"""
+    for _ in range(k):
+        a = fp12_pow(a, P)
+    return a
+
+
+# Fp words where lazily reduced arithmetic can go wrong: 0, 1, 2, p - 2, p - 1, (p -+ 1) / 2 and 2^256 mod p (the Montgomery radix)
+EDGE_WORDS = (0, 1, 2, P - 2, P - 1, (P - 1) // 2, (P + 1) // 2, (1 << 256) % P)
+
+
+def fp12_operand_classes(seed):
+    """(name, a, b) operand pairs of 12 x BE-32 Fp12 elements at the edges of the tower arithmetic, shared by the GPU and host-emulation
+    tests of csrc/lazy.cuh: all words p - 1, zero, one, -1, words drawn from EDGE_WORDS, Fp2 / Fp4 / Fp6 subfield elements, c0 = 0, c1 = 0,
+    and a second operand equal to the first or to its conjugate.  Every class appears with a random partner and with an edge partner."""
+    import random
+    rnd = random.Random(seed)
+    rand = lambda: [rnd.randrange(P) for _ in range(12)]
+    edge = lambda: [rnd.choice(EDGE_WORDS) for _ in range(12)]
+    keep = lambda ws, idx: [w if i in idx else 0 for i, w in enumerate(ws)]
+    e = fp12_from_words
+    firsts = [
+        ("all_p-1", e([P - 1] * 12)),
+        ("zero", bytes(384)),
+        ("one", FP12_ONE),
+        ("minus_one", e([P - 1] + [0] * 11)),
+        ("edge_words_a", e(edge())),
+        ("edge_words_b", e(edge())),
+        ("edge_words_c", e(edge())),
+        ("fp2_subfield", e(keep(rand(), (0, 1)))),
+        ("fp2_subfield_edge", e(keep([P - 1] * 12, (0, 1)))),
+        ("fp4_subfield", e(keep(rand(), (0, 1, 8, 9)))),            # c0.c0 + c1.c1 (v w = w^3)
+        ("fp6_subfield", e(keep(edge(), range(6)))),
+        ("c0_zero", e(keep(rand(), range(6, 12)))),
+        ("c0_zero_edge", e(keep([P - 1] * 12, range(6, 12)))),
+        ("c1_zero", e(keep(rand(), range(6)))),
+        ("random", e(rand())),
+    ]
+    out = []
+    for name, a in firsts:
+        out.append((name + "|random", a, e(rand())))
+        out.append((name + "|all_p-1", a, e([P - 1] * 12)))
+        out.append((name + "|same", a, a))
+        out.append((name + "|conj", a, fp12_conj(a)))
+    out.append(("random|edge_words", e(rand()), e(edge())))
+    out.append(("random|zero", e(rand()), bytes(384)))
+    out.append(("random|one", e(rand()), FP12_ONE))
+    out.append(("random|c0_zero", e(rand()), e(keep(rand(), range(6, 12)))))
+    return out
+
+
+def fp12_cyclotomic_operands(seed, nfrob=2):
+    """(name, g) elements of the cyclotomic subgroup, the only inputs the Granger-Scott squaring is defined on: one, the final-exponentiation
+    outputs of the nonzero operand classes (the subfield ones map to one), their conjugates, and Frobenius images of `nfrob` of them"""
+    seen, out = {FP12_ONE}, [("one", FP12_ONE)]
+
+    def add(name, g):
+        if g not in seen:
+            seen.add(g); out.append((name, g))
+    gts = []
+    for name, a, _ in fp12_operand_classes(seed):
+        if a != bytes(384):
+            g = final_exp(a)
+            if g not in seen:
+                gts.append((name.split("|")[0], g))
+            add("final_exp(%s)" % name.split("|")[0], g)
+    for name, g in gts:
+        add("conj(final_exp(%s))" % name, fp12_conj(g))
+    for name, g in gts[-nfrob:]:
+        for k in (1, 2, 3):
+            add("final_exp(%s)^(p^%d)" % (name, k), fp12_frob(g, k))
+    return out
+
+
 def ate_naf():
     buf = (C.c_int8 * 80)()
     n = lib().zkvo_ate_naf(buf, 80)

@@ -172,6 +172,39 @@ def test_lazy_tower_on_slots_matches_round1_tower(emu):
         emu.emu_lz_f12sqr(x, o12); assert o12.raw == O.fp12_mul(x, x), it
 
 
+def test_lazy_fp12_routines_match_oracle(emu):
+    """The Fp12-level routines of csrc/lazy.cuh on slots, over the operand classes of oracle_lib.fp12_operand_classes (all p - 1, zero,
+    one, -1, edge words, subfield elements, c0 = 0, c1 = 0, b = a, b = conj(a)): lz_f12mul_g plain and conjugated against the oracle and the
+    round-1 tower, lz_f12inv by its product with the operand (inv(0) = 0), lz_frob against the round-1 Frobenius and, on some operands,
+    against a^(p^k) by square-and-multiply, lz_cyc_sqr on cyclotomic elements only, the staged lz_final_exp_stage against the oracle."""
+    mul, mulc, inv, csq, rmulc, fe = (C.create_string_buffer(384) for _ in range(6))
+    fr, rfr = C.create_string_buffer(3 * 384), C.create_string_buffer(3 * 384)
+    firsts = {}
+    for name, a, b in O.fp12_operand_classes(31):
+        emu.emu_lz_f12_ops(a, b, mul, mulc, inv, csq, fr)
+        emu.emu_f12_misc(a, b, rmulc, rfr)
+        assert mul.raw == O.fp12_mul(a, b), name
+        assert mulc.raw == rmulc.raw == O.fp12_mul(a, O.fp12_conj(b)), name
+        if a == bytes(384):
+            assert inv.raw == bytes(384), name
+        else:
+            assert O.fp12_mul(a, inv.raw) == O.FP12_ONE, name
+        assert fr.raw == rfr.raw, name
+        firsts.setdefault(a, (name.split("|")[0], fr.raw))
+    for a, (name, frs) in list(firsts.items())[::2]:
+        x = a
+        for k in range(3):
+            x = O.fp12_frob(x, 1)
+            assert frs[384 * k:384 * k + 384] == x, (name, k + 1)
+    for a, (name, _) in firsts.items():
+        emu.emu_lz_final_exp(a, fe)
+        assert fe.raw == O.final_exp(a), name
+    for name, g in O.fp12_cyclotomic_operands(31):
+        emu.emu_lz_f12_ops(g, g, mul, mulc, inv, csq, fr)
+        assert csq.raw == O.fp12_cyc_sqr(g) == O.fp12_mul(g, g), name
+        assert mulc.raw == O.FP12_ONE, name                          # g * conj(g) = 1 on the cyclotomic subgroup
+
+
 def test_lazy_miller_loop_bit_exact_with_round1_loop(emu, consts):
     """lz_miller_norm_seg (one and several segments, pairs switched off) reproduces miller_loop_norm's Fp12 value bit for bit."""
     rng = SplitMix64(21)
