@@ -136,6 +136,51 @@ int zkv_risc0_verify_batch_device(const zkv_risc0* h, int device, const void* d_
 int zkv_sp1_verify_batch_device(const zkv_sp1* h, int device, const void* d_vkeys, const void* d_public_values, size_t pv_stride,
                                 const void* d_proofs260, size_t n, void* d_status_out, void* stream);
 
+/* An SP1 handle for another verifier version (sp1/config.rs:4-9,18-20): its own key (vk = NULL -> the embedded v5 key, as
+ * zkv_sp1_create), verifier hash (the selector is its first 4 bytes) and version string, both copied; zkv_sp1_verifier_hash and
+ * zkv_sp1_version return them.  ZKV_ERR_ARG for a null hash or version, or a key that is not ZKV_VM_SP1 with 3 IC points. */
+int zkv_sp1_create_version(const zkv_vk* vk_or_null, const uint8_t verifier_hash[32], const char* version,
+                           const int* devices, int n_dev, zkv_sp1** out);
+
+/* ---- routers: many verifier versions in one batch, routed by selector -----------------------------------
+ * RiscZeroVerifierRouter (forwards bytes4(seal[0:4]) to the verifier registered under it) and SP1VerifierGateway (proofBytes[:4]).
+ * A router is built from 1..256 verifier handles of one kind and BORROWS them: they must outlive it.  At creation it takes a
+ * snapshot of each handle's selector and per-proof constants (handles cannot change after zkv_risc0_initialize).  Every route's key
+ * must be loaded on every device of the router (devices == NULL -> device 0).
+ * Creation returns ZKV_ERR_ARG for 0 or more than 256 handles, a null handle, two handles with the same selector (SelectorInUse),
+ * a handle of the other kind, or a route key missing on a router device; ZKV_ERR_STATE for an uninitialised RISC Zero handle.
+ *
+ * Record i is verified by the route whose selector equals its first 4 bytes; status_out[i] is what zkv_risc0_verify[_integrity] /
+ * zkv_sp1_verify_proof on that route's handle returns for it alone: a record shorter than 4 bytes -> ZKV_INVALID_PROOF_DATA; no route
+ * has its selector -> ZKV_SELECTOR_MISMATCH (what every route handle would return: in a router call it means exactly "no route");
+ * routed, length != 260 -> ZKV_INVALID_PROOF_DATA; routed to a handle whose key has an invalid point, or a RISC Zero handle whose
+ * bn254_control_id >= r -> ZKV_VERIFICATION_FAILED; otherwise the Groth16 verification under the route's key.  Argument layouts are
+ * those of the matching single-handle calls; null pointers and decreasing offsets return ZKV_ERR_ARG with status_out untouched, and
+ * n == 0 does nothing.  A multi-device router splits the batch into contiguous caller ranges.
+ * Each device pass (up to 2^20 records) is routed and grouped by route on the device; its kernel launches do not depend on the
+ * number of routes (zkv_launch_count: 11 for a pass of one kernel chain, 42 once the slot bound n + 31 x min(n_routes, n) reaches the
+ * automatic chunking threshold of ZKV_TUNE_OVERLAP: the key-set pass plus the routing kernel).  A router runs the default schedule;
+ * the route keys' zkv_vk_tune settings do not apply to it.
+ * The _device forms take the fixed 260-byte records of zkv_risc0_verify_batch_device / zkv_sp1_verify_batch_device on one router
+ * device, n <= 2^23, enqueued on `stream` (a cudaStream_t), asynchronous. */
+typedef struct zkv_risc0_router zkv_risc0_router;
+int zkv_risc0_router_create(const zkv_risc0* const* verifiers, int n, const int* devices, int n_dev, zkv_risc0_router** out);
+void zkv_risc0_router_destroy(zkv_risc0_router* r);
+int zkv_risc0_router_verify_batch(const zkv_risc0_router* r, const uint8_t* seals, const uint64_t* seal_off, const uint8_t* image_ids,
+                                  const uint8_t* journal_digests, size_t n, uint8_t* status_out);
+int zkv_risc0_router_verify_integrity_batch(const zkv_risc0_router* r, const uint8_t* seals, const uint64_t* seal_off,
+                                            const uint8_t* claim_digests, size_t n, uint8_t* status_out);
+int zkv_risc0_router_verify_batch_device(const zkv_risc0_router* r, int device, const void* d_seals260, const void* d_image_ids,
+                                         const void* d_journal_digests, size_t n, void* d_status_out, void* stream);
+
+typedef struct zkv_sp1_gateway zkv_sp1_gateway;
+int zkv_sp1_gateway_create(const zkv_sp1* const* verifiers, int n, const int* devices, int n_dev, zkv_sp1_gateway** out);
+void zkv_sp1_gateway_destroy(zkv_sp1_gateway* g);
+int zkv_sp1_gateway_verify_batch(const zkv_sp1_gateway* g, const uint8_t* vkeys, const uint8_t* public_values, const uint64_t* pv_off,
+                                 const uint8_t* proofs, const uint64_t* proof_off, size_t n, uint8_t* status_out);
+int zkv_sp1_gateway_verify_batch_device(const zkv_sp1_gateway* g, int device, const void* d_vkeys, const void* d_public_values,
+                                        size_t pv_stride, const void* d_proofs260, size_t n, void* d_status_out, void* stream);
+
 /* ---- pairing service (the 0x08 seam, common/groth16.rs:109-128) ---------------------------
  * n instances of a 4-pair product check e(P0,Q) e(P1,beta) e(P2,gamma) e(P3,delta) == 1 with the three
  * fixed G2 points taken from `vk`.  g1s: n x 4 x 64 B, g2s: n x 128 B.  ok_out[i] = 1 / 0, or 2 if the

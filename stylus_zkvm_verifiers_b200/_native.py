@@ -45,6 +45,16 @@ _SIGS = {
     "zkv_sp1_verify_proof": (C.c_int, [_P, _P, _P, C.c_size_t, _P, C.c_size_t, _P]),
     "zkv_risc0_verify_batch_device": (C.c_int, [_P, C.c_int, _P, _P, _P, C.c_size_t, _P, _P]),
     "zkv_sp1_verify_batch_device": (C.c_int, [_P, C.c_int, _P, _P, C.c_size_t, _P, C.c_size_t, _P, _P]),
+    "zkv_sp1_create_version": (C.c_int, [_P, _P, C.c_char_p, _P, C.c_int, C.POINTER(_P)]),
+    "zkv_risc0_router_create": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(_P)]),
+    "zkv_risc0_router_destroy": (None, [_P]),
+    "zkv_risc0_router_verify_batch": (C.c_int, [_P, _P, _P, _P, _P, C.c_size_t, _P]),
+    "zkv_risc0_router_verify_integrity_batch": (C.c_int, [_P, _P, _P, _P, C.c_size_t, _P]),
+    "zkv_risc0_router_verify_batch_device": (C.c_int, [_P, C.c_int, _P, _P, _P, C.c_size_t, _P, _P]),
+    "zkv_sp1_gateway_create": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(_P)]),
+    "zkv_sp1_gateway_destroy": (None, [_P]),
+    "zkv_sp1_gateway_verify_batch": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
+    "zkv_sp1_gateway_verify_batch_device": (C.c_int, [_P, C.c_int, _P, _P, C.c_size_t, _P, C.c_size_t, _P, _P]),
     "zkv_pairing4_batch": (C.c_int, [_P, _P, _P, C.c_size_t, _P, _P, _P]),
     "zkv_pairing4_batch_device": (C.c_int, [_P, C.c_int, _P, _P, C.c_size_t, _P, _P, _P]),
     "zkv_ec_pairing_batch": (C.c_int, [_P, C.c_int, C.c_size_t, _P, _P, _P, C.c_int]),

@@ -89,18 +89,25 @@ __device__ __forceinline__ void decode_points(int i, const uint8_t* p, int vm, f
     if (rc == 1) fl |= F_SKIPC;
     flags[i] = fl;
 }
+// record i of a batch and its length: fixed-stride records, or (rec_off != nullptr) the caller's concatenated blobs
+__device__ __forceinline__ const uint8_t* record_of(int i, const uint8_t* recs, size_t stride, const uint64_t* rec_off, uint64_t rec_base, uint64_t& len) {
+    const uint8_t* rec = rec_off ? recs + (size_t)(rec_off[i] - rec_base) : recs + (size_t)i * stride;
+    len = rec_off ? rec_off[i + 1] - rec_off[i] : (uint64_t)stride;
+    return rec;
+}
+// the selector (first 4 bytes) of a record, little-endian
+__device__ __forceinline__ uint32_t selector_of(const uint8_t* rec) { return (uint32_t)rec[0] | (uint32_t)rec[1] << 8 | (uint32_t)rec[2] << 16 | (uint32_t)rec[3] << 24; }
 __global__ void k_decode(int n, const uint8_t* recs, size_t stride, size_t off, uint32_t selector_le, int check_selector, int vm,
                          const uint64_t* rec_off, uint64_t rec_base,
                          fp* ax, fp* ay, fp2* bx, fp2* by, fp* cx, fp* cy, uint8_t* flags) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const uint8_t* rec = rec_off ? recs + (size_t)(rec_off[i] - rec_base) : recs + (size_t)i * stride;
-    const uint64_t len = rec_off ? rec_off[i + 1] - rec_off[i] : (uint64_t)stride;
+    uint64_t len;
+    const uint8_t* rec = record_of(i, recs, stride, rec_off, rec_base, len);
     uint8_t fl = 0;
     if (rec_off && len < 4) fl = F_BADDATA;
     else if (check_selector) {
-        uint32_t s = (uint32_t)rec[0] | (uint32_t)rec[1] << 8 | (uint32_t)rec[2] << 16 | (uint32_t)rec[3] << 24;
-        if (s != selector_le) fl = F_SELMIS;
+        if (selector_of(rec) != selector_le) fl = F_SELMIS;
     }
     if (rec_off && !fl && len != off + 256) fl = F_BADDATA;
     if (fl) { decode_reject(i, fl, ax, ay, bx, by, cx, cy, flags); return; }
@@ -111,39 +118,48 @@ __global__ void k_decode(int n, const uint8_t* recs, size_t stride, size_t off, 
 // claim_lo / claim_hi are the little-endian readings of claim[0..16) / claim[16..32).
 // mode 0: claim = ReceiptClaim::ok(image_id, journal).digest(); mode 1: claim digest supplied (verify_integrity).
 struct Risc0HashConsts { uint32_t tag_out[8], claim_mid[8], sys0[8]; };
-__global__ void k_risc0_signals(int n, const uint8_t* image_ids, const uint8_t* journals, const uint8_t* claims, int mode,
-                                Risc0HashConsts hc, uint32_t* scal /* [n][2][8] */) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+// signals 2 and 3 of record p (its 32-byte inputs at p) into the 16 scalar words of slot i (k_risc0_signals, k_risc0_signals_route)
+__device__ __forceinline__ void risc0_signals_one(int p, int i, const uint8_t* image_ids, const uint8_t* journals, const uint8_t* claims, int mode,
+                                                  const Risc0HashConsts& hc, uint32_t* scal) {
     uint32_t claim[8];
     if (mode == 0) {
         uint32_t im[8], jr[8];
-        for (int k = 0; k < 8; k++) { im[k] = load_be32(image_ids + 32 * (size_t)i + 4 * k); jr[k] = load_be32(journals + 32 * (size_t)i + 4 * k); }
+        for (int k = 0; k < 8; k++) { im[k] = load_be32(image_ids + 32 * (size_t)p + 4 * k); jr[k] = load_be32(journals + 32 * (size_t)p + 4 * k); }
         risc0_claim_digest(claim, im, jr, hc.tag_out, hc.claim_mid, hc.sys0);
     } else {
-        for (int k = 0; k < 8; k++) claim[k] = load_be32(claims + 32 * (size_t)i + 4 * k);
+        for (int k = 0; k < 8; k++) claim[k] = load_be32(claims + 32 * (size_t)p + 4 * k);
     }
     uint32_t* o = scal + (size_t)i * 16;
     for (int k = 0; k < 4; k++) { o[k] = __byte_perm(claim[k], 0, 0x0123); o[8 + k] = __byte_perm(claim[4 + k], 0, 0x0123); o[4 + k] = 0; o[12 + k] = 0; }
 }
+__global__ void k_risc0_signals(int n, const uint8_t* image_ids, const uint8_t* journals, const uint8_t* claims, int mode,
+                                Risc0HashConsts hc, uint32_t* scal /* [n][2][8] */) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    risc0_signals_one(i, i, image_ids, journals, claims, mode, hc, scal);
+}
 
 // K4: SP1 public signals (sp1/types.rs:21-38): s0 = U256_be(program_vkey), s1 = SHA256(pv) & (2^253 - 1).
 // A signal >= R makes the proof fail (groth16.rs:32-34); only s0 can be.
-__global__ void k_sp1_signals(int n, const uint8_t* vkeys, const uint8_t* pv, const uint64_t* pv_off, uint64_t pv_base, size_t pv_stride,
-                              uint32_t* scal /* [n][2][8] */, uint8_t* flags) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    uint32_t* o = scal + (size_t)i * 16;
+// signals of record p (vkey at p, public values p of pv) into the 16 scalar words at o; *fl gets F_INVALID (k_sp1_signals, k_sp1_signals_route)
+__device__ __forceinline__ void sp1_signals_one(int p, const uint8_t* vkeys, const uint8_t* pv, const uint64_t* pv_off, uint64_t pv_base, size_t pv_stride,
+                                                uint32_t* o, uint8_t* fl) {
     uint32_t s0[8];
-    be32_to_raw(s0, vkeys + 32 * (size_t)i);
-    if (u256_geq(s0, C_R)) flags[i] |= F_INVALID;
+    be32_to_raw(s0, vkeys + 32 * (size_t)p);
+    if (u256_geq(s0, C_R)) *fl |= F_INVALID;
     for (int k = 0; k < 8; k++) o[k] = s0[k];
     const uint8_t* msg; size_t len;
-    if (pv_off) { msg = pv + (size_t)(pv_off[i] - pv_base); len = (size_t)(pv_off[i + 1] - pv_off[i]); } else { msg = pv + (size_t)i * pv_stride; len = pv_stride; }
+    if (pv_off) { msg = pv + (size_t)(pv_off[p] - pv_base); len = (size_t)(pv_off[p + 1] - pv_off[p]); } else { msg = pv + (size_t)p * pv_stride; len = pv_stride; }
     uint32_t h[8];
     sha256_msg(h, msg, len);
     h[0] &= 0x1fffffffu;
     for (int k = 0; k < 8; k++) o[8 + k] = h[7 - k];
+}
+__global__ void k_sp1_signals(int n, const uint8_t* vkeys, const uint8_t* pv, const uint64_t* pv_off, uint64_t pv_base, size_t pv_stride,
+                              uint32_t* scal /* [n][2][8] */, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    sp1_signals_one(i, vkeys, pv, pv_off, pv_base, pv_stride, scal + (size_t)i * 16, flags + i);
 }
 
 // generic signals: n x k x BE-32 -> limbs; any signal >= R invalidates the proof (groth16.rs:32-34)
@@ -543,8 +559,9 @@ struct KeyDesc {                       // one key of a set on one device (device
     const g1aff* tab;                  // window tables of IC1..
     const nline_t* nt[2];              // normalised gamma / delta line tables
     const fp12* pre;                   // Miller(alpha, beta)
-    int ns, vm, reject;                // signals per proof (n_ic - 1), ZKV_VM_*, every proof fails (a key point is invalid)
+    int ns, vm, reject;                // signals per proof, ZKV_VM_*, every proof fails (a key point is invalid)
     uint8_t vk_skip;                   // pairs 1 / 2 disabled for every proof (gamma / delta at infinity), as MillerArgs::vk_skip
+    uint8_t nwin;                      // windows per scalar of vk_x (ZKV_WIN_PER_SCALAR; 32 for the 128-bit claim halves of a RISC Zero route)
 };
 __device__ __forceinline__ uint32_t group_of(uint32_t k, int nk) { return k < (uint32_t)nk ? k : 0u; }   // out-of-range keys fail in group 0
 // per tile t of ZKV_GROUP_TILE records: cnt[t * nk + k] = records of key k
@@ -651,7 +668,7 @@ __global__ void k_vkx_keys(int n, const uint32_t* perm, const uint8_t* slot_key,
     if (perm[i] == ZKV_SLOT_EMPTY) { vx[i] = fp_zero(); vy[i] = fp_zero(); return; }
     const KeyDesc* kd = keys + slot_key[i];
     const g1aff base = kd->base;
-    vkx_one(i, scal, stride, kd->ns, ZKV_WIN_PER_SCALAR, kd->tab, base, vx, vy, flags);
+    vkx_one(i, scal, stride, kd->ns, kd->nwin, kd->tab, base, vx, vy, flags);
 }
 // slots of a chunk [o, o + m) that lie in a group: the rest of the chunk is not run (whole blocks return; the last block's surplus threads
 // redo the chunk's last grouped slot, whose warp is of a single key since group sizes are multiples of 32)
@@ -673,6 +690,64 @@ __global__ void __launch_bounds__(LZ_NT, 2) k_final_exp_lz_keys(const uint32_t* 
     if ((int)blockIdx.x * LZ_NT >= n) return;
     final_exp_lz(n, s_lo, s_hi, in, st, flags, status, nullptr, 0);
 }
+// ---------------------------------------------------------------------------- routers (zkv_risc0_router, zkv_sp1_gateway)
+// A router is a key set whose key index comes from the record itself: k_route looks each record's selector up in the router's table and
+// writes its route word, which the grouping kernels read as the key index.  A record that no route verifies (shorter than 4 bytes, an
+// unknown selector, a routed length other than 4 + 256) gets ZKV_ROUTE_VERDICT | its reject flag instead: out of range, so it is grouped
+// with route 0, and k_decode_route gives it that flag, whose status (reject_status) is the one every route handle would return for it.
+#define ZKV_ROUTE_VERDICT 0x100u
+// sel[0..nr): the routes' selectors (selector_of), ascending; route r is the one with selector sel[r]
+__global__ void __launch_bounds__(256) k_route(int n, const uint8_t* recs, size_t stride, const uint64_t* rec_off, uint64_t rec_base,
+                                               const uint32_t* sel, int nr, uint32_t* route) {
+    __shared__ uint32_t t[ZKV_MAX_KEYS];
+    for (int k = threadIdx.x; k < nr; k += blockDim.x) t[k] = sel[k];
+    __syncthreads();
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint64_t len;
+    const uint8_t* rec = record_of(i, recs, stride, rec_off, rec_base, len);
+    uint32_t w = ZKV_ROUTE_VERDICT | F_BADDATA;
+    if (len >= 4) {
+        const uint32_t s = selector_of(rec);
+        int lo = 0, hi = nr;                                       // first entry >= s
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (t[mid] < s) lo = mid + 1; else hi = mid; }
+        if (lo == nr || t[lo] != s) w = ZKV_ROUTE_VERDICT | F_SELMIS;
+        else if (len == 4 + 256) w = (uint32_t)lo;
+    }
+    route[i] = w;
+}
+// k_decode in slot order for routers: record perm[s] (the 8 words at +4), the vm of its route's key; a record with a verdict gets its flag,
+// every record of a rejecting route (an invalid key point, or a RISC Zero control id >= r) F_INVALID, as k_decode + k_status_all_fail give it
+__global__ void k_decode_route(int n, const uint32_t* perm, const uint8_t* slot_key, const KeyDesc* keys, const uint32_t* route,
+                               const uint8_t* recs, size_t stride, const uint64_t* rec_off, uint64_t rec_base,
+                               fp* ax, fp* ay, fp2* bx, fp2* by, fp* cx, fp* cy, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t p = perm[i];
+    if (p == ZKV_SLOT_EMPTY) { decode_reject(i, F_INVALID, ax, ay, bx, by, cx, cy, flags); return; }
+    const uint32_t w = route[p];
+    if (w & ZKV_ROUTE_VERDICT) { decode_reject(i, (uint8_t)w, ax, ay, bx, by, cx, cy, flags); return; }
+    const KeyDesc* kd = keys + slot_key[i];
+    if (kd->reject) { decode_reject(i, F_INVALID, ax, ay, bx, by, cx, cy, flags); return; }
+    uint64_t len;
+    decode_points(i, record_of((int)p, recs, stride, rec_off, rec_base, len) + 4, kd->vm, ax, ay, bx, by, cx, cy, flags);
+}
+// k_risc0_signals / k_sp1_signals in slot order (the inputs of record perm[s])
+__global__ void k_risc0_signals_route(int n, const uint32_t* perm, const uint8_t* image_ids, const uint8_t* journals, const uint8_t* claims, int mode,
+                                      Risc0HashConsts hc, uint32_t* scal /* [n][2][8] */) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t p = perm[i];
+    if (p != ZKV_SLOT_EMPTY) risc0_signals_one((int)p, i, image_ids, journals, claims, mode, hc, scal);
+}
+__global__ void k_sp1_signals_route(int n, const uint32_t* perm, const uint8_t* vkeys, const uint8_t* pv, const uint64_t* pv_off, uint64_t pv_base, size_t pv_stride,
+                                    uint32_t* scal /* [n][2][8] */, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t p = perm[i];
+    if (p != ZKV_SLOT_EMPTY) sp1_signals_one((int)p, vkeys, pv, pv_off, pv_base, pv_stride, scal + (size_t)i * 16, flags + i);
+}
+
 // slot statuses back to caller order
 __global__ void k_status_to_caller(int n, const uint32_t* total, const uint32_t* perm, const uint8_t* slot_status, uint8_t* status) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;

@@ -610,6 +610,7 @@ struct SetDev {
     KeyDesc* d_keys = nullptr;
     uint32_t* perm = nullptr; uint8_t* slot_key = nullptr; uint8_t* slot_status = nullptr; size_t slot_cap = 0;
     uint32_t* tile = nullptr; size_t tile_cap = 0; uint32_t* total = nullptr;
+    uint32_t* d_sel = nullptr; uint32_t* route = nullptr; size_t route_cap = 0;     // routers only: the selector table, k_route's route words
 };
 struct zkv_vkset {
     std::vector<const zkv_vk*> keys;
@@ -621,30 +622,39 @@ static SetDev* set_dev(const zkv_vkset* s, int device) {
     for (auto& d : s->devs) if (d.c->device == device) return const_cast<SetDev*>(&d);
     return nullptr;
 }
-extern "C" void zkv_vkset_destroy(zkv_vkset* s) {
-    if (!s) return;
-    for (auto& d : s->devs) {
+static void setdev_free(std::vector<SetDev>& devs) {
+    for (auto& d : devs) {
         if (!d.c) continue;
         cudaSetDevice(d.c->device);
-        cudaFree(d.d_keys); cudaFree(d.perm); cudaFree(d.slot_key); cudaFree(d.slot_status); cudaFree(d.tile); cudaFree(d.total);
+        cudaFree(d.d_keys); cudaFree(d.perm); cudaFree(d.slot_key); cudaFree(d.slot_status); cudaFree(d.tile); cudaFree(d.total); cudaFree(d.d_sel); cudaFree(d.route);
         ctx_free(d.c);
     }
+}
+extern "C" void zkv_vkset_destroy(zkv_vkset* s) {
+    if (!s) return;
+    setdev_free(s->devs);
     delete s;
 }
-static int vkset_build_on(zkv_vkset* s, SetDev& sd) {
+// the KeyDesc of key vk on the device of its context kc, as a key set uses it (routers replace the vk_x part: base, tab, ns, nwin)
+static KeyDesc key_desc(const zkv_vk* vk, const DevCtx* kc) {
+    KeyDesc q; memset(&q, 0, sizeof q);
+    q.base = kc->h_ic0; q.tab = kc->d_tab; q.nt[0] = kc->d_nlines; q.nt[1] = kc->d_nlines + ZKV_LINES_PER_G2; q.pre = kc->d_pre;
+    q.ns = vk->n_ic - 1; q.vm = vk->vm; q.reject = !vk->valid;
+    q.vk_skip = (uint8_t)((kc->h_vk.g2_inf[1] ? 2 : 0) | (kc->h_vk.g2_inf[2] ? 4 : 0));
+    q.nwin = ZKV_WIN_PER_SCALAR;
+    return q;
+}
+// streams and events of sd's context, its KeyDesc array h and the slot total
+static int setdev_build(SetDev& sd, const std::vector<KeyDesc>& h) {
     int rc = ctx_init(sd.c); if (rc) return rc;
-    std::vector<KeyDesc> h(s->keys.size());
-    for (size_t k = 0; k < h.size(); k++) {
-        const zkv_vk* vk = s->keys[k];
-        const DevCtx* kc = vk_ctx(vk, sd.c->device);
-        KeyDesc& q = h[k]; memset(&q, 0, sizeof q);
-        q.base = kc->h_ic0; q.tab = kc->d_tab; q.nt[0] = kc->d_nlines; q.nt[1] = kc->d_nlines + ZKV_LINES_PER_G2; q.pre = kc->d_pre;
-        q.ns = vk->n_ic - 1; q.vm = vk->vm; q.reject = !vk->valid;
-        q.vk_skip = (uint8_t)((kc->h_vk.g2_inf[1] ? 2 : 0) | (kc->h_vk.g2_inf[2] ? 4 : 0));
-    }
     CK(cudaMalloc(&sd.d_keys, sizeof(KeyDesc) * h.size())); CK(cudaMalloc(&sd.total, sizeof(uint32_t)));
     CK(cudaMemcpy(sd.d_keys, h.data(), sizeof(KeyDesc) * h.size(), cudaMemcpyHostToDevice));
     return 0;
+}
+static int vkset_build_on(zkv_vkset* s, SetDev& sd) {
+    std::vector<KeyDesc> h;
+    for (const zkv_vk* vk : s->keys) h.push_back(key_desc(vk, vk_ctx(vk, sd.c->device)));
+    return setdev_build(sd, h);
 }
 extern "C" int zkv_vkset_create(const zkv_vk* const* keys, int n_keys, const int* devices, int n_dev, zkv_vkset** out) {
     if (!out || !keys) return fail(ZKV_ERR_ARG, "zkv_vkset_create: null argument");
@@ -675,36 +685,39 @@ extern "C" int zkv_vkset_create(const zkv_vk* const* keys, int n_keys, const int
 }
 // Slots of a pass of m records: each key present pads its group by at most 31 slots (a multiple of 32, so chunks keep whole warps)
 static size_t slot_bound(size_t m, size_t n_keys) { return (m + 31 * std::min(n_keys, m) + 31) / 32 * 32; }
-// Grow the set's grouping arrays to S slots and ntk per-tile counters; like ctx_reserve, it waits for an asynchronous user before freeing.
-static int set_reserve(SetDev* sd, size_t S, size_t ntk) {
-    if (S > sd->slot_cap || ntk > sd->tile_cap) { int rc = ctx_wait_idle(sd->c); if (rc) return rc; }
+// Grow the set's grouping arrays to S slots, ntk per-tile counters and nroute route words; like ctx_reserve, it waits for an asynchronous
+// user before freeing.
+static int set_reserve(SetDev* sd, size_t S, size_t ntk, size_t nroute) {
+    if (S > sd->slot_cap || ntk > sd->tile_cap || nroute > sd->route_cap) { int rc = ctx_wait_idle(sd->c); if (rc) return rc; }
     if (S > sd->slot_cap) {
         cudaFree(sd->perm); cudaFree(sd->slot_key); cudaFree(sd->slot_status); sd->slot_cap = 0;
         CK(cudaMalloc(&sd->perm, S * sizeof(uint32_t))); CK(cudaMalloc(&sd->slot_key, S)); CK(cudaMalloc(&sd->slot_status, S)); sd->slot_cap = S;
     }
     if (ntk > sd->tile_cap) { cudaFree(sd->tile); sd->tile_cap = 0; CK(cudaMalloc(&sd->tile, ntk * sizeof(uint32_t))); sd->tile_cap = ntk; }
+    if (nroute > sd->route_cap) { cudaFree(sd->route); sd->route_cap = 0; CK(cudaMalloc(&sd->route, nroute * sizeof(uint32_t))); sd->route_cap = nroute; }
     return 0;
 }
-// One device pass of m records already in device memory (key_idx, 256-byte proofs, signal words with offsets relative to sig_base), enqueued
-// on stream st; statuses in caller order to d_status.  Caller holds c->mu and has set the device.  Launches: 3 grouping kernels, decode,
-// signals, vk_x, G2 check, Miller loop, final exponentiation, status scatter = 10 for a pass of one chain; from chunk_count's threshold on,
-// + 1 (flag merge of the forked front) and 4 chunks x (4 Miller segments + 4 final-exponentiation stages) instead of 2: 41.
-static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t* d_key_idx, const uint8_t* d_proofs, const uint8_t* d_sig,
-                       const uint64_t* d_sig_off, uint64_t sig_base, uint8_t* d_status, cudaStream_t st) {
+// One grouped device pass of m records in device memory, enqueued on stream st; statuses in caller order to d_status.  Caller holds c->mu and
+// has set the device.  Key sets and routers differ only in the front: keys() enqueues what the grouping kernels read as key indices and
+// returns it (a key set: the caller's array, no launch; a router: k_route's route words in sd->route, `nroute` = m of them), front(S) the
+// decode and signal kernels over the S slots.  Launches: [k_route], 3 grouping kernels, decode, signals, vk_x, G2 check, Miller loop, final
+// exponentiation, status scatter = 10 (a router: 11) for a pass of one chain; from chunk_count's threshold on, + 1 (flag merge of the forked
+// front) and 4 chunks x (4 Miller segments + 4 final-exponentiation stages) instead of 2: 41 (42).  ns: scalars per slot.
+template <class Keys, class Front>
+static int grouped_pass(SetDev* sd, int nk, int ns, size_t m, size_t nroute, uint8_t* d_status, cudaStream_t st, Keys keys, Front front) {
     DevCtx* c = sd->c;
-    const int nk = (int)s->keys.size(), ns = s->ns_max;
     const size_t S = slot_bound(m, (size_t)nk), ntiles = (m + ZKV_GROUP_TILE - 1) / ZKV_GROUP_TILE;
     int rc = ctx_acquire(c, st); if (rc) return rc;
     rc = ctx_reserve(c, S, (size_t)ns * 8); if (rc) return rc;
-    rc = set_reserve(sd, S, ntiles * nk); if (rc) return rc;
+    rc = set_reserve(sd, S, ntiles * nk, nroute); if (rc) return rc;
     CK(cudaMemsetAsync(sd->perm, 0xff, S * sizeof(uint32_t), st)); CK(cudaMemsetAsync(sd->slot_key, 0, S, st));
+    const uint32_t* d_key_idx = keys();
     launch(k_group_count, (int)ntiles, 256, 0, st, (int)m, nk, d_key_idx, sd->tile);
     launch(k_group_scan, 1, ZKV_MAX_KEYS, 0, st, (int)ntiles, nk, sd->tile, sd->slot_key, sd->total);
     launch(k_group_scatter, (int)ntiles, 256, 0, st, (int)m, nk, d_key_idx, sd->tile, sd->perm, sd->slot_key);
     const int n = (int)S;
     uint8_t* flags = c->flags;
-    launch(k_decode_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, nk, d_key_idx, d_proofs, c->px[0], c->py[0], c->qx, c->qy, c->px[3], c->py[3], flags);
-    launch(k_signals_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, d_sig, d_sig_off, sig_base, ns, c->scal, flags);
+    front(n);
     const int chunks = chunk_count(c, S, 0);
     rc = enqueue_vkx_g2(c, 0, n, flags, st, chunks > 1, false, [&](uint8_t* fl) {   // forked when chunked: the front phase of run_verify's schedule
         launch(k_vkx_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, c->scal, ns, c->px[2], c->py[2], fl);
@@ -727,6 +740,41 @@ static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t*
     CK(cudaGetLastError());
     return 0;
 }
+// A key set's pass: key_idx, 256-byte proofs, signal words with offsets relative to sig_base
+static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t* d_key_idx, const uint8_t* d_proofs, const uint8_t* d_sig,
+                       const uint64_t* d_sig_off, uint64_t sig_base, uint8_t* d_status, cudaStream_t st) {
+    DevCtx* c = sd->c;
+    const int nk = (int)s->keys.size(), ns = s->ns_max;
+    return grouped_pass(sd, nk, ns, m, 0, d_status, st, [&]() { return d_key_idx; }, [&](int n) {
+        launch(k_decode_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, nk, d_key_idx, d_proofs, c->px[0], c->py[0], c->qx, c->qy, c->px[3], c->py[3], c->flags);
+        launch(k_signals_keys, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, d_sig, d_sig_off, sig_base, ns, c->scal, c->flags);
+    });
+}
+// Host-buffer form of a grouped call: the records [b, e) of each device's contiguous range in passes of up to MAX_CHUNK.  A pass is grouped
+// as a whole, so it is uploaded as a whole before its kernels run: pack(s0, m, sink) returns the size of pass [s0, s0 + m)'s input block and,
+// given a sink, writes the block there (gathered in the pinned staging buffer, or with `direct` uploaded in place from the caller's
+// page-locked arrays); pass(sd, s0, m, d_block) enqueues its kernels on c->stream with the statuses to c->d_out.
+template <class SetOf, class Pack, class Pass>
+static int grouped_host(const std::vector<DevCtx*>& ctxs, SetOf set_of, size_t n, bool direct, uint8_t* status_out, Pack pack, Pass pass) {
+    return for_each_device(ctxs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
+        SetDev* sd = set_of(c->device);
+        if (int rc = ctx_wait_idle(c)) return rc;      // a host call blocks anyway: wait out an earlier asynchronous device call here
+        for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
+            const size_t m = std::min(MAX_CHUNK, e - s0), bytes = pack(s0, m, (Sink*)nullptr);
+            int rc = ctx_stage(c, bytes, m); if (rc) return rc;
+            Sink sk{direct ? nullptr : c->h_pin, c->d_in, c->stream, 0};
+            pack(s0, m, &sk);
+            if (sk.bad) return fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (page-locked caller memory to device)");
+            if (!direct) CK(cudaMemcpyAsync(c->d_in, c->h_pin, bytes, cudaMemcpyHostToDevice, c->stream));
+            rc = pass(sd, s0, m, c->d_in);
+            if (rc) return rc;
+            CK(cudaMemcpyAsync(c->h_out, c->d_out, m, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            memcpy(status_out + s0, c->h_out, m);
+        }
+        return 0;
+    });
+}
 extern "C" int zkv_groth16_verify_batch_keys(const zkv_vkset* s, const uint32_t* key_idx, const uint8_t* proofs, const uint8_t* signals,
                                              const uint64_t* sig_off, size_t n, uint8_t* status_out) {
     if (!s || (n && (!key_idx || !proofs || !sig_off || !status_out))) return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch_keys: null argument");
@@ -737,27 +785,23 @@ extern "C" int zkv_groth16_verify_batch_keys(const zkv_vkset* s, const uint32_t*
     const bool any_sig = sig_off[n] != sig_off[0];
     if (any_sig && !signals) return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch_keys: null signals");
     const bool direct = n >= 4096 && is_pinned(key_idx) && is_pinned(proofs) && is_pinned(sig_off) && (!any_sig || is_pinned(signals));   // page-locked caller arrays are uploaded in place
-    return for_each_device(s->ctxs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
-        SetDev* sd = set_dev(s, c->device);
-        if (int rc = ctx_wait_idle(c)) return rc;      // a host call blocks anyway: wait out an earlier asynchronous device call here
-        // A pass is grouped as a whole, so it is uploaded as a whole before its kernels run: [key_idx][signal offsets][proofs][signal words]
-        for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
-            const size_t m = std::min(MAX_CHUNK, e - s0), words = (size_t)(sig_off[s0 + m] - sig_off[s0]);
-            const size_t o_off = (m * 4 + 255) / 256 * 256, o_pr = o_off + ((m + 1) * 8 + 255) / 256 * 256, o_sig = o_pr + m * 256, bytes = o_sig + words * 32;
-            int rc = ctx_stage(c, bytes, m); if (rc) return rc;
-            Sink sk{direct ? nullptr : c->h_pin, c->d_in, c->stream, 0};
-            sk.put(0, key_idx + s0, m * 4, true); sk.put(o_off, sig_off + s0, (m + 1) * 8, true); sk.put(o_pr, proofs + s0 * 256, m * 256, true);
-            if (words) sk.put(o_sig, signals + sig_off[s0] * 32, words * 32, true);
-            if (sk.bad) return fail(ZKV_ERR_CUDA, "cudaMemcpyAsync (page-locked caller memory to device)");
-            if (!direct) CK(cudaMemcpyAsync(c->d_in, c->h_pin, bytes, cudaMemcpyHostToDevice, c->stream));
-            rc = keyset_pass(s, sd, m, (const uint32_t*)c->d_in, c->d_in + o_pr, c->d_in + o_sig, (const uint64_t*)(c->d_in + o_off), sig_off[s0], c->d_out, c->stream);
-            if (rc) return rc;
-            CK(cudaMemcpyAsync(c->h_out, c->d_out, m, cudaMemcpyDeviceToHost, c->stream));
-            CK(cudaStreamSynchronize(c->stream));
-            memcpy(status_out + s0, c->h_out, m);
-        }
-        return 0;
-    });
+    // pass block layout: [key_idx][signal offsets][proofs][signal words]
+    auto layout = [&](size_t s0, size_t m, size_t& o_off, size_t& o_pr, size_t& o_sig) {
+        o_off = (m * 4 + 255) / 256 * 256; o_pr = o_off + ((m + 1) * 8 + 255) / 256 * 256; o_sig = o_pr + m * 256;
+        return o_sig + (size_t)(sig_off[s0 + m] - sig_off[s0]) * 32;
+    };
+    return grouped_host(s->ctxs, [&](int d) { return set_dev(s, d); }, n, direct, status_out,
+        [&](size_t s0, size_t m, Sink* sk) -> size_t {
+            size_t o_off, o_pr, o_sig; const size_t bytes = layout(s0, m, o_off, o_pr, o_sig);
+            if (!sk) return bytes;
+            sk->put(0, key_idx + s0, m * 4, true); sk->put(o_off, sig_off + s0, (m + 1) * 8, true); sk->put(o_pr, proofs + s0 * 256, m * 256, true);
+            if (bytes > o_sig) sk->put(o_sig, signals + sig_off[s0] * 32, bytes - o_sig, true);
+            return bytes;
+        },
+        [&](SetDev* sd, size_t s0, size_t m, uint8_t* d) {
+            size_t o_off, o_pr, o_sig; layout(s0, m, o_off, o_pr, o_sig);
+            return keyset_pass(s, sd, m, (const uint32_t*)d, d + o_pr, d + o_sig, (const uint64_t*)(d + o_off), sig_off[s0], sd->c->d_out, sd->c->stream);
+        });
 }
 extern "C" int zkv_groth16_verify_batch_keys_device(const zkv_vkset* s, int device, const void* d_key_idx, const void* d_proofs, const void* d_signals,
                                                     const void* d_sig_off, size_t n, void* d_status_out, void* stream) {
@@ -772,7 +816,10 @@ extern "C" int zkv_groth16_verify_batch_keys_device(const zkv_vkset* s, int devi
 }
 
 // ------------------------------------------------------------------------------------------ RISC Zero
+// first member of both verifier handles: a router refuses a handle of the other kind
+enum HandleKind : uint32_t { HANDLE_RISC0 = 0x7a6b7652u, HANDLE_SP1 = 0x7a6b7653u };
 struct zkv_risc0 {
+    HandleKind kind = HANDLE_RISC0;
     const zkv_vk* vk = nullptr; zkv_vk* owned = nullptr;
     int initialized = 0;
     uint8_t control_root_0[16], control_root_1[16], bn254_control_id[32], selector[4], vk_digest[32];
@@ -925,18 +972,23 @@ extern "C" int zkv_risc0_verify_batch_device(const zkv_risc0* h, int device, con
 }
 
 // ------------------------------------------------------------------------------------------ SP1
-struct zkv_sp1 { const zkv_vk* vk = nullptr; zkv_vk* owned = nullptr; uint8_t verifier_hash[32]; };
-extern "C" int zkv_sp1_create(const zkv_vk* vk_or_null, const int* devices, int n_dev, zkv_sp1** out) {
-    if (!out) return fail(ZKV_ERR_ARG, "zkv_sp1_create: null out");
+struct zkv_sp1 { HandleKind kind = HANDLE_SP1; const zkv_vk* vk = nullptr; zkv_vk* owned = nullptr; uint8_t verifier_hash[32]; std::string version; };
+extern "C" int zkv_sp1_create_version(const zkv_vk* vk_or_null, const uint8_t verifier_hash[32], const char* version, const int* devices, int n_dev, zkv_sp1** out) {
+    if (!out || !verifier_hash || !version) return fail(ZKV_ERR_ARG, "zkv_sp1_create_version: null argument");
+    if (vk_or_null && (vk_or_null->n_ic != 3 || vk_or_null->vm != ZKV_VM_SP1)) return fail(ZKV_ERR_ARG, "zkv_sp1_create: need a ZKV_VM_SP1 key with 3 IC points");
     zkv_sp1* h = new zkv_sp1();
-    memcpy(h->verifier_hash, ZKV_SP1_VERIFIER_HASH, 32);
-    if (vk_or_null) { if (vk_or_null->n_ic != 3 || vk_or_null->vm != ZKV_VM_SP1) { delete h; return fail(ZKV_ERR_ARG, "zkv_sp1_create: need a ZKV_VM_SP1 key with 3 IC points"); } h->vk = vk_or_null; }
+    memcpy(h->verifier_hash, verifier_hash, 32); h->version = version;
+    if (vk_or_null) h->vk = vk_or_null;
     else { int rc = zkv_vk_load_sp1(devices, n_dev, &h->owned); if (rc) { delete h; return rc; } h->vk = h->owned; }
     *out = h; return 0;
 }
+extern "C" int zkv_sp1_create(const zkv_vk* vk_or_null, const int* devices, int n_dev, zkv_sp1** out) {
+    if (!out) return fail(ZKV_ERR_ARG, "zkv_sp1_create: null out");
+    return zkv_sp1_create_version(vk_or_null, ZKV_SP1_VERIFIER_HASH, ZKV_SP1_VERSION, devices, n_dev, out);
+}
 extern "C" void zkv_sp1_destroy(zkv_sp1* h) { if (!h) return; if (h->owned) zkv_vk_free(h->owned); delete h; }
 extern "C" int zkv_sp1_verifier_hash(const zkv_sp1* h, uint8_t out[32]) { if (!h || !out) return fail(ZKV_ERR_ARG, "null"); memcpy(out, h->verifier_hash, 32); return 0; }
-extern "C" const char* zkv_sp1_version(const zkv_sp1*) { return ZKV_SP1_VERSION; }
+extern "C" const char* zkv_sp1_version(const zkv_sp1* h) { return h ? h->version.c_str() : ZKV_SP1_VERSION; }
 
 extern "C" int zkv_sp1_verify_batch(const zkv_sp1* h, const uint8_t* vkeys, const uint8_t* public_values, const uint64_t* pv_off, const uint8_t* proofs, const uint64_t* proof_off, size_t n, uint8_t* status_out) {
     if (!h || (n && (!vkeys || !public_values || !pv_off || !proofs || !proof_off || !status_out))) return fail(ZKV_ERR_ARG, "zkv_sp1_verify_batch: null argument");
@@ -985,6 +1037,200 @@ extern "C" int zkv_sp1_verify_batch_device(const zkv_sp1* h, int device, const v
     return device_call(c, device, stream, [&](cudaStream_t s) { return run_verify(c, j, s); });
 }
 
+// ------------------------------------------------------------------------------------------ routers: RiscZeroVerifierRouter / SP1VerifierGateway
+// A router borrows 1..256 verifier handles of one kind and routes each record to the handle whose selector its first 4 bytes are.  It is a
+// key set (one KeyDesc per route, the grouped pass) whose key indices the routing kernel k_route computes on the device.  Per route it takes
+// a snapshot at creation: the selector, and the vk_x part of its KeyDesc (a RISC Zero handle's folded base K = IC0 + s0 IC1 + s1 IC2 + s4 IC5
+// with the IC3 / IC4 tables over the 128-bit claim halves, an SP1 handle's IC0 and tables).  Routes are kept in ascending selector order, so
+// route r is the r-th entry of the selector table k_route searches.
+struct Router {
+    std::vector<SetDev> devs;
+    std::vector<DevCtx*> ctxs;            // devs[d].c (for_each_device)
+    int nr = 0;
+};
+struct zkv_risc0_router : Router { Risc0HashConsts hc; };
+struct zkv_sp1_gateway : Router {};
+static SetDev* router_dev(const Router* r, int device) {
+    for (auto& d : r->devs) if (d.c->device == device) return const_cast<SetDev*>(&d);
+    return nullptr;
+}
+struct RouteSpec { const zkv_vk* vk; uint32_t sel; int risc0; g1aff base; int all_fail; };
+// routes sorted by selector -> r's per-device key descriptors and selector tables; r is destroyed by the caller on error
+static int router_build(const char* fn, std::vector<RouteSpec>& rs, const int* devices, int n_dev, Router* r) {
+    std::sort(rs.begin(), rs.end(), [](const RouteSpec& a, const RouteSpec& b) { return a.sel < b.sel; });
+    for (size_t k = 1; k < rs.size(); k++) if (rs[k].sel == rs[k - 1].sel) return fail(ZKV_ERR_ARG, std::string(fn) + ": SelectorInUse: two handles have the same selector");
+    int ndev_sys = zkv_device_count();
+    if (ndev_sys <= 0) return fail(ZKV_ERR_CUDA, std::string(fn) + ": no CUDA device (this library has no CPU path)");
+    std::vector<int> devs;
+    if (!devices || n_dev <= 0) devs.push_back(0); else devs.assign(devices, devices + n_dev);
+    for (int d : devs) if (d < 0 || d >= ndev_sys) return fail(ZKV_ERR_ARG, std::string(fn) + ": bad device index");
+    for (size_t k = 0; k < rs.size(); k++)
+        for (int d : devs) if (!vk_ctx(rs[k].vk, d)) return fail(ZKV_ERR_ARG, std::string(fn) + ": the key of a route is not loaded on device " + std::to_string(d));
+    r->nr = (int)rs.size();
+    std::vector<uint32_t> sel;
+    for (auto& q : rs) sel.push_back(q.sel);
+    r->devs.resize(devs.size());
+    for (size_t j = 0; j < devs.size(); j++) {
+        SetDev& sd = r->devs[j];
+        sd.c = new DevCtx(); sd.c->device = devs[j]; r->ctxs.push_back(sd.c);
+        std::vector<KeyDesc> h;
+        for (auto& q : rs) {
+            const DevCtx* kc = vk_ctx(q.vk, devs[j]);
+            KeyDesc kd = key_desc(q.vk, kc);
+            kd.ns = 2;
+            if (q.risc0) { kd.base = q.base; kd.tab = kc->d_tab + (size_t)2 * ZKV_WIN_PER_SCALAR * ZKV_WIN_ENTRIES; kd.nwin = 32; }
+            kd.reject = !q.vk->valid || q.all_fail;
+            h.push_back(kd);
+        }
+        int rc = setdev_build(sd, h); if (rc) return rc;
+        CK(cudaMalloc(&sd.d_sel, sizeof(uint32_t) * sel.size()));
+        CK(cudaMemcpy(sd.d_sel, sel.data(), sizeof(uint32_t) * sel.size(), cudaMemcpyHostToDevice));
+    }
+    return 0;
+}
+// one router pass of m records (variable records with rec_off, else `stride` apart); signals(n) enqueues the signal kernel over the n slots
+template <class Signals>
+static int router_pass(const Router* r, SetDev* sd, size_t m, const uint8_t* recs, size_t stride, const uint64_t* rec_off, uint64_t rec_base,
+                       uint8_t* d_status, cudaStream_t st, Signals signals) {
+    DevCtx* c = sd->c;
+    return grouped_pass(sd, r->nr, 2, m, m, d_status, st,
+        [&]() { launch(k_route, nblk(m, 256), 256, 0, st, (int)m, recs, stride, rec_off, rec_base, (const uint32_t*)sd->d_sel, r->nr, sd->route); return (const uint32_t*)sd->route; },
+        [&](int n) {
+            launch(k_decode_route, nblk(n), TPB, 0, st, n, sd->perm, sd->slot_key, sd->d_keys, sd->route, recs, stride, rec_off, rec_base, c->px[0], c->py[0], c->qx, c->qy, c->px[3], c->py[3], c->flags);
+            signals(n);
+        });
+}
+static int risc0_router_pass(const zkv_risc0_router* r, SetDev* sd, size_t m, const uint8_t* recs, size_t stride, const uint64_t* rec_off, uint64_t rec_base,
+                             const uint8_t* a32, const uint8_t* b32, int integrity, uint8_t* d_status, cudaStream_t st) {
+    DevCtx* c = sd->c;
+    return router_pass(r, sd, m, recs, stride, rec_off, rec_base, d_status, st, [&](int n) {
+        launch(k_risc0_signals_route, nblk(n), TPB, 0, st, n, sd->perm, integrity ? nullptr : a32, integrity ? nullptr : b32, integrity ? a32 : nullptr, integrity, r->hc, c->scal);
+    });
+}
+static int sp1_gateway_pass(const zkv_sp1_gateway* g, SetDev* sd, size_t m, const uint8_t* recs, size_t stride, const uint64_t* rec_off, uint64_t rec_base,
+                            const uint8_t* vkeys, const uint8_t* pv, const uint64_t* pv_off, uint64_t pv_base, size_t pv_stride, uint8_t* d_status, cudaStream_t st) {
+    DevCtx* c = sd->c;
+    return router_pass(g, sd, m, recs, stride, rec_off, rec_base, d_status, st, [&](int n) {
+        launch(k_sp1_signals_route, nblk(n), TPB, 0, st, n, sd->perm, vkeys, pv, pv_off, pv_base, pv_stride, c->scal, c->flags);
+    });
+}
+
+extern "C" int zkv_risc0_router_create(const zkv_risc0* const* verifiers, int n, const int* devices, int n_dev, zkv_risc0_router** out) {
+    if (!out || !verifiers) return fail(ZKV_ERR_ARG, "zkv_risc0_router_create: null argument");
+    if (n < 1 || n > ZKV_MAX_KEYS) return fail(ZKV_ERR_ARG, "zkv_risc0_router_create: n must be 1..256");
+    for (int k = 0; k < n; k++) {
+        if (!verifiers[k]) return fail(ZKV_ERR_ARG, "zkv_risc0_router_create: null handle");
+        if (verifiers[k]->kind != HANDLE_RISC0) return fail(ZKV_ERR_ARG, "zkv_risc0_router_create: handle " + std::to_string(k) + " is not a RISC Zero verifier");
+    }
+    for (int k = 0; k < n; k++) if (!verifiers[k]->initialized) return fail(ZKV_ERR_STATE, "zkv_risc0_router_create: handle " + std::to_string(k) + " is not initialised (it has no selector)");
+    std::vector<RouteSpec> rs;
+    for (int k = 0; k < n; k++) { const zkv_risc0* h = verifiers[k]; rs.push_back({h->vk, sel_le(h->selector), 1, h->base, h->all_fail}); }
+    zkv_risc0_router* r = new zkv_risc0_router();
+    r->hc = verifiers[0]->hc;             // the same for every handle: tags of risc0/types.rs and the zero system-state digest
+    int rc = router_build("zkv_risc0_router_create", rs, devices, n_dev, r);
+    if (rc) { zkv_risc0_router_destroy(r); return rc; }
+    *out = r;
+    return 0;
+}
+extern "C" void zkv_risc0_router_destroy(zkv_risc0_router* r) { if (!r) return; setdev_free(r->devs); delete r; }
+static int risc0_router_batch(const zkv_risc0_router* r, const uint8_t* seals, const uint64_t* seal_off, const uint8_t* a32, const uint8_t* b32, int integrity, size_t n, uint8_t* status_out) {
+    if (!r || (n && (!seals || !seal_off || !a32 || (!integrity && !b32) || !status_out))) return fail(ZKV_ERR_ARG, "zkv_risc0_router_verify_batch: null argument");
+    if (n == 0) return 0;
+    if (n > 0xffffffffull) return fail(ZKV_ERR_ARG, "batch too large");
+    if (!offsets_ok(seal_off, n)) return fail(ZKV_ERR_ARG, "seal offsets must be non-decreasing");
+    const bool direct = n >= 4096 && is_pinned(seals) && is_pinned(seal_off) && is_pinned(a32) && (integrity || is_pinned(b32));      // page-locked caller arrays are uploaded in place
+    const size_t per = integrity ? 32 : 64;
+    // pass block layout: [offsets (m + 1) x 8][a32 m x 32][b32 m x 32][seal bytes][slack]
+    return grouped_host(r->ctxs, [&](int d) { return router_dev(r, d); }, n, direct, status_out,
+        [&](size_t s0, size_t m, Sink* sk) -> size_t {
+            const size_t bytes = (size_t)(seal_off[s0 + m] - seal_off[s0]);
+            if (!sk) return (m + 1) * 8 + m * per + bytes + 320;
+            size_t p = 0;
+            sk->put(p, seal_off + s0, (m + 1) * 8, true); p += (m + 1) * 8;
+            sk->put(p, a32 + s0 * 32, m * 32, true); p += m * 32;
+            if (!integrity) { sk->put(p, b32 + s0 * 32, m * 32, true); p += m * 32; }
+            sk->put(p, seals + seal_off[s0], bytes, true);
+            return p + bytes + 320;
+        },
+        [&](SetDev* sd, size_t s0, size_t m, uint8_t* d) {
+            const uint8_t* a = d + (m + 1) * 8;
+            return risc0_router_pass(r, sd, m, a + m * per, 0, (const uint64_t*)d, seal_off[s0], a, a + m * 32, integrity, sd->c->d_out, sd->c->stream);
+        });
+}
+extern "C" int zkv_risc0_router_verify_batch(const zkv_risc0_router* r, const uint8_t* seals, const uint64_t* seal_off, const uint8_t* image_ids,
+                                             const uint8_t* journal_digests, size_t n, uint8_t* status_out) {
+    return risc0_router_batch(r, seals, seal_off, image_ids, journal_digests, 0, n, status_out);
+}
+extern "C" int zkv_risc0_router_verify_integrity_batch(const zkv_risc0_router* r, const uint8_t* seals, const uint64_t* seal_off, const uint8_t* claim_digests,
+                                                       size_t n, uint8_t* status_out) {
+    return risc0_router_batch(r, seals, seal_off, claim_digests, nullptr, 1, n, status_out);
+}
+extern "C" int zkv_risc0_router_verify_batch_device(const zkv_risc0_router* r, int device, const void* d_seals260, const void* d_image_ids, const void* d_journal_digests,
+                                                    size_t n, void* d_status_out, void* stream) {
+    if (!r || !d_seals260 || !d_image_ids || !d_journal_digests || !d_status_out) return fail(ZKV_ERR_ARG, "zkv_risc0_router_verify_batch_device: null argument");
+    SetDev* sd = router_dev(r, device);
+    if (!sd) return fail(ZKV_ERR_ARG, "device not in the router's device list");
+    if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, "device batch too large");
+    if (n == 0) return 0;
+    return device_call(sd->c, device, stream, [&](cudaStream_t st) {
+        return risc0_router_pass(r, sd, n, (const uint8_t*)d_seals260, 260, nullptr, 0, (const uint8_t*)d_image_ids, (const uint8_t*)d_journal_digests, 0, (uint8_t*)d_status_out, st);
+    });
+}
+
+extern "C" int zkv_sp1_gateway_create(const zkv_sp1* const* verifiers, int n, const int* devices, int n_dev, zkv_sp1_gateway** out) {
+    if (!out || !verifiers) return fail(ZKV_ERR_ARG, "zkv_sp1_gateway_create: null argument");
+    if (n < 1 || n > ZKV_MAX_KEYS) return fail(ZKV_ERR_ARG, "zkv_sp1_gateway_create: n must be 1..256");
+    for (int k = 0; k < n; k++) {
+        if (!verifiers[k]) return fail(ZKV_ERR_ARG, "zkv_sp1_gateway_create: null handle");
+        if (verifiers[k]->kind != HANDLE_SP1) return fail(ZKV_ERR_ARG, "zkv_sp1_gateway_create: handle " + std::to_string(k) + " is not an SP1 verifier");
+    }
+    std::vector<RouteSpec> rs;
+    for (int k = 0; k < n; k++) rs.push_back({verifiers[k]->vk, sel_le(verifiers[k]->verifier_hash), 0, g1aff{}, 0});
+    zkv_sp1_gateway* g = new zkv_sp1_gateway();
+    int rc = router_build("zkv_sp1_gateway_create", rs, devices, n_dev, g);
+    if (rc) { zkv_sp1_gateway_destroy(g); return rc; }
+    *out = g;
+    return 0;
+}
+extern "C" void zkv_sp1_gateway_destroy(zkv_sp1_gateway* g) { if (!g) return; setdev_free(g->devs); delete g; }
+extern "C" int zkv_sp1_gateway_verify_batch(const zkv_sp1_gateway* g, const uint8_t* vkeys, const uint8_t* public_values, const uint64_t* pv_off,
+                                            const uint8_t* proofs, const uint64_t* proof_off, size_t n, uint8_t* status_out) {
+    if (!g || (n && (!vkeys || !public_values || !pv_off || !proofs || !proof_off || !status_out))) return fail(ZKV_ERR_ARG, "zkv_sp1_gateway_verify_batch: null argument");
+    if (n == 0) return 0;
+    if (n > 0xffffffffull) return fail(ZKV_ERR_ARG, "batch too large");
+    if (!offsets_ok(proof_off, n) || !offsets_ok(pv_off, n)) return fail(ZKV_ERR_ARG, "proof / public-value offsets must be non-decreasing");
+    const bool direct = n >= 4096 && is_pinned(proofs) && is_pinned(proof_off) && is_pinned(pv_off) && is_pinned(vkeys) && is_pinned(public_values);      // page-locked caller arrays are uploaded in place
+    // pass block layout: [proof offsets (m + 1) x 8][public-value offsets (m + 1) x 8][vkeys m x 32][proof bytes][public values][slack]
+    return grouped_host(g->ctxs, [&](int d) { return router_dev(g, d); }, n, direct, status_out,
+        [&](size_t s0, size_t m, Sink* sk) -> size_t {
+            const size_t pr = (size_t)(proof_off[s0 + m] - proof_off[s0]), pv = (size_t)(pv_off[s0 + m] - pv_off[s0]);
+            if (!sk) return (m + 1) * 16 + m * 32 + pr + pv + 320;
+            size_t p = 0;
+            sk->put(p, proof_off + s0, (m + 1) * 8, true); p += (m + 1) * 8;
+            sk->put(p, pv_off + s0, (m + 1) * 8, true); p += (m + 1) * 8;
+            sk->put(p, vkeys + s0 * 32, m * 32, true); p += m * 32;
+            sk->put(p, proofs + proof_off[s0], pr, true); p += pr;
+            sk->put(p, public_values + pv_off[s0], pv, true); p += pv;
+            return p + 320;
+        },
+        [&](SetDev* sd, size_t s0, size_t m, uint8_t* d) {
+            const uint8_t* vk = d + (m + 1) * 16; const uint8_t* recs = vk + m * 32;
+            return sp1_gateway_pass(g, sd, m, recs, 0, (const uint64_t*)d, proof_off[s0], vk, recs + (size_t)(proof_off[s0 + m] - proof_off[s0]),
+                                    (const uint64_t*)(d + (m + 1) * 8), pv_off[s0], 0, sd->c->d_out, sd->c->stream);
+        });
+}
+extern "C" int zkv_sp1_gateway_verify_batch_device(const zkv_sp1_gateway* g, int device, const void* d_vkeys, const void* d_public_values, size_t pv_stride,
+                                                   const void* d_proofs260, size_t n, void* d_status_out, void* stream) {
+    if (!g || !d_vkeys || !d_public_values || !d_proofs260 || !d_status_out) return fail(ZKV_ERR_ARG, "zkv_sp1_gateway_verify_batch_device: null argument");
+    SetDev* sd = router_dev(g, device);
+    if (!sd) return fail(ZKV_ERR_ARG, "device not in the gateway's device list");
+    if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, "device batch too large");
+    if (n == 0) return 0;
+    return device_call(sd->c, device, stream, [&](cudaStream_t st) {
+        return sp1_gateway_pass(g, sd, n, (const uint8_t*)d_proofs260, 260, nullptr, 0, (const uint8_t*)d_vkeys, (const uint8_t*)d_public_values, nullptr, 0, pv_stride,
+                                (uint8_t*)d_status_out, st);
+    });
+}
 
 extern "C" void zkv_test_parallel_copy(void* dst, const void* src, size_t n) { pcopy(dst, src, n); }
 extern "C" void* zkv_host_alloc(size_t bytes) {

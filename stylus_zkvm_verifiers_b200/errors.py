@@ -87,3 +87,19 @@ class WrongVerifierSelector(VerifierError):
     def __init__(self, received, expected):
         super().__init__(bytes(received), bytes(expected))
         self.received, self.expected = bytes(received), bytes(expected)
+
+
+class SelectorUnknown(VerifierError):
+    signature = "SelectorUnknown(bytes4)"               # RiscZeroVerifierRouter: no verifier registered under the seal's selector
+
+    def __init__(self, selector):
+        super().__init__(bytes(selector))
+        self.selector = bytes(selector)
+
+
+class RouteNotFound(VerifierError):
+    signature = "RouteNotFound(bytes4)"                 # SP1VerifierGateway: no route for the proof's selector
+
+    def __init__(self, selector):
+        super().__init__(bytes(selector))
+        self.selector = bytes(selector)

@@ -3,6 +3,7 @@
   RiscZeroVerifier  <- IRiscZeroVerifier, /root/reference/contracts/src/risc0/verifier.rs:18-42
   Sp1Verifier       <- ISp1Verifier,      /root/reference/contracts/src/sp1/verifier.rs:16-29
   Groth16Verifier   <- Groth16Verifier::verify_proof_with_key, contracts/src/common/groth16.rs:23-49
+  RiscZeroVerifierRouter, Sp1VerifierGateway <- the routers that forward a seal / proof to the verifier version its first 4 bytes select
   VerificationKey   <- contracts/src/common/types.rs:17-23
 
 Same method names, argument meaning and error behaviour: the single-proof calls return on success and
@@ -283,13 +284,20 @@ class RiscZeroVerifier:
 
 
 class Sp1Verifier:
-    """sp1/verifier.rs:31-54 (ISp1Verifier)."""
+    """sp1/verifier.rs:31-54 (ISp1Verifier).  verifier_hash / version: another verifier version's 32-byte hash (its first 4 bytes are
+    the selector) and version string, with that version's key as `vk` (None: the embedded v5 key); by default the embedded v5 ones."""
 
-    def __init__(self, vk=None, devices=None):
+    def __init__(self, vk=None, devices=None, verifier_hash=None, version=None):
         self._vk = vk
         self._h = C.c_void_p()
         arr, nd = _dev_array(devices)
-        N.check(N.lib().zkv_sp1_create(vk._h if vk is not None else None, arr, nd, C.byref(self._h)))
+        if verifier_hash is None:
+            if version is not None:
+                raise ValueError("version needs the verifier_hash of that version")
+            N.check(N.lib().zkv_sp1_create(vk._h if vk is not None else None, arr, nd, C.byref(self._h)))
+        else:
+            _need32(verifier_hash=verifier_hash)
+            N.check(N.lib().zkv_sp1_create_version(vk._h if vk is not None else None, bytes(verifier_hash), (version or "").encode(), arr, nd, C.byref(self._h)))
 
     def close(self):
         if getattr(self, "_h", None):
@@ -345,6 +353,136 @@ class Sp1Verifier:
         out = (C.c_float * 5)()
         n = N.lib().zkv_last_stage_ms(N.lib().zkv_sp1_vk(self._h), device, out, 5)
         return dict(zip(("decode_hash", "vk_x", "g2_check", "miller", "final_exp"), list(out)[:max(n, 0)]))
+
+
+def _route_error(status):
+    """the error a route handle raises for a status other than OK / SELECTOR_MISMATCH"""
+    if status == N.ZKV_INVALID_PROOF_DATA:
+        return E.InvalidProofData()
+    return E.VerificationFailed()
+
+
+def _handles(verifiers):
+    return (C.c_void_p * max(len(verifiers), 1))(*[v._h for v in verifiers])
+
+
+class RiscZeroVerifierRouter:
+    """RiscZeroVerifierRouter: 1..256 initialised RiscZeroVerifier handles (zkv_risc0_router_create), each registered under its selector.
+    A seal goes to the verifier whose selector is bytes4(seal[0:4]); a selector no verifier has raises SelectorUnknown.  The router keeps
+    references to its verifiers, which must outlive it."""
+
+    def __init__(self, verifiers, devices=None):
+        self.verifiers = list(verifiers)
+        self._h = C.c_void_p()
+        arr, nd = _dev_array(devices)
+        N.check(N.lib().zkv_risc0_router_create(_handles(self.verifiers), len(self.verifiers), arr, nd, C.byref(self._h)))
+        self._by_selector = {v.get_selector(): v for v in self.verifiers}
+
+    def __len__(self):
+        return len(self.verifiers)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            N.lib().zkv_risc0_router_destroy(self._h); self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def get_verifier(self, selector):
+        v = self._by_selector.get(bytes(selector))
+        if v is None:
+            raise E.SelectorUnknown(selector)
+        return v
+
+    def _result(self, status, seal):
+        if status == N.ZKV_OK:
+            return True
+        if status == N.ZKV_SELECTOR_MISMATCH:
+            raise E.SelectorUnknown(seal[:4])
+        raise _route_error(status)
+
+    def verify(self, seal, image_id, journal_digest):
+        return self._result(int(self.verify_batch([seal], [image_id], [journal_digest])[0]), seal)
+
+    def verify_integrity(self, receipt_seal, claim_digest):
+        return self._result(int(self.verify_integrity_batch([receipt_seal], [claim_digest])[0]), receipt_seal)
+
+    def verify_batch(self, seals, image_ids, journal_digests):
+        n = len(seals)
+        _need32_each(n, image_ids=image_ids, journal_digests=journal_digests)
+        return self.verify_batch_packed(b"".join(seals) or b"\0", _offsets(seals), b"".join(image_ids) or b"\0", b"".join(journal_digests) or b"\0", n)
+
+    def verify_integrity_batch(self, seals, claim_digests):
+        n = len(seals)
+        _need32_each(n, claim_digests=claim_digests)
+        st = np.zeros(n, dtype=np.uint8)
+        off = _offsets(seals)
+        N.check(N.lib().zkv_risc0_router_verify_integrity_batch(self._h, N.buf(b"".join(seals) or b"\0"), off.ctypes.data, N.buf(b"".join(claim_digests) or b"\0"), n, st.ctypes.data))
+        return st
+
+    def verify_batch_packed(self, seal_blob, seal_off, image_ids, journal_digests, n, status_out=None):
+        """Zero-copy form: contiguous buffers (bytes or numpy uint8) + numpy uint64 offsets."""
+        st = status_out if status_out is not None else np.zeros(n, dtype=np.uint8)
+        N.check(N.lib().zkv_risc0_router_verify_batch(self._h, N.buf(seal_blob), seal_off.ctypes.data, N.buf(image_ids), N.buf(journal_digests), n, st.ctypes.data))
+        return st
+
+    def verify_batch_device(self, device, d_seals260, d_image_ids, d_journal_digests, n, d_status, stream=None):
+        """Inputs already in HBM (raw device pointers as ints, n x 260-byte seals); asynchronous on `stream`."""
+        N.check(N.lib().zkv_risc0_router_verify_batch_device(self._h, device, d_seals260, d_image_ids, d_journal_digests, n, d_status, stream))
+
+
+class Sp1VerifierGateway:
+    """SP1VerifierGateway: 1..256 Sp1Verifier handles of different verifier versions (zkv_sp1_gateway_create).  A proof goes to the verifier
+    whose verifier hash starts with proof[:4]; a selector no verifier has raises RouteNotFound.  The gateway keeps references to its
+    verifiers, which must outlive it."""
+
+    def __init__(self, verifiers, devices=None):
+        self.verifiers = list(verifiers)
+        self._h = C.c_void_p()
+        arr, nd = _dev_array(devices)
+        N.check(N.lib().zkv_sp1_gateway_create(_handles(self.verifiers), len(self.verifiers), arr, nd, C.byref(self._h)))
+
+    def __len__(self):
+        return len(self.verifiers)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            N.lib().zkv_sp1_gateway_destroy(self._h); self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def verify_proof(self, program_vkey, public_values, proof_bytes):
+        _need32(program_vkey=program_vkey)
+        st = int(self.verify_batch([program_vkey], [public_values], [proof_bytes])[0])
+        if st == N.ZKV_OK:
+            return None
+        if st == N.ZKV_SELECTOR_MISMATCH:
+            raise E.RouteNotFound(proof_bytes[:4])
+        raise _route_error(st)
+
+    def verify_batch(self, program_vkeys, public_values, proofs):
+        n = len(proofs)
+        _need32_each(n, program_vkeys=program_vkeys)
+        if len(public_values) != n:
+            raise ValueError("public_values: expected %d entries, got %d" % (n, len(public_values)))
+        return self.verify_batch_packed(b"".join(program_vkeys) or b"\0", b"".join(public_values) or b"\0", _offsets(public_values),
+                                        b"".join(proofs) or b"\0", _offsets(proofs), n)
+
+    def verify_batch_packed(self, vkeys, pv_blob, pv_off, proof_blob, proof_off, n, status_out=None):
+        st = status_out if status_out is not None else np.zeros(n, dtype=np.uint8)
+        N.check(N.lib().zkv_sp1_gateway_verify_batch(self._h, N.buf(vkeys), N.buf(pv_blob), pv_off.ctypes.data, N.buf(proof_blob), proof_off.ctypes.data, n, st.ctypes.data))
+        return st
+
+    def verify_batch_device(self, device, d_vkeys, d_public_values, pv_stride, d_proofs260, n, d_status, stream=None):
+        """Inputs already in HBM (raw device pointers as ints, n x 260-byte proofs, n x pv_stride public values); asynchronous on `stream`."""
+        N.check(N.lib().zkv_sp1_gateway_verify_batch_device(self._h, device, d_vkeys, d_public_values, pv_stride, d_proofs260, n, d_status, stream))
 
 
 # ------------------------------------------------------------------ precompile-shaped services and hooks
