@@ -196,7 +196,8 @@ int zkv_pairing4_batch_device(const zkv_vk* vk, int device, const void* d_g1s, c
  * with EVERY G2 point variable.  in: n x k x 192 B, each pair G1 (64 B) || G2 (128 B, wire order).  out: n x 32 B, the precompile's return
  * word (0..01 / 0..00).  reverted[i] = 1 where the call would fail (coordinate >= p, point off its curve, G2 point outside the order-r
  * subgroup); a pair with a member at infinity contributes 1; k = 0 is the empty product (true).  miller_out (optional, n x 384 B): the
- * Miller-loop value in the oracle's convention.  zkv_ec_pairing is one call on raw bytes (len % 192 != 0 -> reverted). */
+ * Miller-loop value in the oracle's convention.  zkv_ec_pairing is one call on raw bytes (len % 192 != 0 -> reverted).
+ * At most 64 pairs per instance: k > 64 (zkv_ec_pairing: len > 64 x 192) returns ZKV_ERR_ARG. */
 int zkv_ec_pairing_batch(const uint8_t* in, int k, size_t n, uint8_t* out, uint8_t* reverted, uint8_t* miller_out, int device);
 int zkv_ec_pairing(const uint8_t* in, size_t len, uint8_t out[32], uint8_t* reverted, int device);
 

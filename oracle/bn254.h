@@ -406,9 +406,10 @@ static void g2_frob_affine(fp2 *x, fp2 *y, int k) {  /* pi^k on the twist, k=1,2
 }
 typedef struct { g1a p; g2a q; } pair_t;
 /* multi-Miller: prod over pairs; pairs with an infinity member are skipped */
+#define ORACLE_MAX_PAIRS 64     /* the library's ecPairing limit (include/zkv.h); the precompile itself has none */
 static void miller_multi(fp12 *out, const pair_t *pairs, int n) {
     fp12 f = F12_ONE;
-    g2j R[16]; int act[16]; int na = 0;
+    g2j R[ORACLE_MAX_PAIRS]; int act[ORACLE_MAX_PAIRS]; int na = 0;
     for (int i = 0; i < n; i++) { act[i] = !(pairs[i].p.inf || pairs[i].q.inf); if (act[i]) { R[i].x = pairs[i].q.x; R[i].y = pairs[i].q.y; R[i].z = F2_ONE; na++; } }
     if (!na) { *out = f; return; }
     fp2 l0, l3, l4, a, b;

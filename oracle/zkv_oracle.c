@@ -102,8 +102,8 @@ int zkvo_ec_mul(const uint8_t *in, size_t len, uint8_t out[64]) {
 static int ec_pairing_ex(const uint8_t *in, size_t len, uint8_t out[32], uint8_t *miller_out, uint8_t *gt_out) {
     bn254_init();
     if (len % 192) return -1;
-    int n = (int)(len / 192); if (n > 16) return -2;
-    pair_t pr[16];
+    int n = (int)(len / 192); if (n > ORACLE_MAX_PAIRS) return -2;
+    pair_t pr[ORACLE_MAX_PAIRS];
     for (int i = 0; i < n; i++) if (dec_g1(&pr[i].p, in + 192 * i) || dec_g2(&pr[i].q, in + 192 * i + 64)) return -1;
     fp12 m, gt; miller_multi(&m, pr, n); final_exp(&gt, &m);
     memset(out, 0, 32); out[31] = f12_eq(&gt, &F12_ONE) ? 1 : 0;

@@ -14,7 +14,7 @@ G1 = w32(1) + w32(2)
 
 
 def test_sha256_matches_hashlib():
-    for n in (0, 1, 55, 56, 63, 64, 65, 98, 119, 120, 170, 194, 1000):
+    for n in (0, 1, 55, 56, 63, 64, 65, 98, 119, 120, 128, 170, 183, 184, 194, 447, 448, 1000, 4096, 65536, 1 << 20):
         m = bytes((i * 7 + n) & 0xFF for i in range(n))
         assert O.sha256(m) == hashlib.sha256(m).digest()
 
