@@ -90,6 +90,39 @@ int zkv_groth16_verify_batch_keys(const zkv_vkset* s, const uint32_t* key_idx, c
 int zkv_groth16_verify_batch_keys_device(const zkv_vkset* s, int device, const void* d_key_idx, const void* d_proofs,
                                          const void* d_signals, const void* d_sig_off, size_t n, void* d_status_out, void* stream);
 
+/* ---- keys passed as bytes in the call: N verify_proof_with_key(vm, &vk, a, b, c, &signals) calls (common/groth16.rs:23-49) -------------
+ * A handle owns a workspace and streams per device (devices == NULL -> device 0) and no keys; there is nothing to load.  Key j is
+ * keys[key_off[j] .. key_off[j+1]): alpha (64 B), beta, gamma, delta (128 B each, wire order), IC_0 .. IC_{n_ic-1} (64 B each), the EVM words of
+ * common/types.rs:17-23, so 448 + 64 n_ic bytes with n_ic in 2..16; key_vm[j] is ZKV_VM_RISC0 or ZKV_VM_SP1.  Proofs (n x 256 B), signals and
+ * their offsets (n+1 uint64 word offsets) are laid out as for zkv_groth16_verify_batch_keys.
+ * zkv_groth16_verify_batch_rawkeys: status_out[i] = ZKV_OK or ZKV_VERIFICATION_FAILED, exactly what verify_proof_with_key returns for proof i
+ * under key key_idx[i].  Key bytes are untrusted: a key point out of range or off its curve fails the proof (through ecMul / ecAdd for the IC
+ * points, ecPairing for alpha, beta, gamma, delta), so does a beta, gamma or delta outside the order-r subgroup; a pair with a member at
+ * infinity contributes 1; A is negated for ZKV_VM_RISC0 keys; a signal count other than n_ic - 1 or a signal >= r fails that proof only.  For a
+ * key that zkv_vk_load accepts the status equals zkv_groth16_verify_batch's under that loaded key; keys that zkv_vk_load refuses for a missing
+ * normalised line table are verified too (this path uses unscaled lines).  ZKV_ERR_ARG with status_out untouched for a key length not of that
+ * form, a vm byte other than 0 / 1, key_idx[i] >= n_keys, decreasing offsets, a null pointer, or n_keys == 0 with n > 0; n == 0 does nothing.
+ * A multi-device handle splits the batch into contiguous caller ranges; a device pass holds up to 2^20 proofs and carries all the keys; when
+ * every input array is page-locked it is uploaded in place.  The kernel launches per pass do not depend on n_keys (zkv_launch_count: 4 for a
+ * pass of one kernel chain, 34 from the automatic chunking threshold of ZKV_TUNE_OVERLAP on).
+ * zkv_groth16_verify_batch_rawkeys_device: the same on device-resident arrays of one handle device (offsets index d_keys and d_signals
+ * directly), n <= 2^23, enqueued on `stream` (a cudaStream_t), asynchronous.  The checks run on the device there, per proof: a malformed key,
+ * a key index >= n_keys or a decreasing offset fails that proof (ZKV_VERIFICATION_FAILED).
+ * zkv_vk_x_rawkeys_batch (parity hook, first handle device): vk_x of proof i under its key (the chain of ecMul / ecAdd calls of compute_vk_x,
+ * groth16.rs:51-58, any 256-bit signal), 64 B per proof, all-zero for infinity or a failure; failed[i] = 1 where an ecMul / ecAdd call fails (an
+ * IC point out of range or off the curve) or the signal count is not n_ic - 1.  Argument errors as above (there are no vm bytes). */
+typedef struct zkv_rawkey_verifier zkv_rawkey_verifier;
+int zkv_rawkey_create(const int* devices, int n_dev, zkv_rawkey_verifier** out);
+void zkv_rawkey_destroy(zkv_rawkey_verifier* h);
+int zkv_groth16_verify_batch_rawkeys(const zkv_rawkey_verifier* h, const uint8_t* keys, const uint64_t* key_off, const uint8_t* key_vm, uint32_t n_keys,
+                                     const uint32_t* key_idx, const uint8_t* proofs, const uint8_t* signals, const uint64_t* sig_off,
+                                     size_t n, uint8_t* status_out);
+int zkv_groth16_verify_batch_rawkeys_device(const zkv_rawkey_verifier* h, int device, const void* d_keys, const void* d_key_off, const void* d_key_vm,
+                                            uint32_t n_keys, const void* d_key_idx, const void* d_proofs, const void* d_signals, const void* d_sig_off,
+                                            size_t n, void* d_status_out, void* stream);
+int zkv_vk_x_rawkeys_batch(const zkv_rawkey_verifier* h, const uint8_t* keys, const uint64_t* key_off, uint32_t n_keys, const uint32_t* key_idx,
+                           const uint8_t* signals, const uint64_t* sig_off, size_t n, uint8_t* out_points, uint8_t* failed);
+
 /* ---- RISC Zero (risc0/verifier.rs) -------------------------------------------------------
  * zkv_risc0_create(vk = NULL) uses the reference's hard-coded key; a custom vk (synthetic
  * benchmarks) is borrowed, not owned.  A handle starts un-initialised, like the contract. */

@@ -25,6 +25,11 @@ _SIGS = {
     "zkv_vkset_destroy": (None, [_P]),
     "zkv_groth16_verify_batch_keys": (C.c_int, [_P, _P, _P, _P, _P, C.c_size_t, _P]),
     "zkv_groth16_verify_batch_keys_device": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, C.c_size_t, _P, _P]),
+    "zkv_rawkey_create": (C.c_int, [_P, C.c_int, C.POINTER(_P)]),
+    "zkv_rawkey_destroy": (None, [_P]),
+    "zkv_groth16_verify_batch_rawkeys": (C.c_int, [_P, _P, _P, _P, C.c_uint32, _P, _P, _P, _P, C.c_size_t, _P]),
+    "zkv_groth16_verify_batch_rawkeys_device": (C.c_int, [_P, C.c_int, _P, _P, _P, C.c_uint32, _P, _P, _P, _P, C.c_size_t, _P, _P]),
+    "zkv_vk_x_rawkeys_batch": (C.c_int, [_P, _P, _P, C.c_uint32, _P, _P, _P, C.c_size_t, _P, _P]),
     "zkv_risc0_create": (C.c_int, [_P, _P, C.c_int, C.POINTER(_P)]),
     "zkv_risc0_destroy": (None, [_P]),
     "zkv_risc0_initialize": (C.c_int, [_P, _P, _P]),

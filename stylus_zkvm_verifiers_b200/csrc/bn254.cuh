@@ -806,9 +806,106 @@ ZKV_HD ZKV_INLINE void raw_to_be32(uint8_t* b, const uint32_t* v) {
     for (int i = 0; i < 8; i++) { uint8_t* q = b + 4 * (7 - i); q[0] = v[i] >> 24; q[1] = v[i] >> 16; q[2] = v[i] >> 8; q[3] = v[i]; }
 }
 ZKV_HD ZKV_INLINE void fp_to_be32(uint8_t* b, const fp& a) { fp t; fp_from_mont(t, a); raw_to_be32(b, t.v); }
+// EIP-196 G1 decoding from raw limbs: returns 0 valid point (Montgomery x,y), 1 infinity, 2 invalid
+ZKV_HD ZKV_INLINE int g1_decode_raw(fp& x, fp& y, const uint32_t* rx, const uint32_t* ry) {
+    if (u256_geq(rx, C_P) || u256_geq(ry, C_P)) return 2;
+    uint32_t any = 0;
+    for (int i = 0; i < 8; i++) any |= rx[i] | ry[i];
+    if (!any) { x = fp_zero(); y = fp_zero(); return 1; }
+    fp t;
+    for (int i = 0; i < 8; i++) t.v[i] = rx[i];
+    fp_to_mont(x, t);
+    for (int i = 0; i < 8; i++) t.v[i] = ry[i];
+    fp_to_mont(y, t);
+    return g1_on_curve(x, y) ? 0 : 2;
+}
 ZKV_HD inline void f12_to_bytes(uint8_t* out, const fp12& a) {   // 12 x BE-32, tower order c0.c0.c0, c0.c0.c1, c0.c1.c0, ...
     const fp* w = &a.c0.c0.c0;
     for (int i = 0; i < 12; i++) fp_to_be32(out + 32 * i, w[i]);
+}
+
+// ------------------------------------------------------------------------------------------ variable-base vk_x (keys passed as bytes)
+// acc += q, both Jacobian, complete: either at infinity, equal points (doubling) and opposite points (infinity) included
+ZKV_HD ZKV_NOINLINE void g1_add_jac(g1j& acc, const g1j& q) {
+    if (fp_is_zero(q.z)) return;
+    if (fp_is_zero(acc.z)) { acc = q; return; }
+    fp z1z1, z2z2, u1, u2, s1, s2, h, rr, t;
+    fp_sqr(z1z1, acc.z); fp_sqr(z2z2, q.z);
+    fp_mul(u1, acc.x, z2z2); fp_mul(u2, q.x, z1z1);
+    fp_mul(s1, acc.y, q.z); fp_mul(s1, s1, z2z2); fp_mul(s2, q.y, acc.z); fp_mul(s2, s2, z1z1);
+    fp_sub(h, u2, u1); fp_sub(rr, s2, s1);
+    if (fp_is_zero(h)) {
+        if (fp_is_zero(rr)) { g1j d; g1_dbl(d, acc); acc = d; }
+        else { acc.x = fp_one(); acc.y = fp_one(); acc.z = fp_zero(); }
+        return;
+    }
+    fp hh, hhh, v, x3, y3;
+    fp_sqr(hh, h); fp_mul(hhh, hh, h); fp_mul(v, u1, hh);
+    fp_sqr(x3, rr); fp_sub(x3, x3, hhh); fp_dbl(t, v); fp_sub(x3, x3, t);
+    fp_sub(t, v, x3); fp_mul(y3, rr, t); fp_mul(t, s1, hhh); fp_sub(y3, y3, t);
+    fp_mul(t, acc.z, q.z); fp_mul(acc.z, t, h); acc.x = x3; acc.y = y3;
+}
+#define ZKV_VKX_MAX_SCALARS 15            /* n_ic <= 16 */
+// width-4 NAF of k < 2^255 (odd digits -7..7, each non-zero digit followed by at least three zeros) as 256 nibbles, digit b in nibble b & 7 of
+// w[b >> 3].  Scanned from bit 0 with the carry c of the negative digits: an even window value is a zero digit and leaves c as it is.
+ZKV_HD ZKV_INLINE void g1_wnaf4(uint32_t* w, const uint32_t* k) {
+    for (int q = 0; q < 32; q++) w[q] = 0;
+    uint32_t c = 0;
+    for (int b = 0; b < 256;) {
+        const int q = b >> 5, sh = b & 31;
+        uint32_t win = k[q] >> sh;
+        if (sh > 28 && q < 7) win |= k[q + 1] << (32 - sh);
+        win = (win & 15u) + c;
+        if (!(win & 1u)) { b++; continue; }
+        c = win >= 8u;
+        w[b >> 3] |= (win & 15u) << (4 * (b & 7));         // win - 16 for a negative digit: the same low four bits
+        b += 4;
+    }
+}
+// vk_x = IC_0 + sum_j s_j IC_{j+1} (compute_vk_x, groth16.rs:51-58: the chain of ecMul / ecAdd precompile calls) for a key whose IC points
+// arrive as bytes: ic = n_ic x 64 B (EVM words), s = n_ic - 1 scalars as 32-byte BE words.  Any 256-bit scalar is taken (ecMul reduces it:
+// s P = (s mod r) P on G1).  Straus: one doubling chain shared by all scalars, each recoded as a width-4 NAF whose digits are added from a
+// per-thread table of P, 3P, 5P, 7P (Jacobian).  Every addition is complete, so IC points or partial sums at infinity, and partial sums
+// equal or opposite to a table entry, give the group's sum, which is what the chain computes; one inversion takes it to affine.
+// Returns 0 (x, y) finite, 1 infinity (x = y = 0), 2 an IC point fails the EIP-196 checks (the chain's ecMul / ecAdd call fails; x = y = 0).
+ZKV_HD ZKV_NOINLINE int g1_vkx_var(fp& x, fp& y, const uint8_t* ic, int n_ic, const uint8_t* s) {
+    g1j tab[ZKV_VKX_MAX_SCALARS][4];
+    uint32_t naf[ZKV_VKX_MAX_SCALARS][32];
+    bool bad = false;
+    g1j base; base.x = fp_one(); base.y = fp_one(); base.z = fp_zero();
+    for (int j = 0; j < n_ic; j++) {
+        uint32_t rx[8], ry[8];
+        be32_to_raw(rx, ic + 64 * j); be32_to_raw(ry, ic + 64 * j + 32);
+        fp px, py;
+        const int r = g1_decode_raw(px, py, rx, ry);
+        bad |= r == 2;
+        if (j == 0) { if (r == 0) { base.x = px; base.y = py; base.z = fp_one(); } continue; }
+        uint32_t k[8];
+        be32_to_raw(k, s + 32 * (j - 1));
+        while (u256_geq(k, C_R)) { uint32_t bo = 0; for (int t = 0; t < 8; t++) { uint64_t d = (uint64_t)k[t] - C_R[t] - bo; k[t] = (uint32_t)d; bo = (uint32_t)(d >> 63); } }
+        if (r != 0) for (int t = 0; t < 8; t++) k[t] = 0;      // IC_j at infinity adds nothing
+        g1_wnaf4(naf[j - 1], k);
+        if (r != 0) continue;
+        g1j* T = tab[j - 1];
+        T[0].x = px; T[0].y = py; T[0].z = fp_one();
+        g1j p2; g1_dbl(p2, T[0]);
+        for (int m = 1; m < 4; m++) { T[m] = T[m - 1]; g1_add_jac(T[m], p2); }
+    }
+    if (bad) { x = fp_zero(); y = fp_zero(); return 2; }
+    g1j acc; acc.x = fp_one(); acc.y = fp_one(); acc.z = fp_zero();
+    for (int b = 255; b >= 0; b--) {
+        if (!fp_is_zero(acc.z)) { g1j d; g1_dbl(d, acc); acc = d; }
+        for (int j = 0; j + 1 < n_ic; j++) {
+            const uint32_t nb = (naf[j][b >> 3] >> (4 * (b & 7))) & 15u;
+            if (!nb) continue;
+            const bool neg = nb >= 8u;
+            g1j e = tab[j][((neg ? 16u - nb : nb) >> 1)];
+            if (neg) fp_neg(e.y, e.y);
+            g1_add_jac(acc, e);
+        }
+    }
+    g1_add_jac(acc, base);
+    return g1_to_affine(x, y, acc) ? 0 : 1;
 }
 
 }  // namespace zkv

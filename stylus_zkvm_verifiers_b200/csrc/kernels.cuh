@@ -25,19 +25,7 @@ __device__ __forceinline__ uint8_t reject_status(uint8_t fl) { return (fl & F_BA
 struct g1aff { fp x, y; };             // (0,0) encodes infinity (not on the curve, so unambiguous)
 
 // ---------------------------------------------------------------------------- decode helpers
-// EIP-196 G1 decoding from raw limbs: returns 0 valid point (Montgomery x,y), 1 infinity, 2 invalid
-__device__ __forceinline__ int g1_decode_raw(fp& x, fp& y, const uint32_t* rx, const uint32_t* ry) {
-    if (u256_geq(rx, C_P) || u256_geq(ry, C_P)) return 2;
-    uint32_t any = 0;
-    for (int i = 0; i < 8; i++) any |= rx[i] | ry[i];
-    if (!any) { x = fp_zero(); y = fp_zero(); return 1; }
-    fp t;
-    for (int i = 0; i < 8; i++) t.v[i] = rx[i];
-    fp_to_mont(x, t);
-    for (int i = 0; i < 8; i++) t.v[i] = ry[i];
-    fp_to_mont(y, t);
-    return g1_on_curve(x, y) ? 0 : 2;
-}
+// (g1_decode_raw, the EIP-196 G1 decoding, lives in bn254.cuh: the variable-base vk_x of raw keys uses it on the host emulation too)
 // EIP-197 G2 decoding (wire order x_im, x_re, y_im, y_re), WITHOUT the subgroup test
 __device__ __forceinline__ int g2_decode_bytes(fp2& x, fp2& y, const uint8_t* b) {
     uint32_t r[4][8]; uint32_t any = 0; bool big = false;
@@ -754,6 +742,115 @@ __global__ void k_status_to_caller(int n, const uint32_t* total, const uint32_t*
     if (i >= n || (uint32_t)i >= *total) return;
     const uint32_t p = perm[i];
     if (p != ZKV_SLOT_EMPTY) status[p] = slot_status[i];
+}
+
+// ---------------------------------------------------------------------------- raw keys (zkv_groth16_verify_batch_rawkeys)
+// Proof i is verified under key key_idx[i] given as bytes: alpha (64 B), beta, gamma, delta (128 B each, wire order), IC_0 .. IC_{n_ic-1} (64 B
+// each) at keys + key_off[j] - key_base, with its vm byte key_vm[j].  There are no per-key tables: each thread gathers its own key's bytes, the
+// variable-base vk_x (g1_vkx_var) runs on its IC points, the Miller loop takes all four pairs as variable pairs with unscaled lines
+// (lz_miller_gen_seg, the loop of k_pairing_lz) and finishes the order-r test of B, beta, gamma and delta in its last segment
+// (lz_gen_subgroup_ok), so no grouping, table or G2-check kernel runs.  Pairs (pair-major, `stride` apart): 0 (A', B), 1 (alpha, beta),
+// 2 (vk_x, gamma), 3 (C, delta).
+#define ZKV_RAWKEY_FIXED 448                  /* alpha + beta + gamma + delta */
+enum : uint8_t { F_SKIPAB = 0x40 };           // pair 1 contributes 1 (pairs 0, 2, 3: F_SKIP0, F_SKIPX, F_SKIPC)
+struct RawKeysIn {                            // device pointers of a pass; offsets relative to key_base / sig_base
+    const uint8_t* keys; const uint64_t* key_off; uint64_t key_base; const uint8_t* key_vm; uint32_t nk;
+    const uint32_t* key_idx; const uint8_t* sig; const uint64_t* sig_off; uint64_t sig_base;
+};
+// proof i's key bytes and IC count, or nullptr for a key index >= nk, decreasing key offsets, a key length other than 448 + 64 n_ic with
+// n_ic in 2..16, a vm byte other than 0 / 1 (key_vm == nullptr: no vm byte) or a signal count other than n_ic - 1 (groth16.rs:32)
+__device__ __forceinline__ const uint8_t* rawkey_of(const RawKeysIn& in, int i, int& n_ic, int& vm, const uint8_t*& sig) {
+    const uint32_t j = in.key_idx[i];
+    if (j >= in.nk) return nullptr;
+    const uint64_t a = in.key_off[j], b = in.key_off[j + 1];
+    if (b < a || b - a < ZKV_RAWKEY_FIXED + 2 * 64 || b - a > ZKV_RAWKEY_FIXED + 16 * 64 || (b - a - ZKV_RAWKEY_FIXED) % 64) return nullptr;
+    n_ic = (int)((b - a - ZKV_RAWKEY_FIXED) / 64);
+    vm = in.key_vm ? in.key_vm[j] : 0;
+    if (vm > 1) return nullptr;
+    const uint64_t s0 = in.sig_off[i], s1 = in.sig_off[i + 1];
+    if (s1 < s0 || s1 - s0 != (uint64_t)(n_ic - 1)) return nullptr;
+    sig = in.sig + (size_t)(s0 - in.sig_base) * 32;
+    return in.keys + (size_t)(a - in.key_base);
+}
+// decode of proof i and its key's alpha, beta, gamma, delta (EIP-196/197 range, curve and infinity rules; the RISC Zero negation of A by the
+// key's vm); each signal < r (groth16.rs:32-34); T_j = -psi^3(Q_j) of the four G2 points for the Miller loop's subgroup test
+__global__ void k_decode_rawkeys(int n, RawKeysIn in, const uint8_t* proofs, size_t stride, fp* px, fp* py, fp2* qx, fp2* qy, fp2* tx, fp2* ty, uint8_t* flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int n_ic = 0, vm = 0; const uint8_t* sig = nullptr;
+    const uint8_t* key = rawkey_of(in, i, n_ic, vm, sig);
+    if (!key) {
+        for (int j = 0; j < 4; j++) { const size_t o = (size_t)j * stride + i; px[o] = fp_zero(); py[o] = fp_zero(); qx[o] = f2_zero(); qy[o] = f2_zero(); tx[o] = f2_zero(); ty[o] = f2_zero(); }
+        flags[i] = F_INVALID | F_SKIP0 | F_SKIPAB | F_SKIPX | F_SKIPC;
+        return;
+    }
+    decode_points(i, proofs + (size_t)i * 256, vm, px, py, qx, qy, px + 3 * stride, py + 3 * stride, flags);
+    uint8_t fl = flags[i];
+    for (int j = 0; j < n_ic - 1; j++) { uint32_t s[8]; be32_to_raw(s, sig + 32 * j); if (u256_geq(s, C_R)) fl |= F_INVALID; }
+    {
+        uint32_t rx[8], ry[8]; be32_to_raw(rx, key); be32_to_raw(ry, key + 32);
+        fp x = fp_zero(), y = fp_zero(); const int r = g1_decode_raw(x, y, rx, ry);
+        px[stride + i] = x; py[stride + i] = y;
+        if (r == 2) fl |= F_INVALID;
+        if (r == 1) fl |= F_SKIPAB;
+    }
+    const uint8_t inf_bit[3] = {F_SKIPAB, F_SKIPX, F_SKIPC};
+    for (int j = 1; j < 4; j++) {
+        fp2 x = f2_zero(), y = f2_zero();
+        const int r = g2_decode_bytes(x, y, key + 64 + 128 * (j - 1));
+        if (r == 2) { fl |= F_INVALID; x = f2_zero(); y = f2_zero(); }
+        if (r == 1) fl |= inf_bit[j - 1];
+        qx[(size_t)j * stride + i] = x; qy[(size_t)j * stride + i] = y;
+    }
+    for (int j = 0; j < 4; j++) {
+        const size_t o = (size_t)j * stride + i;
+        fp2 x = qx[o], y = qy[o];
+        g2_neg_psi3(x, y);
+        tx[o] = x; ty[o] = y;
+    }
+    flags[i] = fl;
+}
+// vk_x of each proof that is still valid from its key's IC points (g1_vkx_var) into pair 2; an invalid IC point fails the proof, vk_x = infinity
+// switches the pair off.  Then the per-pair skip bytes of the Miller loop: every pair of a failed proof, and each pair with a member at infinity.
+__global__ void k_vkx_rawkeys(int n, RawKeysIn in, size_t stride, fp* px, fp* py, uint8_t* flags, uint8_t* pskip) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint8_t fl = flags[i];
+    fp x = fp_zero(), y = fp_zero();
+    if (!(fl & F_INVALID)) {
+        int n_ic = 0, vm = 0; const uint8_t* sig = nullptr;
+        const uint8_t* key = rawkey_of(in, i, n_ic, vm, sig);
+        const int r = g1_vkx_var(x, y, key + ZKV_RAWKEY_FIXED, n_ic, sig);
+        if (r == 2) fl |= F_INVALID;
+        if (r == 1) fl |= F_SKIPX;
+    }
+    px[2 * stride + i] = x; py[2 * stride + i] = y;
+    flags[i] = fl;
+    const uint8_t bits[4] = {F_SKIP0, F_SKIPAB, F_SKIPX, F_SKIPC};
+    for (int j = 0; j < 4; j++) pskip[(size_t)j * stride + i] = (fl & (F_INVALID | bits[j])) ? 1 : 0;
+}
+// the four-variable-pair Miller loop (k_pairing_lz's body) whose last segment ORs F_INVALID into the flag byte of a proof with a G2 point outside
+// the order-r subgroup; `in` and tx / ty start at the chunk's first proof
+__global__ void __launch_bounds__(LZ_NT, 2) k_miller_rawkeys(int n, LzGenIn in, const fp2* tx, const fp2* ty, uint8_t* flags, fp12* fio, int d_hi, int d_lo, int first, int last) {
+    const size_t i = (size_t)blockIdx.x * LZ_NT + threadIdx.x;
+    const uint32_t tid = lz_tid();
+    if (first) { fp2 z = f2_zero(); lz_st2(tid + LZ_F * LZ_SLOT, f2_one()); for (int k = 1; k < 6; k++) lz_st2(tid + (LZ_F + 2 * k) * LZ_SLOT, z); }
+    else lz_ldg12(tid + LZ_F * LZ_SLOT, fio + i);
+    lz_miller_gen_seg(in, i, d_hi, d_lo, first != 0, last != 0);
+    if (last && !lz_gen_subgroup_ok(in, i, tx, ty) && i < (size_t)n) flags[i] |= F_INVALID;
+    lz_stg12(fio + i, tid + LZ_F * LZ_SLOT);
+}
+// parity hook: vk_x of proof i under its key as 64 bytes (zero for infinity or a failure); failed[i] = 1 for a malformed key or signal count
+// (rawkey_of) or an IC point that fails the EIP-196 checks
+__global__ void k_vkx_rawkeys_points(int n, RawKeysIn in, uint8_t* out, uint8_t* failed) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int n_ic = 0, vm = 0; const uint8_t* sig = nullptr;
+    const uint8_t* key = rawkey_of(in, i, n_ic, vm, sig);
+    fp x = fp_zero(), y = fp_zero();
+    const int r = key ? g1_vkx_var(x, y, key + ZKV_RAWKEY_FIXED, n_ic, sig) : 2;
+    fp_to_be32(out + 64 * (size_t)i, x); fp_to_be32(out + 64 * (size_t)i + 32, y);
+    failed[i] = r == 2;
 }
 
 // ---------------------------------------------------------------------------- small services

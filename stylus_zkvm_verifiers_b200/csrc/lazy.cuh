@@ -376,6 +376,20 @@ LZ_FN2 void lz_miller_gen_seg(LzGenIn in, size_t i, int d_hi, int d_lo, bool fir
     }
     if (keep && !last) { g2j* R = in.rst + i; R->x = lz_ld2(RR); R->y = lz_ld2(RR + 2 * LZ_SLOT); R->z = lz_ld2(RR + 4 * LZ_SLOT); }
 }
+// After the last segment of a loop with nvar > 1 (R_j in in.rst): the order-r test of every variable G2 point, R_j against T_j = -psi^3(Q_j)
+// (pair-major like the points).  The argument of lz_r_is holds per pair: each R_j ran through every doubling, addition and Frobenius step of
+// its own Q_j, whatever its skip byte said.  Uses the R slots.
+LZ_INL bool lz_gen_subgroup_ok(const LzGenIn& in, size_t i, const fp2* tx, const fp2* ty) {
+    const uint32_t RR = lz_tid() + LZ_R * LZ_SLOT;
+    bool ok = true;
+    for (int j = 0; j < in.nvar; j++) {
+        const size_t ij = (size_t)j * in.stride + i;
+        const g2j* R = in.rst + ij;
+        lz_st2(RR, R->x); lz_st2(RR + 2 * LZ_SLOT, R->y); lz_st2(RR + 4 * LZ_SLOT, R->z);
+        ok &= lz_r_is(RR, tx[ij], ty[ij]);
+    }
+    return ok;
+}
 LZ_INL void lz_miller_init(const fp2& qx, const fp2& qy) {       // f = 1, R = (qx, qy, 1)
     const uint32_t tid = lz_tid();
     fp2 one = f2_one(), z = f2_zero();

@@ -185,6 +185,7 @@ static int ctx_init(DevCtx* c) {
     CK(cudaFuncSetAttribute(k_pairing_lz, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_BYTES));
     CK(cudaFuncSetAttribute(k_miller_lz_keys, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_MILLER));
     CK(cudaFuncSetAttribute(k_final_exp_lz_keys, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_BYTES));
+    CK(cudaFuncSetAttribute(k_miller_rawkeys, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM_BYTES));
     return 0;
 }
 static int vk_build_on(zkv_vk* vk, DevCtx* c) {
@@ -757,7 +758,7 @@ static int keyset_pass(const zkv_vkset* s, SetDev* sd, size_t m, const uint32_t*
 template <class SetOf, class Pack, class Pass>
 static int grouped_host(const std::vector<DevCtx*>& ctxs, SetOf set_of, size_t n, bool direct, uint8_t* status_out, Pack pack, Pass pass) {
     return for_each_device(ctxs, n, [&](DevCtx* c, size_t b, size_t e) -> int {
-        SetDev* sd = set_of(c->device);
+        auto* sd = set_of(c->device);
         if (int rc = ctx_wait_idle(c)) return rc;      // a host call blocks anyway: wait out an earlier asynchronous device call here
         for (size_t s0 = b; s0 < e; s0 += MAX_CHUNK) {
             const size_t m = std::min(MAX_CHUNK, e - s0), bytes = pack(s0, m, (Sink*)nullptr);
@@ -813,6 +814,202 @@ extern "C" int zkv_groth16_verify_batch_keys_device(const zkv_vkset* s, int devi
     return device_call(sd->c, device, stream, [&](cudaStream_t st) {
         return keyset_pass(s, sd, n, (const uint32_t*)d_key_idx, (const uint8_t*)d_proofs, (const uint8_t*)d_signals, (const uint64_t*)d_sig_off, 0, (uint8_t*)d_status_out, st);
     });
+}
+
+// ------------------------------------------------------------------------------------------ raw keys: verify_proof_with_key with the key in the call
+// A handle owns, per device, a context without key tables (streams, events, staging, lock) and the workspace of the four-variable-pair path
+// (kernels.cuh, "raw keys"): per proof the four pairs' G1 and G2 points, the targets T_j, the accumulators R_j, the skip bytes, f, the
+// final-exponentiation state and the flag byte, 4 741 B (4.7 KB) in all.
+struct RawDev {
+    DevCtx* c = nullptr;
+    size_t cap = 0, stride = 0;
+    fp *px = nullptr, *py = nullptr; fp2 *qx = nullptr, *qy = nullptr, *tx = nullptr, *ty = nullptr; g2j* rst = nullptr; uint8_t* pskip = nullptr;
+    fp12 *f = nullptr, *fes = nullptr; uint8_t* flags = nullptr;
+};
+struct zkv_rawkey_verifier {
+    std::vector<RawDev> devs;
+    std::vector<DevCtx*> ctxs;            // devs[d].c (for_each_device)
+};
+static RawDev* raw_dev(const zkv_rawkey_verifier* h, int device) {
+    for (auto& d : h->devs) if (d.c->device == device) return const_cast<RawDev*>(&d);
+    return nullptr;
+}
+static void raw_free_ws(RawDev& d) {
+    cudaFree(d.px); cudaFree(d.py); cudaFree(d.qx); cudaFree(d.qy); cudaFree(d.tx); cudaFree(d.ty); cudaFree(d.rst); cudaFree(d.pskip); cudaFree(d.f); cudaFree(d.fes); cudaFree(d.flags);
+    d.px = d.py = nullptr; d.qx = d.qy = d.tx = d.ty = nullptr; d.rst = nullptr; d.pskip = d.flags = nullptr; d.f = d.fes = nullptr; d.cap = 0;
+}
+extern "C" void zkv_rawkey_destroy(zkv_rawkey_verifier* h) {
+    if (!h) return;
+    for (auto& d : h->devs) { cudaSetDevice(d.c->device); raw_free_ws(d); ctx_free(d.c); }
+    delete h;
+}
+extern "C" int zkv_rawkey_create(const int* devices, int n_dev, zkv_rawkey_verifier** out) {
+    if (!out) return fail(ZKV_ERR_ARG, "zkv_rawkey_create: null argument");
+    int ndev_sys = zkv_device_count();
+    if (ndev_sys <= 0) return fail(ZKV_ERR_CUDA, "zkv_rawkey_create: no CUDA device (this library has no CPU path)");
+    std::vector<int> devs;
+    if (!devices || n_dev <= 0) devs.push_back(0); else devs.assign(devices, devices + n_dev);
+    for (int d : devs) if (d < 0 || d >= ndev_sys) return fail(ZKV_ERR_ARG, "zkv_rawkey_create: bad device index");
+    zkv_rawkey_verifier* h = new zkv_rawkey_verifier();
+    h->devs.resize(devs.size());
+    for (size_t j = 0; j < devs.size(); j++) {
+        h->devs[j].c = new DevCtx(); h->devs[j].c->device = devs[j]; h->ctxs.push_back(h->devs[j].c);
+        int rc = ctx_init(h->devs[j].c);
+        if (rc) { zkv_rawkey_destroy(h); return rc; }
+    }
+    *out = h;
+    return 0;
+}
+// Grow the workspace to n proofs (+ PAD for the surplus threads of the last block); like ctx_reserve, it waits for an asynchronous user first.
+static int raw_reserve(RawDev* d, size_t n) {
+    if (n <= d->cap) return 0;
+    int rc = ctx_wait_idle(d->c); if (rc) return rc;
+    raw_free_ws(*d);
+    const size_t st = n + PAD;
+    CK(cudaMalloc(&d->px, 4 * st * sizeof(fp))); CK(cudaMalloc(&d->py, 4 * st * sizeof(fp)));
+    CK(cudaMalloc(&d->qx, 4 * st * sizeof(fp2))); CK(cudaMalloc(&d->qy, 4 * st * sizeof(fp2))); CK(cudaMalloc(&d->tx, 4 * st * sizeof(fp2))); CK(cudaMalloc(&d->ty, 4 * st * sizeof(fp2)));
+    CK(cudaMalloc(&d->rst, 4 * st * sizeof(g2j))); CK(cudaMalloc(&d->pskip, 4 * st)); CK(cudaMemset(d->pskip, 1, 4 * st));
+    CK(cudaMalloc(&d->f, st * sizeof(fp12))); CK(cudaMalloc(&d->fes, 6 * st * sizeof(fp12))); CK(cudaMalloc(&d->flags, st));
+    d->stride = st; d->cap = n;
+    return 0;
+}
+// One device pass of m <= MAX_CHUNK proofs on stream st, statuses in caller order to d_status; caller holds the context's lock and has set the
+// device.  Launches: decode, vk_x, then the heavy kernels scheduled like a key-set pass (chunk_count / fork_join): one Miller loop and one final
+// exponentiation for a pass of one chain, 4 chunks x (4 Miller segments + 4 final-exponentiation stages) from the automatic chunking threshold
+// on: 4 or 34 launches, whatever the number of keys.
+static int rawkey_pass(RawDev* d, const RawKeysIn& in, size_t m, const uint8_t* d_proofs, uint8_t* d_status, cudaStream_t st) {
+    DevCtx* c = d->c;
+    int rc = ctx_acquire(c, st); if (rc) return rc;
+    rc = raw_reserve(d, m); if (rc) return rc;
+    const int n = (int)m;
+    const size_t S = d->stride;
+    launch(k_decode_rawkeys, nblk(n), TPB, 0, st, n, in, d_proofs, S, d->px, d->py, d->qx, d->qy, d->tx, d->ty, d->flags);
+    launch(k_vkx_rawkeys, nblk(n), TPB, 0, st, n, in, S, d->px, d->py, d->flags, d->pskip);
+    auto heavy = [&](size_t o, int mm, cudaStream_t hs, int segs, bool staged) -> int {
+        LzGenIn gi; memset(&gi, 0, sizeof gi);
+        gi.px = d->px + o; gi.py = d->py + o; gi.qx = d->qx + o; gi.qy = d->qy + o; gi.rst = d->rst + o; gi.pskip = d->pskip + o;
+        gi.stride = S; gi.nvar = 4; gi.nfix = 0;
+        for (int k = 0; k < segs; k++) {
+            auto [hi, lo] = miller_segment(k, segs);
+            launch(k_miller_rawkeys, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs, mm, gi, d->tx + o, d->ty + o, d->flags + o, d->f + o, hi, lo, k == 0, k == segs - 1);
+        }
+        if (staged) for (int q = 0; q < 4; q++) launch(k_final_exp_lz, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs, mm, q, q, d->f + o, d->fes + 6 * o, d->flags + o, d_status + o, nullptr, 0);
+        else launch(k_final_exp_lz, nblk(mm, LZ_NT), LZ_NT, LZ_SMEM_BYTES, hs, mm, 0, 3, d->f + o, d->fes + 6 * o, d->flags + o, d_status + o, nullptr, 0);
+        return 0;
+    };
+    const int chunks = chunk_count(c, m, 0);
+    if (chunks <= 1) rc = heavy(0, n, st, 1, false);
+    else rc = fork_join(c, st, m, chunks, [&](size_t o, int mm, cudaStream_t hs) { return heavy(o, mm, hs, 4, true); });
+    if (rc) return rc;
+    CK(cudaGetLastError());
+    return 0;
+}
+// host-form checks of the key arrays: non-decreasing offsets, each key 448 + 64 n_ic bytes with n_ic in 2..16, vm bytes 0 / 1 (key_vm optional)
+static int rawkeys_check(const char* fn, const uint64_t* key_off, const uint8_t* key_vm, uint32_t n_keys) {
+    for (uint32_t j = 0; j < n_keys; j++) {
+        const uint64_t a = key_off[j], b = key_off[j + 1];
+        if (b < a) return fail(ZKV_ERR_ARG, std::string(fn) + ": key offsets must be non-decreasing");
+        if (b - a < ZKV_RAWKEY_FIXED + 2 * 64 || b - a > ZKV_RAWKEY_FIXED + 16 * 64 || (b - a - ZKV_RAWKEY_FIXED) % 64)
+            return fail(ZKV_ERR_ARG, std::string(fn) + ": key " + std::to_string(j) + " is not 448 + 64 n_ic bytes with n_ic in 2..16");
+        if (key_vm && key_vm[j] > 1) return fail(ZKV_ERR_ARG, std::string(fn) + ": key " + std::to_string(j) + " has a vm byte other than 0 / 1");
+    }
+    return 0;
+}
+static int rawkeys_args(const char* fn, const uint8_t* keys, const uint64_t* key_off, const uint8_t* key_vm, uint32_t n_keys, const uint32_t* key_idx,
+                        const uint8_t* signals, const uint64_t* sig_off, size_t n) {
+    if (n_keys == 0) return fail(ZKV_ERR_ARG, std::string(fn) + ": no keys");
+    if (n > 0xffffffffull) return fail(ZKV_ERR_ARG, std::string(fn) + ": batch too large");
+    if (!keys) return fail(ZKV_ERR_ARG, std::string(fn) + ": null keys");
+    if (int rc = rawkeys_check(fn, key_off, key_vm, n_keys)) return rc;
+    for (size_t i = 0; i < n; i++) if (key_idx[i] >= n_keys) return fail(ZKV_ERR_ARG, std::string(fn) + ": key index " + std::to_string(key_idx[i]) + " out of range");
+    if (!offsets_ok(sig_off, n)) return fail(ZKV_ERR_ARG, std::string(fn) + ": signal offsets must be non-decreasing");
+    if (sig_off[n] != sig_off[0] && !signals) return fail(ZKV_ERR_ARG, std::string(fn) + ": null signals");
+    return 0;
+}
+extern "C" int zkv_groth16_verify_batch_rawkeys(const zkv_rawkey_verifier* h, const uint8_t* keys, const uint64_t* key_off, const uint8_t* key_vm, uint32_t n_keys,
+                                                const uint32_t* key_idx, const uint8_t* proofs, const uint8_t* signals, const uint64_t* sig_off,
+                                                size_t n, uint8_t* status_out) {
+    const char* fn = "zkv_groth16_verify_batch_rawkeys";
+    if (!h || (n && (!key_off || !key_vm || !key_idx || !proofs || !sig_off || !status_out))) return fail(ZKV_ERR_ARG, std::string(fn) + ": null argument");
+    if (n == 0) return 0;
+    if (int rc = rawkeys_args(fn, keys, key_off, key_vm, n_keys, key_idx, signals, sig_off, n)) return rc;
+    const bool any_sig = sig_off[n] != sig_off[0];
+    const size_t key_bytes = (size_t)(key_off[n_keys] - key_off[0]);
+    const bool direct = n >= 4096 && is_pinned(keys) && is_pinned(key_off) && is_pinned(key_vm) && is_pinned(key_idx) && is_pinned(proofs) && is_pinned(sig_off)
+                        && (!any_sig || is_pinned(signals));      // page-locked caller arrays are uploaded in place
+    // pass block layout: [key bytes][key offsets][vm bytes][key_idx][signal offsets][proofs][signal words]; every pass carries all keys
+    auto up = [](size_t x) { return (x + 255) / 256 * 256; };
+    auto layout = [&](size_t s0, size_t m, size_t* o) {
+        o[0] = up(key_bytes); o[1] = o[0] + up(((size_t)n_keys + 1) * 8); o[2] = o[1] + up(n_keys); o[3] = o[2] + up(m * 4);
+        o[4] = o[3] + up((m + 1) * 8); o[5] = o[4] + m * 256;
+        return o[5] + (size_t)(sig_off[s0 + m] - sig_off[s0]) * 32;
+    };
+    return grouped_host(h->ctxs, [&](int d) { return raw_dev(h, d); }, n, direct, status_out,
+        [&](size_t s0, size_t m, Sink* sk) -> size_t {
+            size_t o[6]; const size_t bytes = layout(s0, m, o);
+            if (!sk) return bytes;
+            sk->put(0, keys + key_off[0], key_bytes, true); sk->put(o[0], key_off, ((size_t)n_keys + 1) * 8); sk->put(o[1], key_vm, n_keys);
+            sk->put(o[2], key_idx + s0, m * 4, true); sk->put(o[3], sig_off + s0, (m + 1) * 8, true); sk->put(o[4], proofs + s0 * 256, m * 256, true);
+            if (bytes > o[5]) sk->put(o[5], signals + sig_off[s0] * 32, bytes - o[5], true);
+            return bytes;
+        },
+        [&](RawDev* d, size_t s0, size_t m, uint8_t* blk) {
+            size_t o[6]; layout(s0, m, o);
+            RawKeysIn in;
+            in.keys = blk; in.key_off = (const uint64_t*)(blk + o[0]); in.key_base = key_off[0]; in.key_vm = blk + o[1]; in.nk = n_keys;
+            in.key_idx = (const uint32_t*)(blk + o[2]); in.sig_off = (const uint64_t*)(blk + o[3]); in.sig = blk + o[5]; in.sig_base = sig_off[s0];
+            return rawkey_pass(d, in, m, blk + o[4], d->c->d_out, d->c->stream);
+        });
+}
+extern "C" int zkv_groth16_verify_batch_rawkeys_device(const zkv_rawkey_verifier* h, int device, const void* d_keys, const void* d_key_off, const void* d_key_vm,
+                                                       uint32_t n_keys, const void* d_key_idx, const void* d_proofs, const void* d_signals, const void* d_sig_off,
+                                                       size_t n, void* d_status_out, void* stream) {
+    if (!h || !d_keys || !d_key_off || !d_key_vm || !d_key_idx || !d_proofs || !d_signals || !d_sig_off || !d_status_out)
+        return fail(ZKV_ERR_ARG, "zkv_groth16_verify_batch_rawkeys_device: null argument");
+    RawDev* d = raw_dev(h, device);
+    if (!d) return fail(ZKV_ERR_ARG, "device not in the handle's device list");
+    if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, "device batch too large");
+    if (n == 0) return 0;
+    return device_call(d->c, device, stream, [&](cudaStream_t st) {
+        for (size_t o = 0; o < n; o += MAX_CHUNK) {       // passes of MAX_CHUNK proofs: the signal offsets index d_signals directly
+            RawKeysIn in;
+            in.keys = (const uint8_t*)d_keys; in.key_off = (const uint64_t*)d_key_off; in.key_base = 0; in.key_vm = (const uint8_t*)d_key_vm; in.nk = n_keys;
+            in.key_idx = (const uint32_t*)d_key_idx + o; in.sig = (const uint8_t*)d_signals; in.sig_off = (const uint64_t*)d_sig_off + o; in.sig_base = 0;
+            int rc = rawkey_pass(d, in, std::min(MAX_CHUNK, n - o), (const uint8_t*)d_proofs + o * 256, (uint8_t*)d_status_out + o, st);
+            if (rc) return rc;
+        }
+        return 0;
+    });
+}
+extern "C" int zkv_vk_x_rawkeys_batch(const zkv_rawkey_verifier* h, const uint8_t* keys, const uint64_t* key_off, uint32_t n_keys, const uint32_t* key_idx,
+                                      const uint8_t* signals, const uint64_t* sig_off, size_t n, uint8_t* out_points, uint8_t* failed) {
+    const char* fn = "zkv_vk_x_rawkeys_batch";
+    if (!h || (n && (!key_off || !key_idx || !sig_off || !out_points || !failed))) return fail(ZKV_ERR_ARG, std::string(fn) + ": null argument");
+    if (n == 0) return 0;
+    if (n > MAX_CHUNK * 8) return fail(ZKV_ERR_ARG, std::string(fn) + ": batch too large");
+    if (int rc = rawkeys_args(fn, keys, key_off, nullptr, n_keys, key_idx, signals, sig_off, n)) return rc;
+    DevCtx* c = h->devs[0].c;
+    std::lock_guard<std::mutex> lk(c->mu);
+    CK(cudaSetDevice(c->device));
+    int rc = ctx_wait_idle(c); if (rc) return rc;
+    const size_t kb = (size_t)(key_off[n_keys] - key_off[0]), sb = (size_t)(sig_off[n] - sig_off[0]) * 32;
+    auto up = [](size_t x) { return (x + 255) / 256 * 256; };         // every array on a 256-byte boundary (the offsets are read as uint64)
+    const size_t o1 = up(kb), o2 = o1 + up(((size_t)n_keys + 1) * 8), o3 = o2 + up(n * 4), o4 = o3 + up((n + 1) * 8), total = o4 + sb;
+    rc = ctx_stage(c, total, n * 65); if (rc) return rc;
+    CK(cudaMemcpyAsync(c->d_in, keys + key_off[0], kb, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(c->d_in + o1, key_off, ((size_t)n_keys + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(c->d_in + o2, key_idx, n * 4, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(c->d_in + o3, sig_off, (n + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+    if (sb) CK(cudaMemcpyAsync(c->d_in + o4, signals + sig_off[0] * 32, sb, cudaMemcpyHostToDevice, c->stream));
+    RawKeysIn in;
+    in.keys = c->d_in; in.key_off = (const uint64_t*)(c->d_in + o1); in.key_base = key_off[0]; in.key_vm = nullptr; in.nk = n_keys;
+    in.key_idx = (const uint32_t*)(c->d_in + o2); in.sig_off = (const uint64_t*)(c->d_in + o3); in.sig = c->d_in + o4; in.sig_base = sig_off[0];
+    k_vkx_rawkeys_points<<<nblk(n), TPB, 0, c->stream>>>((int)n, in, c->d_out, c->d_out + n * 64);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(out_points, c->d_out, n * 64, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(failed, c->d_out + n * 64, n, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------ RISC Zero

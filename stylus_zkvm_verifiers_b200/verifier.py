@@ -127,8 +127,111 @@ class VerificationKeySet:
             pass
 
 
+def raw_key_bytes(alpha, beta, gamma, delta, ic):
+    """One key in the byte form of RawKeyVerifier / zkv_groth16_verify_batch_rawkeys: alpha (64 B), beta, gamma, delta (128 B each, wire order),
+    then the IC points (64 B each)."""
+    return bytes(alpha) + bytes(beta) + bytes(gamma) + bytes(delta) + b"".join(bytes(p) for p in ic)
+
+
+class RawKeyVerifier:
+    """Groth16 verification under keys passed as bytes with each call (zkv_rawkey_create): nothing is loaded, so every proof may bring its own
+    key.  The handle owns a workspace and streams per device (devices=None -> device 0)."""
+
+    def __init__(self, devices=None):
+        self._h = C.c_void_p()
+        arr, nd = _dev_array(devices)
+        N.check(N.lib().zkv_rawkey_create(arr, nd, C.byref(self._h)))
+
+    def close(self):
+        if getattr(self, "_h", None):
+            N.lib().zkv_rawkey_destroy(self._h); self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @staticmethod
+    def _pack_keys(keys):
+        """keys: (vm_type, alpha, beta, gamma, delta, ic) tuples -> key blob, key offsets (uint64), vm bytes (uint8)"""
+        blobs = [raw_key_bytes(*k[1:]) for k in keys]
+        return b"".join(blobs), _offsets(blobs), np.array([k[0] for k in keys], dtype=np.uint8)
+
+    @staticmethod
+    def _pack_signals(signals):
+        off = _offsets([b"\0" * 32 * len(s) for s in signals]) // 32
+        return b"".join(int(v).to_bytes(32, "big") for s in signals for v in s), off
+
+    def verify_batch(self, keys, key_idx, proofs, signals):
+        """Proof i (256 B; one n x 256-byte blob or a list of 256-byte proofs) under keys[key_idx[i]] with the integers signals[i] -> n status
+        bytes (ZKV_OK or ZKV_VERIFICATION_FAILED): what verify_proof_with_key returns for each."""
+        n = len(key_idx)
+        if len(signals) != n:
+            raise ValueError("signals: expected %d entries, got %d" % (n, len(signals)))
+        kb, ko, kv = self._pack_keys(keys)
+        sb, so = self._pack_signals(signals)
+        pr = proofs if isinstance(proofs, (bytes, bytearray, np.ndarray)) else b"".join(proofs)
+        return self.verify_batch_packed(kb, ko, kv, key_idx, pr, sb, so)
+
+    def verify_batch_packed(self, key_blob, key_off, key_vm, key_idx, proofs, sig_blob, sig_off, status_out=None):
+        """Zero-copy form: key_blob with n_keys + 1 uint64 byte offsets key_off and n_keys vm bytes; key_idx (uint32), proofs n x 256 B,
+        sig_blob = the signals as 32-byte words with n + 1 uint64 word offsets sig_off."""
+        key_off = np.ascontiguousarray(key_off, dtype=np.uint64)
+        key_vm = np.ascontiguousarray(key_vm, dtype=np.uint8)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        sig_off = np.ascontiguousarray(sig_off, dtype=np.uint64)
+        n, nk = len(key_idx), len(key_vm)
+        if len(key_off) != nk + 1:
+            raise ValueError("key_off: expected %d offsets, got %d" % (nk + 1, len(key_off)))
+        if (proofs.nbytes if isinstance(proofs, np.ndarray) else len(proofs)) != 256 * n:
+            raise ValueError("proofs: expected %d bytes" % (256 * n))
+        if len(sig_off) != n + 1:
+            raise ValueError("sig_off: expected %d offsets, got %d" % (n + 1, len(sig_off)))
+        st = status_out if status_out is not None else np.zeros(n, dtype=np.uint8)
+        nkb = key_blob.nbytes if isinstance(key_blob, np.ndarray) else len(key_blob)
+        nsb = sig_blob.nbytes if isinstance(sig_blob, np.ndarray) else len(sig_blob)
+        N.check(N.lib().zkv_groth16_verify_batch_rawkeys(self._h, N.buf(key_blob) if nkb else None, key_off.ctypes.data, key_vm.ctypes.data if nk else None, nk,
+                                                         key_idx.ctypes.data, N.buf(proofs) if n else None, N.buf(sig_blob) if nsb else None,
+                                                         sig_off.ctypes.data, n, st.ctypes.data))
+        return st
+
+    def verify_batch_device(self, device, d_keys, d_key_off, d_key_vm, n_keys, d_key_idx, d_proofs, d_signals, d_sig_off, n, d_status, stream=None):
+        """Inputs already in HBM (raw device pointers as ints; the offsets index d_keys and d_signals directly); asynchronous on `stream`.
+        A malformed key, a bad key index or a decreasing offset fails that proof."""
+        N.check(N.lib().zkv_groth16_verify_batch_rawkeys_device(self._h, device, d_keys, d_key_off, d_key_vm, n_keys, d_key_idx, d_proofs, d_signals,
+                                                                d_sig_off, n, d_status, stream))
+
+    def vk_x_batch(self, keys, key_idx, signals):
+        """vk_x of proof i under keys[key_idx[i]] (keys as for verify_batch; the vm byte is not used) -> (n x 64-byte points, n failed flags)"""
+        n = len(key_idx)
+        kb, ko, _ = self._pack_keys(keys)
+        sb, so = self._pack_signals(signals)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        out = C.create_string_buffer(64 * max(n, 1))
+        failed = np.zeros(n, dtype=np.uint8)
+        N.check(N.lib().zkv_vk_x_rawkeys_batch(self._h, N.buf(kb) if kb else None, ko.ctypes.data, len(keys), key_idx.ctypes.data,
+                                               N.buf(sb) if sb else None, so.ctypes.data, n, out, failed.ctypes.data))
+        return [out.raw[64 * i:64 * i + 64] for i in range(n)], failed
+
+
+_raw_default = None
+
+
 class Groth16Verifier:
     """common/groth16.rs:16-49."""
+
+    @staticmethod
+    def verify_proof_with_raw_key(vm_type, alpha, beta, gamma, delta, ic, a, b, c, signals):
+        """verify_proof_with_key(vm, &vk, a, b, c, &signals) with the key as bytes (alpha 64 B, beta / gamma / delta 128 B in wire order, ic a
+        list of 64-byte points), nothing loaded; a, b, c, signals as for verify_proof_with_key.  Returns bool.  Runs on device 0."""
+        global _raw_default
+        if _raw_default is None:
+            _raw_default = RawKeyVerifier()
+        w = lambda v: int(v).to_bytes(32, "big")
+        proof = w(a[0]) + w(a[1]) + w(b[0][0]) + w(b[0][1]) + w(b[1][0]) + w(b[1][1]) + w(c[0]) + w(c[1])
+        st = _raw_default.verify_batch([(vm_type, alpha, beta, gamma, delta, ic)], [0], proof, [list(signals)])
+        return bool(st[0] == N.ZKV_OK)
 
     @staticmethod
     def verify_proof_with_key(vk, a, b, c, signals):
